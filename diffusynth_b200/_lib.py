@@ -84,6 +84,10 @@ _SIGNATURES = {
     "ds_decode_stft": (_I, [_P, _P, _L, _I, _P]),
     "ds_encode_stft": (_I, [_P, _P, _L, _I, _P]),
     "ds_griffinlim_update": (_I, [_P, _P, _P, _F, _I, _I, _I, _P]),
+    "ds_pitch_shift_workspace": (_I, [_P, _P, _I, _P, _P]),
+    "ds_pitch_shift": (_I, [_P, _P, _P, _P, _I, _P, _L, _P]),
+    "ds_mix_track_workspace": (_I, [_P, _P, _I, _L, _P]),
+    "ds_mix_track": (_I, [_P, _P, _P, _P, _P, _I, _P, _L, _P, _L, _P]),
     "ds_spec_images": (_I, [_P, _P, _P, _P, _I, _I, _P]),
     "ds_latent_image": (_I, [_P, _P, _P, _I, _I, _I, _P]),
     "ds_text_embed_ln": (_I, [_P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _F, _P]),

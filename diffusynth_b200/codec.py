@@ -6,6 +6,7 @@ encode glue (sound2sound_with_text.py:80-94: ``adjust_audio_length`` -> ``libros
 ``encode_stft``) with one fused kernel sequence each (ds_stft_decode_istft / ds_stft_encode), fp32."""
 from __future__ import annotations
 
+import ctypes as C
 from typing import List, Optional
 
 import numpy as np
@@ -147,6 +148,100 @@ def griffinlim(magnitude: torch.Tensor, n_iter: int = 32, momentum: float = 0.99
               "ds_griffinlim_update")
     check(lib.ds_stft_decode_istft(spec.data_ptr(), frames.data_ptr(), wave.data_ptr(), B, T, st), "ds_stft_decode_istft")
     return wave
+
+
+# ---- note arrangements: pitch shift and track mix (track_maker.py:42 and the placement loop after it) -------------------------
+SAMPLE_RATE = 16000
+MAX_SEMITONES = 24
+
+
+def _check_steps(n_steps, count: int) -> np.ndarray:
+    n = np.broadcast_to(np.asarray(n_steps, dtype=np.float64), (count,)).copy()
+    if not np.all(np.isfinite(n)) or np.any(np.abs(n) > MAX_SEMITONES):
+        raise ValueError(f"n_steps must be finite with |n_steps| <= {MAX_SEMITONES}, got {n_steps}")
+    return n
+
+
+@torch.no_grad()
+def pitch_shift_packed(packed: torch.Tensor, lengths, n_steps, stages: Optional[dict] = None) -> torch.Tensor:
+    """Batched pitch shift of items packed back to back in one fp32 device tensor (item k: lengths[k] samples) by n_steps[k]
+    semitones (ds_pitch_shift); the result has the same layout.  ``stages`` (a dict, tests): receives the workspace and the byte
+    offsets of the intermediate stages (see the header)."""
+    lib = _lib.load()
+    L = np.ascontiguousarray(lengths, dtype=np.int64)
+    n = _check_steps(n_steps, len(L))
+    packed = packed.float().contiguous()
+    assert packed.dim() == 1 and packed.numel() == int(L.sum()), "packed length must equal the sum of the item lengths"
+    nbytes, offs = C.c_longlong(0), (C.c_longlong * 4)()
+    check(lib.ds_pitch_shift_workspace(L.ctypes.data, n.ctypes.data, len(L), C.byref(nbytes), offs), "ds_pitch_shift_workspace")
+    ws = torch.empty((nbytes.value,), dtype=torch.uint8, device=packed.device)
+    out = torch.empty_like(packed)
+    check(lib.ds_pitch_shift(packed.data_ptr(), out.data_ptr(), L.ctypes.data, n.ctypes.data, len(L), ws.data_ptr(), nbytes.value,
+                             ops._stream()), "ds_pitch_shift")
+    if stages is not None:
+        stages.update(workspace=ws, offsets=list(offs))
+    return out
+
+
+def pitch_shift(waves, n_steps):
+    """On-device, batched ``librosa.effects.pitch_shift(y, sr=16000, n_steps=n_steps, bins_per_octave=12)`` (track_maker.py:42)
+    with librosa's default STFT arguments; the resampler is a Kaiser-windowed sinc (resampy kaiser_best) instead of librosa's soxr.
+    ``waves``: a [B, L] or [L] tensor / numpy array, or a list of 1-D ones of different lengths; ``n_steps``: a scalar or one per
+    item, finite, |n_steps| <= 24.  Returns the same layout (numpy in, numpy out; fp32)."""
+    is_list = isinstance(waves, (list, tuple))
+    items = list(waves) if is_list else None
+    if not is_list:
+        arr = waves
+        if arr.ndim == 1:
+            items = [arr]
+        else:
+            assert arr.ndim == 2, "expected [B, L], [L] or a list of 1-D signals"
+            items = [arr[b] for b in range(arr.shape[0])]
+    is_np = isinstance(items[0], np.ndarray)
+    dev = _device() if is_np or not items[0].is_cuda else items[0].device
+    ts = [(torch.from_numpy(np.ascontiguousarray(w, dtype=np.float32)) if is_np else w).reshape(-1).to(dev, torch.float32)
+          for w in items]
+    lengths = [t.numel() for t in ts]
+    out = pitch_shift_packed(torch.cat(ts), lengths, n_steps)
+    parts = list(torch.split(out, lengths))
+    if is_list:
+        return [p.cpu().numpy() for p in parts] if is_np else parts
+    res = out.view(len(lengths), lengths[0]) if waves.ndim == 2 else out
+    return res.cpu().numpy() if is_np else res
+
+
+@torch.no_grad()
+def mix_track(packed: torch.Tensor, src_offsets, lengths, onsets, gains, track_len: Optional[int] = None) -> torch.Tensor:
+    """Place and sum notes into one fp32 track (ds_mix_track): note n is ``packed[src_offsets[n] : src_offsets[n] + lengths[n]]``
+    times gains[n], starting at sample onsets[n]; notes may share a source.  Summed in note order, bit-identical run to run.
+    ``track_len`` defaults to the end of the last note."""
+    lib = _lib.load()
+    off = np.ascontiguousarray(src_offsets, dtype=np.int64)
+    L = np.ascontiguousarray(lengths, dtype=np.int64)
+    on = np.ascontiguousarray(onsets, dtype=np.int64)
+    g = np.ascontiguousarray(gains, dtype=np.float32)
+    K = len(L)
+    if track_len is None:
+        track_len = int((on + L).max())
+    nbytes = C.c_longlong(0)
+    check(lib.ds_mix_track_workspace(L.ctypes.data, on.ctypes.data, K, int(track_len), C.byref(nbytes)), "ds_mix_track_workspace")
+    packed = packed.float().contiguous()
+    ws = torch.empty((nbytes.value,), dtype=torch.uint8, device=packed.device)
+    track = torch.empty((int(track_len),), dtype=torch.float32, device=packed.device)
+    check(lib.ds_mix_track(packed.data_ptr(), off.ctypes.data, L.ctypes.data, on.ctypes.data, g.ctypes.data, K, track.data_ptr(),
+                           int(track_len), ws.data_ptr(), nbytes.value, ops._stream()), "ds_mix_track")
+    return track
+
+
+def shift_and_mix(sources, semitones, note_source, onsets, gains) -> torch.Tensor:
+    """The arrangement stage after synthesis: every source (1-D fp32 device tensor) is pitch-shifted by its semitones in ONE batched
+    call, then note n -- source note_source[n] at sample onsets[n], scaled by gains[n] -- is mixed in ONE call.  Two library
+    calls plus their workspace queries, whatever the number of notes."""
+    lengths = [int(s.numel()) for s in sources]
+    shifted = pitch_shift_packed(torch.cat([s.reshape(-1) for s in sources]), lengths, semitones)
+    starts = np.concatenate([[0], np.cumsum(lengths)[:-1]]).astype(np.int64)
+    idx = np.asarray(note_source, dtype=np.int64)
+    return mix_track(shifted, starts[idx], np.asarray(lengths, dtype=np.int64)[idx], onsets, gains)
 
 
 @torch.no_grad()

@@ -8,6 +8,7 @@
 // butterflies in registers and across lanes with warp shuffles, one staging pass through shared memory for the natural-order
 // result; everything is fp32 (the reference runs float64 on the CPU).
 #include "common.cuh"
+#include "fft_warp.cuh"
 #include <mutex>
 #include "../../include/diffusynth_b200.h"
 
@@ -15,55 +16,7 @@ namespace ds {
 
 static constexpr int NFFT = 1024, NH = 512, HOP = 256;
 static constexpr int FR = 8;   // frames per block
-
-__device__ __forceinline__ float2 cmul(float2 a, float2 b) { return make_float2(a.x * b.x - a.y * b.y, a.x * b.y + a.y * b.x); }
-
-// 512-point complex DFT of one frame per WARP, in registers with warp-shuffle butterflies:
-//   out[n] = sum_k in[k] e^{SIGN*2*pi*i*k*n/512}.
-// Lane l holds the 16 points i = l + 32 r (r = register index).  Radix-2 decimation in frequency: the four stages that pair
-// points 256 / 128 / 64 / 32 apart are register-to-register, the five that pair points 16 .. 1 apart exchange registers between
-// lanes with __shfl_xor_sync; no shared memory and no block barrier inside the transform.  On return x[r] holds
-// out[bitrev9(l + 32 r)] = out[(bitrev5(l) << 4) | bitrev4(r)].
-__device__ __forceinline__ float2 cadd(float2 a, float2 b) { return make_float2(a.x + b.x, a.y + b.y); }
-__device__ __forceinline__ float2 csub(float2 a, float2 b) { return make_float2(a.x - b.x, a.y - b.y); }
-
-template <int SIGN>
-__device__ __forceinline__ void fft512_warp(float2 (&x)[16], const float2* __restrict__ tw /* e^{+2 pi i j/512}, j<256 */, int lane) {
-#pragma unroll
-  for (int rb = 3; rb >= 0; --rb) {          // point-index bit b = rb + 5 lives in the register index
-    const int half = 1 << rb;
-#pragma unroll
-    for (int r = 0; r < 16; ++r) {
-      if (r & half) continue;
-      float2 w = __ldg(tw + ((lane + 32 * (r & (half - 1))) << (3 - rb)));      // W_512^((i mod 2^b) * 2^(8-b))
-      if (SIGN < 0) w.y = -w.y;
-      const float2 u = x[r], v = x[r + half];
-      x[r] = cadd(u, v);
-      x[r + half] = cmul(csub(u, v), w);
-    }
-  }
-#pragma unroll
-  for (int b = 4; b >= 0; --b) {             // point-index bit b is lane bit b
-    const int m = 1 << b;
-    const bool upper = (lane & m) != 0;
-    float2 w = __ldg(tw + ((lane & (m - 1)) << (8 - b)));
-    if (SIGN < 0) w.y = -w.y;
-#pragma unroll
-    for (int r = 0; r < 16; ++r) {
-      const float2 o = make_float2(__shfl_xor_sync(0xffffffffu, x[r].x, m), __shfl_xor_sync(0xffffffffu, x[r].y, m));
-      x[r] = upper ? cmul(csub(o, x[r]), w) : cadd(x[r], o);
-    }
-  }
-}
-// The transform's results are staged once in shared memory in natural order, one padding entry per 16 (the lanes of a warp
-// write bins 16 apart): xs[frame][pidx(bin)].
-static constexpr int XS_PITCH = NH + NH / 16;
-__device__ __forceinline__ int pidx(int k) { return k + (k >> 4); }
-__device__ __forceinline__ void store_bitrev(float2* __restrict__ xs, const float2 (&x)[16], int lane) {
-  const int hi = (int)(__brev((unsigned)lane) >> 27) << 4;
-#pragma unroll
-  for (int r = 0; r < 16; ++r) xs[pidx(hi | (int)(__brev((unsigned)r) >> 28))] = x[r];
-}
+static constexpr int XS_PITCH = NH + NH / 16;   // staging row of a 512-point transform (fft_warp.cuh)
 
 // ---- inverse: spec [B,3,512,T] fp32 -> windowed frames [B][T][1024] fp32; one frame per warp, FR = 8 frames per block ----
 __global__ void __launch_bounds__(256)
@@ -104,14 +57,14 @@ istft_frames_kernel(const float* __restrict__ spec, float* __restrict__ frames, 
     const float2 o = cmul(make_float2(a.x - c.x, a.y + c.y), __ldg(tw1024 + k));
     x[r] = make_float2(e.x - o.y, e.y + o.x);
   }
-  fft512_warp<+1>(x, tw512, lane);
-  store_bitrev(xs[fr], x, lane);
+  fft_warp<+1, 16>(x, tw512, lane);
+  store_bitrev<16>(xs[fr], x, lane);
   __syncwarp();
   // x[2n] = Re z[n] / 1024, x[2n+1] = Im z[n] / 1024; times the periodic Hann window
   const int t = t0 + fr;
   if (t >= T) return;
   for (int n = lane; n < NH; n += 32) {
-    const float2 z = xs[fr][pidx(n)];
+    const float2 z = xs[fr][pidx<16>(n)];
     const float w0 = 0.5f - 0.5f * cospif((float)(2 * n) / 512.0f), w1 = 0.5f - 0.5f * cospif((float)(2 * n + 1) / 512.0f);
     reinterpret_cast<float2*>(frames + ((size_t)b * T + t) * NFFT)[n] = make_float2(z.x * (1.0f / NFFT) * w0, z.y * (1.0f / NFFT) * w1);
   }
@@ -161,8 +114,8 @@ stft_encode_kernel(const float* __restrict__ wave, long long L, float* __restric
       const float w0 = 0.5f - 0.5f * cospif((float)(2 * n) / 512.0f), w1 = 0.5f - 0.5f * cospif((float)(2 * n + 1) / 512.0f);
       x[r] = make_float2(a * w0, c * w1);
     }
-    fft512_warp<-1>(x, tw512, lane);
-    store_bitrev(xs[fr], x, lane);
+    fft_warp<-1, 16>(x, tw512, lane);
+    store_bitrev<16>(xs[fr], x, lane);
   }
   __syncthreads();
   // X[k] = (Z[k] + conj Z[512-k])/2 - i/2 * e^{-2 pi i k/1024} (Z[k] - conj Z[512-k]),  k = 1..512 (row k-1); DC row dropped (pad_STFT)
@@ -172,7 +125,7 @@ stft_encode_kernel(const float* __restrict__ wave, long long L, float* __restric
     if (t >= Tpad) continue;
     float lm = 0.f, co = 1.f, si = 0.f;      // padded frames: |D| = 0 -> log1p 0 = 0, angle(0) = 0 -> cos 1, sin 0
     if (t < T) {
-      const float2 zk = xs[fr][pidx(k & (NH - 1))], zc = xs[fr][pidx((NH - k) & (NH - 1))];
+      const float2 zk = xs[fr][pidx<16>(k & (NH - 1))], zc = xs[fr][pidx<16>((NH - k) & (NH - 1))];
       const float2 e = make_float2(0.5f * (zk.x + zc.x), 0.5f * (zk.y - zc.y));
       const float2 d = make_float2(0.5f * (zk.x - zc.x), 0.5f * (zk.y + zc.y));
       float2 w = k < NH ? __ldg(tw1024 + k) : make_float2(-1.f, 0.f);
@@ -236,20 +189,21 @@ __global__ void encode_stft_kernel(const T* __restrict__ D, T* __restrict__ out,
   }
 }
 
-__global__ void twiddle_init_kernel(float2* tw512, float2* tw1024) {
+__global__ void twiddle_init_kernel(float2* tw512, float2* tw1024, float2* tw2048) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < 256) { double s, c; sincospi((double)i / 256.0, &s, &c); tw512[i] = make_float2((float)c, (float)s); }
   if (i < 512) { double s, c; sincospi((double)i / 512.0, &s, &c); tw1024[i] = make_float2((float)c, (float)s); }
+  if (i < 1024) { double s, c; sincospi((double)i / 1024.0, &s, &c); tw2048[i] = make_float2((float)c, (float)s); }
 }
 
-struct Twiddles { float2* tw512 = nullptr; float2* tw1024 = nullptr; bool ready = false; };
+struct Twiddles { float2* tw512 = nullptr; float2* tw1024 = nullptr; float2* tw2048 = nullptr; bool ready = false; };
 static Twiddles g_tw[64];
 static std::mutex g_tw_mutex;
 
 // Per-device twiddle tables, built once under a mutex on a private blocking stream and synchronised before the first use, so
 // the first caller's stream (or a second host thread on another stream) can never read a half-built table.  The build
 // allocates, so it must not run during a stream capture: a capturing first call is refused (callers warm up once).
-static int get_twiddles(cudaStream_t stream, float2** a, float2** b) {
+int get_twiddles(cudaStream_t stream, float2** a, float2** b, float2** c) {
   int dev = 0;
   DS_CHECK_CUDA(cudaGetDevice(&dev));
   DS_REQUIRE(dev >= 0 && dev < 64, "istft: device index %d out of range", dev);
@@ -261,9 +215,10 @@ static int get_twiddles(cudaStream_t stream, float2** a, float2** b) {
     DS_REQUIRE(cs == cudaStreamCaptureStatusNone, "istft: the first STFT/iSTFT call on a device builds its twiddle tables and cannot be captured in a graph; run it once eagerly");
     DS_CHECK_CUDA(cudaMalloc(&t.tw512, 256 * sizeof(float2)));
     DS_CHECK_CUDA(cudaMalloc(&t.tw1024, 512 * sizeof(float2)));
+    DS_CHECK_CUDA(cudaMalloc(&t.tw2048, 1024 * sizeof(float2)));
     cudaStream_t s0;
     DS_CHECK_CUDA(cudaStreamCreate(&s0));
-    twiddle_init_kernel<<<2, 256, 0, s0>>>(t.tw512, t.tw1024);
+    twiddle_init_kernel<<<4, 256, 0, s0>>>(t.tw512, t.tw1024, t.tw2048);
     DS_CHECK_CUDA(cudaGetLastError());
     DS_CHECK_CUDA(cudaStreamSynchronize(s0));
     DS_CHECK_CUDA(cudaStreamDestroy(s0));
@@ -271,6 +226,7 @@ static int get_twiddles(cudaStream_t stream, float2** a, float2** b) {
   }
   *a = t.tw512;
   *b = t.tw1024;
+  *c = t.tw2048;
   return DS_OK;
 }
 
@@ -285,8 +241,8 @@ long long ds_istft_length(int T) { return (long long)HOP * (T - 1); }
 /* d_spec fp32 [B,3,512,T] (decoder output) -> d_wave fp32 [B, 256*(T-1)].  d_frames: scratch fp32 [B*T*1024]. */
 int ds_stft_decode_istft(const float* d_spec, float* d_frames, float* d_wave, int B, int T, void* stream) {
   DS_REQUIRE(d_spec && d_frames && d_wave && B > 0 && T > 1, "ds_stft_decode_istft: bad arguments");
-  float2 *tw512, *tw1024;
-  int rc = get_twiddles((cudaStream_t)stream, &tw512, &tw1024);
+  float2 *tw512, *tw1024, *tw2048;
+  int rc = get_twiddles((cudaStream_t)stream, &tw512, &tw1024, &tw2048);
   if (rc) return rc;
   const size_t smem = FR * (NH + 1) * sizeof(float2) + FR * XS_PITCH * sizeof(float2);
   DS_CHECK_CUDA(cudaFuncSetAttribute(istft_frames_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -303,8 +259,8 @@ int ds_stft_encode(const float* d_wave, long long L, float* d_spec, int B, int T
   DS_REQUIRE(d_wave && d_spec && B > 0 && L > 0 && Tpad > 0, "ds_stft_encode: bad arguments");
   const int T = 1 + (int)(L / HOP);
   DS_REQUIRE(T <= Tpad, "ds_stft_encode: %d frames exceed the time resolution %d", T, Tpad);
-  float2 *tw512, *tw1024;
-  int rc = get_twiddles((cudaStream_t)stream, &tw512, &tw1024);
+  float2 *tw512, *tw1024, *tw2048;
+  int rc = get_twiddles((cudaStream_t)stream, &tw512, &tw1024, &tw2048);
   if (rc) return rc;
   const size_t smem = FR * XS_PITCH * sizeof(float2);
   DS_CHECK_CUDA(cudaFuncSetAttribute(stft_encode_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));

@@ -1,0 +1,455 @@
+// Pitch shifting and track mixing for note arrangements (track_maker.DiffSynth after the per-note closure, track_maker.py:42):
+//   librosa.effects.pitch_shift(y, sr=16000, n_steps=n, bins_per_octave=12) with librosa's default STFT arguments
+//     = time_stretch(y, rate = 2^(-n/12)) -> resample(16000/rate -> 16000 Hz) -> fix_length(len(y)),
+//     time_stretch = stft(n_fft 2048, hop 512, periodic Hann, centre zero padding) -> phase_vocoder(hop 512)
+//                    -> istft(length = round(len(y)/rate));
+//   then every note is scaled by its gain, placed at its onset and summed into one track.
+// The resampler is a Kaiser-windowed sinc evaluated directly (resampy's kaiser_best parameters), not librosa's default soxr
+// (DESIGN.md section 8).  Every stage runs over a ragged batch: per-item prefix offsets into packed buffers, lengths and rates as
+// plain device arrays, one launch per stage whatever the number of items.  Everything is fp32 except the positions and the
+// rates, which are float64 like numpy's.
+#include "common.cuh"
+#include "fft_warp.cuh"
+#include <cmath>
+#include <vector>
+#include "../../include/diffusynth_b200.h"
+
+namespace ds {
+namespace {
+
+constexpr int NFFT = 2048, NC = 1024 /* complex points */, NBIN = NFFT / 2 + 1, HOP = 512;
+constexpr int R = NC / 32;                      // points per lane
+constexpr int XS_PITCH = NC + NC / R;           // staging row (fft_warp.cuh)
+constexpr int FR = 8;                           // frames (warps) per block
+constexpr int MIX_TILE = 1024;                  // track samples per mix block
+constexpr double kPi = 3.14159265358979323846;
+// resampy's kaiser_best filter: 64 zero crossings per side, roll-off and Kaiser beta
+constexpr int RS_ZEROS = 64;
+constexpr double RS_ROLLOFF = 0.9475937167399596, RS_BETA = 14.769656459379492;
+
+// item of a global index: the k with off[k] <= g < off[k+1] (off is a prefix array of B+1 entries, off[0] = 0)
+__device__ __forceinline__ int find_item(const long long* __restrict__ off, int B, long long g) {
+  int lo = 0, hi = B - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (__ldg(off + mid) <= g) lo = mid; else hi = mid - 1;
+  }
+  return lo;
+}
+
+__device__ __forceinline__ float hann2048(int m) { return 0.5f - 0.5f * cospif((float)m / 1024.0f); }
+
+// ---- forward STFT: y (packed, item k at loff[k], length L_k) -> D [frames][1025] complex; one frame per warp ----------------
+// frame t of item k covers samples t*512 - 1024 .. t*512 + 1023 (centre zero padding); z[n] = x[2n] + i x[2n+1] of the windowed
+// frame goes through one 1024-point complex FFT, the real spectrum is unpacked from it.
+__global__ void __launch_bounds__(256)
+pitch_stft_kernel(const float* __restrict__ y, const long long* __restrict__ loff, const long long* __restrict__ fin, int B,
+                  float2* __restrict__ D, const float2* __restrict__ tw1024, const float2* __restrict__ tw2048) {
+  pdl_enter();
+  extern __shared__ __align__(16) uint8_t ps_smem[];
+  float2 (*xs)[XS_PITCH] = reinterpret_cast<float2 (*)[XS_PITCH]>(ps_smem);
+  const int fr = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const long long g = (long long)blockIdx.x * FR + fr;
+  if (g >= __ldg(fin + B)) return;                       // whole warps leave: the transform is warp-local
+  const int k = find_item(fin, B, g);
+  const long long t = g - __ldg(fin + k), L = __ldg(loff + k + 1) - __ldg(loff + k);
+  const float* wv = y + __ldg(loff + k);
+  float2 x[R];
+#pragma unroll
+  for (int r = 0; r < R; ++r) {
+    const int n = lane + 32 * r;
+    const long long s0 = t * HOP - NFFT / 2 + 2 * n;
+    const float a = (s0 >= 0 && s0 < L) ? __ldg(wv + s0) : 0.f;
+    const float c = (s0 + 1 >= 0 && s0 + 1 < L) ? __ldg(wv + s0 + 1) : 0.f;
+    x[r] = make_float2(a * hann2048(2 * n), c * hann2048(2 * n + 1));
+  }
+  fft_warp<-1, R>(x, tw1024, lane);
+  store_bitrev<R>(xs[fr], x, lane);
+  __syncwarp();
+  // X[k] = (Z[k] + conj Z[1024-k])/2 - i/2 e^{-2 pi i k/2048} (Z[k] - conj Z[1024-k]),  k = 0..1024
+  float2* out = D + g * NBIN;
+  for (int b = lane; b < NBIN; b += 32) {
+    const float2 zk = xs[fr][pidx<R>(b & (NC - 1))], zc = xs[fr][pidx<R>((NC - b) & (NC - 1))];
+    const float2 e = make_float2(0.5f * (zk.x + zc.x), 0.5f * (zk.y - zc.y));
+    const float2 d = make_float2(0.5f * (zk.x - zc.x), 0.5f * (zk.y + zc.y));
+    float2 w = b < NC ? __ldg(tw2048 + b) : make_float2(-1.f, 0.f);
+    w.y = -w.y;
+    const float2 o = cmul(d, w);                          // then multiply by -i: (x, y) -> (y, -x)
+    out[b] = make_float2(e.x + o.y, e.y - o.x);
+  }
+}
+
+// ---- phase vocoder (librosa.phase_vocoder, hop 512): one thread per (item, bin), output frames walked in order ----------------
+// step_t = t * rate (float64, numpy's arange); |S| interpolates |D| linearly between frames floor(step) and floor(step)+1 (D
+// zero-padded by two frames); the phase accumulator starts at angle(D[0]) and advances by phi + wrap(dphase - phi).  It is kept
+// wrapped to [-pi, pi): unwrapped it grows to ~1e5 rad, where an fp32 ulp is ~0.008 rad.  phi = bin * pi * hop / 1024 is
+// reduced mod 2 pi in float64.
+__device__ __forceinline__ float wrap_pi(float v) {           // x - 2 pi round(x / 2 pi), numpy's rounding (half to even)
+  return v - 6.283185307179586f * rintf(v * 0.15915494309189535f);
+}
+__global__ void __launch_bounds__(256)
+pitch_vocoder_kernel(const float2* __restrict__ D, float2* __restrict__ S, const long long* __restrict__ fin,
+                     const long long* __restrict__ fout, const double* __restrict__ rate, int B) {
+  pdl_enter();
+  const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (gid >= (long long)B * NBIN) return;
+  const int k = (int)(gid / NBIN), bin = (int)(gid - (long long)k * NBIN);
+  const long long f0 = __ldg(fin + k), T_in = __ldg(fin + k + 1) - f0, o0 = __ldg(fout + k), T_out = __ldg(fout + k + 1) - o0;
+  const double rt = __ldg(rate + k);
+  double adv = fmod((double)bin * (kPi * HOP / (NFFT / 2)), 2.0 * kPi);
+  if (adv >= kPi) adv -= 2.0 * kPi;
+  const float phi = (float)adv;
+  const float2* Dk = D + f0 * NBIN + bin;
+  float2* Sk = S + o0 * NBIN + bin;
+  float2 c0 = __ldg(Dk);
+  float acc = atan2f(c0.y, c0.x);
+  for (long long t = 0; t < T_out; ++t) {
+    const double step = (double)t * rt;
+    const long long i = (long long)floor(step);
+    const float a = (float)(step - (double)i);
+    c0 = __ldg(Dk + i * NBIN);
+    const float2 c1 = i + 1 < T_in ? __ldg(Dk + (i + 1) * NBIN) : make_float2(0.f, 0.f);
+    const float mag = (1.0f - a) * hypotf(c0.x, c0.y) + a * hypotf(c1.x, c1.y);
+    float sn, cs;
+    sincosf(acc, &sn, &cs);
+    Sk[t * NBIN] = make_float2(mag * cs, mag * sn);
+    const float dph = wrap_pi(atan2f(c1.y, c1.x) - atan2f(c0.y, c0.x) - phi);
+    acc = acc + phi + dph;
+    acc -= 6.283185307179586f * floorf((acc + 3.14159265358979f) * 0.15915494309189535f);     // back to [-pi, pi)
+  }
+}
+
+// ---- inverse STFT frames: S [frames][1025] -> windowed frames [frames][2048]; one frame per warp -------------------------------
+// Z[k] = (X[k] + conj X[1024-k]) + i e^{2 pi i k/2048} (X[k] - conj X[1024-k]); irfft ignores Im of DC and Nyquist.
+__global__ void __launch_bounds__(256)
+pitch_istft_frames_kernel(const float2* __restrict__ S, float* __restrict__ frames, long long n_frames,
+                          const float2* __restrict__ tw1024, const float2* __restrict__ tw2048) {
+  pdl_enter();
+  extern __shared__ __align__(16) uint8_t pi_smem[];
+  float2 (*xs)[XS_PITCH] = reinterpret_cast<float2 (*)[XS_PITCH]>(pi_smem);
+  const int fr = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const long long g = (long long)blockIdx.x * FR + fr;
+  if (g >= n_frames) return;
+  const float2* X = S + g * NBIN;
+  float2 x[R];
+#pragma unroll
+  for (int r = 0; r < R; ++r) {
+    const int k = lane + 32 * r;
+    float2 a = __ldg(X + k), c = __ldg(X + NC - k);
+    if (k == 0) { a.y = 0.f; c.y = 0.f; }
+    const float2 e = make_float2(a.x + c.x, a.y - c.y);
+    const float2 o = cmul(make_float2(a.x - c.x, a.y + c.y), __ldg(tw2048 + k));
+    x[r] = make_float2(e.x - o.y, e.y + o.x);
+  }
+  fft_warp<+1, R>(x, tw1024, lane);
+  store_bitrev<R>(xs[fr], x, lane);
+  __syncwarp();
+  float2* out = reinterpret_cast<float2*>(frames + g * NFFT);
+  for (int n = lane; n < NC; n += 32) {
+    const float2 z = xs[fr][pidx<R>(n)];
+    out[n] = make_float2(z.x * (1.0f / NFFT) * hann2048(2 * n), z.y * (1.0f / NFFT) * hann2048(2 * n + 1));
+  }
+}
+
+// ---- overlap-add with librosa's `length`: ys_k[j] = OLA / window-sum-square at j + 1024 over the first tcap[k] frames (zero past
+// the overlap-added extent); item k at yoff[k], length round(L_k / rate_k) --------------------------------------------------------
+__global__ void pitch_ola_kernel(const float* __restrict__ frames, float* __restrict__ ys, const long long* __restrict__ fout,
+                                 const long long* __restrict__ yoff, const long long* __restrict__ tcap, int B) {
+  pdl_enter();
+  const long long total = __ldg(yoff + B);
+  for (long long g = blockIdx.x * (long long)blockDim.x + threadIdx.x; g < total; g += (long long)gridDim.x * blockDim.x) {
+    const int k = find_item(yoff, B, g);
+    const long long jj = g - __ldg(yoff + k) + NFFT / 2;
+    const float* fk = frames + __ldg(fout + k) * NFFT;
+    long long t = jj / HOP;
+    const long long tc = __ldg(tcap + k);
+    if (t > tc - 1) t = tc - 1;
+    float acc = 0.f, wss = 0.f;
+    for (; t >= 0 && jj - t * HOP < NFFT; --t) {
+      const int m = (int)(jj - t * HOP);
+      const float w = hann2048(m);
+      acc += __ldg(fk + t * NFFT + m);
+      wss = fmaf(w, w, wss);
+    }
+    ys[g] = wss > 1.17549435e-38f ? acc / wss : acc;
+  }
+}
+
+// ---- resample 16000/rate -> 16000 Hz + fix_length: out_k[j] = sum_i ys_k[i] h(i - j/rate) for j < nval[k], zero after ------------
+// h(d) = s * roll * sinc(s * roll * d) * I0(beta sqrt(1 - (s d / 64)^2)) / I0(beta), |d| <= 64 / s, s = min(1, rate); samples
+// outside [0, len) count as zero.  rate == 1 (n_steps 0) copies: librosa.resample returns its input when the rates are equal.
+__global__ void __launch_bounds__(256)
+pitch_resample_kernel(const float* __restrict__ ys, float* __restrict__ out, const long long* __restrict__ loff,
+                      const long long* __restrict__ yoff, const long long* __restrict__ nval, const double* __restrict__ rate, int B,
+                      float inv_i0_beta) {
+  pdl_enter();
+  const long long total = __ldg(loff + B);
+  for (long long g = blockIdx.x * (long long)blockDim.x + threadIdx.x; g < total; g += (long long)gridDim.x * blockDim.x) {
+    const int k = find_item(loff, B, g);
+    const long long j = g - __ldg(loff + k);
+    const float* src = ys + __ldg(yoff + k);
+    const long long len = __ldg(yoff + k + 1) - __ldg(yoff + k);
+    const double rt = __ldg(rate + k);
+    float acc = 0.f;
+    if (j < __ldg(nval + k)) {
+      if (rt == 1.0) {
+        acc = __ldg(src + j);
+      } else {
+        const double pos = (double)j / rt, sc = rt < 1.0 ? rt : 1.0, half = RS_ZEROS / sc;
+        const double i0d = floor(pos);
+        const long long ip = (long long)i0d;
+        const float f = (float)(pos - i0d);
+        long long lo = (long long)ceil(pos - half), hi = (long long)floor(pos + half);
+        if (lo < 0) lo = 0;
+        if (hi > len - 1) hi = len - 1;
+        const float cut = (float)(sc * RS_ROLLOFF), wscale = (float)(sc / RS_ZEROS);
+        for (long long i = lo; i <= hi; ++i) {
+          const float d = (float)(i - ip) - f;
+          const float u = d * wscale;
+          const float win = cyl_bessel_i0f((float)RS_BETA * sqrtf(fmaxf(0.f, 1.0f - u * u))) * inv_i0_beta;
+          const float z = cut * d;
+          const float sinc = z == 0.f ? 1.f : sinpif(z) / (3.14159265358979f * z);
+          acc = fmaf(__ldg(src + i), cut * sinc * win, acc);
+        }
+      }
+    }
+    out[g] = acc;
+  }
+}
+
+// ---- track mix: track[j] = sum over notes n covering j, in input order, of gain_n * src[src_off_n + j - onset_n] ---------------
+// a gather over track samples (one block per MIX_TILE samples) through the per-tile note lists, so the sum order is fixed.
+__global__ void __launch_bounds__(256)
+pitch_mix_kernel(const float* __restrict__ src, float* __restrict__ track, long long track_len, const int* __restrict__ tile_ptr,
+                 const int* __restrict__ tile_notes, const long long* __restrict__ src_off, const long long* __restrict__ len,
+                 const long long* __restrict__ onset, const float* __restrict__ gain) {
+  pdl_enter();
+  const int p0 = __ldg(tile_ptr + blockIdx.x), p1 = __ldg(tile_ptr + blockIdx.x + 1);
+  for (int q = threadIdx.x; q < MIX_TILE; q += blockDim.x) {
+    const long long j = (long long)blockIdx.x * MIX_TILE + q;
+    if (j >= track_len) break;
+    float acc = 0.f;
+    for (int p = p0; p < p1; ++p) {
+      const int n = __ldg(tile_notes + p);
+      const long long r = j - __ldg(onset + n);
+      if (r >= 0 && r < __ldg(len + n)) acc = fmaf(__ldg(gain + n), __ldg(src + __ldg(src_off + n) + r), acc);
+    }
+    track[j] = acc;
+  }
+}
+
+// I0(x) by its power series sum ((x/2)^k / k!)^2 (converged to double precision for the beta used here)
+double bessel_i0(double x) {
+  double term = 1.0, sum = 1.0;
+  for (int k = 1; k < 200 && term > 1e-17 * sum; ++k) {
+    term *= (x / (2.0 * k)) * (x / (2.0 * k));
+    sum += term;
+  }
+  return sum;
+}
+
+size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
+
+// Host-side plan of one batched pitch shift: the per-item metadata (uploaded as one block at the start of the workspace) and the
+// workspace carve-up.  Metadata: loff, fin, fout, yoff (B+1 prefix arrays each), tcap, nval (B each), as int64; rate (B) float64.
+struct PitchPlan {
+  std::vector<long long> meta;         // int64 arrays followed by the float64 rates (bit copies)
+  int B = 0;
+  size_t off_D = 0, off_S = 0, off_frames = 0, off_ys = 0, bytes = 0;
+  long long n_in_frames = 0, n_out_frames = 0, n_ys = 0, n_samples = 0;
+};
+
+int check_pitch_args(const long long* lengths, const double* n_steps, int B, const char* who) {
+  DS_REQUIRE(lengths && n_steps && B > 0, "%s: lengths and n_steps must be non-null and B > 0 (B = %d)", who, B);
+  for (int k = 0; k < B; ++k) {
+    DS_REQUIRE(lengths[k] > 0, "%s: item %d has length %lld (must be > 0)", who, k, lengths[k]);
+    DS_REQUIRE(std::isfinite(n_steps[k]) && std::fabs(n_steps[k]) <= 24.0, "%s: item %d has n_steps %g (must be finite, |n_steps| <= 24)",
+               who, k, n_steps[k]);
+  }
+  return DS_OK;
+}
+
+void make_plan(const long long* lengths, const double* n_steps, int B, PitchPlan& p) {
+  p.B = B;
+  const size_t n1 = (size_t)B + 1;
+  p.meta.assign(4 * n1 + 3 * (size_t)B, 0);
+  long long *loff = p.meta.data(), *fin = loff + n1, *fout = fin + n1, *yoff = fout + n1, *tcap = yoff + n1, *nval = tcap + B;
+  double* rate = reinterpret_cast<double*>(nval + B);
+  for (int k = 0; k < B; ++k) {
+    const long long L = lengths[k];
+    const double rt = std::exp2(-n_steps[k] / 12.0);
+    const long long T_in = 1 + L / HOP;
+    const long long T_out = (long long)std::ceil((double)T_in / rt);              // len(np.arange(0, T_in, rate))
+    const long long len = (long long)std::nearbyint((double)L / rt);             // round(L / rate), half to even like Python
+    long long cap = (long long)std::ceil((double)(len + NFFT) / HOP);            // librosa.istft: frames needed for `length`
+    if (cap > T_out) cap = T_out;
+    long long nv = L;
+    if (rt != 1.0) {
+      const long long n_out = (long long)std::ceil((double)len * rt);            // librosa.resample output length
+      if (n_out < nv) nv = n_out;
+    }
+    loff[k + 1] = loff[k] + L;
+    fin[k + 1] = fin[k] + T_in;
+    fout[k + 1] = fout[k] + T_out;
+    yoff[k + 1] = yoff[k] + len;
+    tcap[k] = cap;
+    nval[k] = nv;
+    rate[k] = rt;
+  }
+  p.n_samples = loff[B];
+  p.n_in_frames = fin[B];
+  p.n_out_frames = fout[B];
+  p.n_ys = yoff[B];
+  size_t o = align256(p.meta.size() * sizeof(long long));
+  p.off_D = o;      o = align256(o + (size_t)p.n_in_frames * NBIN * sizeof(float2));
+  p.off_S = o;      o = align256(o + (size_t)p.n_out_frames * NBIN * sizeof(float2));
+  p.off_frames = o; o = align256(o + (size_t)p.n_out_frames * NFFT * sizeof(float));
+  p.off_ys = o;     o = align256(o + (size_t)p.n_ys * sizeof(float));
+  p.bytes = o;
+}
+
+// Per-tile note lists of a mix: CSR over tiles of MIX_TILE track samples, notes in input order; followed by the per-note arrays.
+struct MixPlan {
+  std::vector<int> tile_ptr, tile_notes;
+  size_t off_notes = 0, off_src = 0, off_len = 0, off_onset = 0, off_gain = 0, bytes = 0;
+  int n_tiles = 0;
+};
+
+int check_mix_args(const long long* lengths, const long long* onsets, int K, long long track_len, const char* who) {
+  DS_REQUIRE(lengths && onsets && K > 0 && track_len > 0, "%s: lengths and onsets must be non-null, K > 0 and track_len > 0", who);
+  for (int n = 0; n < K; ++n) {
+    DS_REQUIRE(lengths[n] > 0, "%s: note %d has length %lld (must be > 0)", who, n, lengths[n]);
+    DS_REQUIRE(onsets[n] >= 0, "%s: note %d has onset %lld (must be >= 0)", who, n, onsets[n]);
+    DS_REQUIRE(onsets[n] + lengths[n] <= track_len, "%s: note %d ends at %lld, past the track length %lld", who, n,
+               onsets[n] + lengths[n], track_len);
+  }
+  return DS_OK;
+}
+
+void make_mix_plan(const long long* lengths, const long long* onsets, int K, long long track_len, MixPlan& p) {
+  p.n_tiles = (int)((track_len + MIX_TILE - 1) / MIX_TILE);
+  std::vector<int> count(p.n_tiles + 1, 0);
+  for (int n = 0; n < K; ++n)
+    for (long long t = onsets[n] / MIX_TILE; t <= (onsets[n] + lengths[n] - 1) / MIX_TILE; ++t) ++count[t + 1];
+  p.tile_ptr.assign(p.n_tiles + 1, 0);
+  for (int t = 0; t < p.n_tiles; ++t) p.tile_ptr[t + 1] = p.tile_ptr[t] + count[t + 1];
+  p.tile_notes.assign(p.tile_ptr[p.n_tiles], 0);
+  std::vector<int> fill(p.tile_ptr.begin(), p.tile_ptr.end() - 1);
+  for (int n = 0; n < K; ++n)                                 // ascending n: every tile's list is in input order
+    for (long long t = onsets[n] / MIX_TILE; t <= (onsets[n] + lengths[n] - 1) / MIX_TILE; ++t) p.tile_notes[fill[t]++] = n;
+  size_t o = align256(p.tile_ptr.size() * sizeof(int));
+  p.off_notes = o; o = align256(o + p.tile_notes.size() * sizeof(int));
+  p.off_src = o;   o = align256(o + (size_t)K * sizeof(long long));
+  p.off_len = o;   o = align256(o + (size_t)K * sizeof(long long));
+  p.off_onset = o; o = align256(o + (size_t)K * sizeof(long long));
+  p.off_gain = o;  o = align256(o + (size_t)K * sizeof(float));
+  p.bytes = o;
+}
+
+unsigned grid_for(long long n, int per_block) {
+  long long b = (n + per_block - 1) / per_block;
+  const long long cap = (long long)num_sms() * 32;
+  if (b > cap) b = cap;
+  return (unsigned)(b > 0 ? b : 1);
+}
+
+}  // namespace
+}  // namespace ds
+
+using namespace ds;
+
+extern "C" {
+
+int ds_pitch_shift_workspace(const long long* lengths, const double* n_steps, int B, long long* bytes, long long* stage_offsets) {
+  DS_REQUIRE(bytes, "ds_pitch_shift_workspace: bytes must be non-null");
+  int rc = check_pitch_args(lengths, n_steps, B, "ds_pitch_shift_workspace");
+  if (rc) return rc;
+  PitchPlan p;
+  make_plan(lengths, n_steps, B, p);
+  *bytes = (long long)p.bytes;
+  if (stage_offsets) {
+    stage_offsets[0] = (long long)p.off_D;
+    stage_offsets[1] = (long long)p.off_S;
+    stage_offsets[2] = (long long)p.off_frames;
+    stage_offsets[3] = (long long)p.off_ys;
+  }
+  return DS_OK;
+}
+
+int ds_pitch_shift(const float* d_in, float* d_out, const long long* lengths, const double* n_steps, int B, void* d_ws, long long ws_bytes,
+                   void* stream) {
+  DS_REQUIRE(d_in && d_out && d_ws, "ds_pitch_shift: d_in, d_out and d_ws must be non-null");
+  int rc = check_pitch_args(lengths, n_steps, B, "ds_pitch_shift");
+  if (rc) return rc;
+  PitchPlan p;
+  make_plan(lengths, n_steps, B, p);
+  DS_REQUIRE(ws_bytes >= (long long)p.bytes, "ds_pitch_shift: workspace of %lld bytes, %zu needed", ws_bytes, p.bytes);
+  float2 *tw512, *tw1024, *tw2048;
+  rc = get_twiddles((cudaStream_t)stream, &tw512, &tw1024, &tw2048);
+  if (rc) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  uint8_t* ws = (uint8_t*)d_ws;
+  const size_t n1 = (size_t)B + 1;
+  const long long* m = (const long long*)ws;
+  const long long *loff = m, *fin = loff + n1, *fout = fin + n1, *yoff = fout + n1, *tcap = yoff + n1, *nval = tcap + B;
+  const double* rate = (const double*)(nval + B);
+  float2* D = (float2*)(ws + p.off_D);
+  float2* S = (float2*)(ws + p.off_S);
+  float* frames = (float*)(ws + p.off_frames);
+  float* ys = (float*)(ws + p.off_ys);
+  // pageable source: the copy is staged before cudaMemcpyAsync returns, so the host plan may go out of scope
+  DS_CHECK_CUDA(cudaMemcpyAsync(ws, p.meta.data(), p.meta.size() * sizeof(long long), cudaMemcpyHostToDevice, st));
+  const size_t smem = FR * XS_PITCH * sizeof(float2);
+  DS_CHECK_CUDA(cudaFuncSetAttribute(pitch_stft_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  DS_CHECK_CUDA(cudaFuncSetAttribute(pitch_istft_frames_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  DS_CHECK_CUDA(launch_pdl(pitch_stft_kernel, dim3((unsigned)((p.n_in_frames + FR - 1) / FR)), dim3(256), smem, st, d_in, loff, fin, B, D,
+                           (const float2*)tw1024, (const float2*)tw2048));
+  DS_CHECK_CUDA(launch_pdl(pitch_vocoder_kernel, dim3((unsigned)(((long long)B * NBIN + 255) / 256)), dim3(256), (size_t)0, st,
+                           (const float2*)D, S, fin, fout, rate, B));
+  DS_CHECK_CUDA(launch_pdl(pitch_istft_frames_kernel, dim3((unsigned)((p.n_out_frames + FR - 1) / FR)), dim3(256), smem, st,
+                           (const float2*)S, frames, p.n_out_frames, (const float2*)tw1024, (const float2*)tw2048));
+  DS_CHECK_CUDA(launch_pdl(pitch_ola_kernel, dim3(grid_for(p.n_ys, 256)), dim3(256), (size_t)0, st, (const float*)frames, ys, fout, yoff,
+                           tcap, B));
+  DS_CHECK_CUDA(launch_pdl(pitch_resample_kernel, dim3(grid_for(p.n_samples, 256)), dim3(256), (size_t)0, st, (const float*)ys, d_out,
+                           loff, yoff, nval, rate, B, (float)(1.0 / bessel_i0(RS_BETA))));
+  DS_CHECK_CUDA(cudaGetLastError());
+  return DS_OK;
+}
+
+int ds_mix_track_workspace(const long long* lengths, const long long* onsets, int K, long long track_len, long long* bytes) {
+  DS_REQUIRE(bytes, "ds_mix_track_workspace: bytes must be non-null");
+  int rc = check_mix_args(lengths, onsets, K, track_len, "ds_mix_track_workspace");
+  if (rc) return rc;
+  MixPlan p;
+  make_mix_plan(lengths, onsets, K, track_len, p);
+  *bytes = (long long)p.bytes;
+  return DS_OK;
+}
+
+int ds_mix_track(const float* d_src, const long long* src_off, const long long* lengths, const long long* onsets, const float* gains, int K,
+                 float* d_track, long long track_len, void* d_ws, long long ws_bytes, void* stream) {
+  DS_REQUIRE(d_src && d_track && d_ws && src_off && gains, "ds_mix_track: d_src, d_track, d_ws, src_off and gains must be non-null");
+  int rc = check_mix_args(lengths, onsets, K, track_len, "ds_mix_track");
+  if (rc) return rc;
+  for (int n = 0; n < K; ++n) DS_REQUIRE(src_off[n] >= 0, "ds_mix_track: note %d has source offset %lld", n, src_off[n]);
+  MixPlan p;
+  make_mix_plan(lengths, onsets, K, track_len, p);
+  DS_REQUIRE(ws_bytes >= (long long)p.bytes, "ds_mix_track: workspace of %lld bytes, %zu needed", ws_bytes, p.bytes);
+  std::vector<uint8_t> host(p.bytes, 0);
+  memcpy(host.data(), p.tile_ptr.data(), p.tile_ptr.size() * sizeof(int));
+  memcpy(host.data() + p.off_notes, p.tile_notes.data(), p.tile_notes.size() * sizeof(int));
+  memcpy(host.data() + p.off_src, src_off, (size_t)K * sizeof(long long));
+  memcpy(host.data() + p.off_len, lengths, (size_t)K * sizeof(long long));
+  memcpy(host.data() + p.off_onset, onsets, (size_t)K * sizeof(long long));
+  memcpy(host.data() + p.off_gain, gains, (size_t)K * sizeof(float));
+  cudaStream_t st = (cudaStream_t)stream;
+  uint8_t* ws = (uint8_t*)d_ws;
+  DS_CHECK_CUDA(cudaMemcpyAsync(ws, host.data(), p.bytes, cudaMemcpyHostToDevice, st));
+  DS_CHECK_CUDA(launch_pdl(pitch_mix_kernel, dim3((unsigned)p.n_tiles), dim3(256), (size_t)0, st, d_src, d_track, track_len,
+                           (const int*)ws, (const int*)(ws + p.off_notes), (const long long*)(ws + p.off_src),
+                           (const long long*)(ws + p.off_len), (const long long*)(ws + p.off_onset), (const float*)(ws + p.off_gain)));
+  DS_CHECK_CUDA(cudaGetLastError());
+  return DS_OK;
+}
+
+}  // extern "C"

@@ -11,7 +11,7 @@ import torch
 
 from . import _lib, ops, weights as W
 from ._lib import check
-from .codec import adjust_audio_length, spectrogram_to_waveform, waveform_to_spectrogram
+from .codec import adjust_audio_length, shift_and_mix, spectrogram_to_waveform, waveform_to_spectrogram
 from .sampler import DiffSynthSampler
 from .unet import ConditionedUnet
 from .vqgan import VQGAN
@@ -23,6 +23,17 @@ class Timbres:
     quantized: torch.Tensor      # [B,4,128,W]
     spectrograms: torch.Tensor   # [B,3,512,4W]
     waveforms: torch.Tensor      # [B, 256*(4W-1)]
+
+
+@dataclass
+class TrackPlan:
+    durations: list              # distinct note durations (s), in order of first appearance
+    pairs: list                  # distinct (index into durations, semitones), in order of first appearance
+    note_pair: list              # per note: index into pairs
+    onsets: list                 # per note: onset in samples
+    gains: list                  # per note
+    lengths: list                # per note: samples of its waveform, 256 * (4 * width - 1)
+    track_len: int               # max(onset + length)
 
 
 class _Tail:
@@ -283,6 +294,47 @@ class TextToTimbre:
             for b, i in enumerate(idx):
                 out[i] = Timbres(t.latents[b:b + 1], t.quantized[b:b + 1], t.spectrograms[b:b + 1], t.waveforms[b:b + 1])
         return out
+
+    @staticmethod
+    def track_plan(notes, time_resolution: int = 256, vae_scale: int = 4, sample_rate: int = 16000) -> TrackPlan:
+        """Host side of render_track: notes ``(onset_sec, duration_sec, semitones, gain)`` -> the distinct durations and the distinct
+        (duration, semitones) pairs in order of first appearance, each note's pair, onsets in samples (round(onset * 16000)), note
+        lengths in samples and the track length."""
+        durations, pairs, note_pair, onsets, gains, lengths = [], [], [], [], [], []
+        for onset_sec, dur, semi, gain in notes:
+            dur, semi = float(dur), float(semi)
+            if dur not in durations:
+                durations.append(dur)
+            key = (durations.index(dur), semi)
+            if key not in pairs:
+                pairs.append(key)
+            note_pair.append(pairs.index(key))
+            onsets.append(int(round(float(onset_sec) * sample_rate)))
+            gains.append(float(gain))
+            lengths.append(256 * (4 * TextToTimbre.note_width(dur, time_resolution, vae_scale) - 1))
+            if onsets[-1] < 0:
+                raise ValueError(f"note onsets must be >= 0, got {onset_sec}")
+        track_len = max(o + n for o, n in zip(onsets, lengths))
+        return TrackPlan(durations, pairs, note_pair, onsets, gains, lengths, track_len)
+
+    @torch.no_grad()
+    def render_track(self, instrument_latent: torch.Tensor, condition: torch.Tensor, notes, sample_steps: int = 20,
+                     noising_strength: float = 1.0, attack: float = 0.5, before_release: float = 0.5, sampler: str = "ddim",
+                     time_resolution: int = 256, vae_scale: int = 4, noise_feeds=None) -> torch.Tensor:
+        """A note arrangement rendered on the device: what track_maker.DiffSynth does after its per-note closure.  ``notes`` is a
+        list of ``(onset_sec, duration_sec, semitones, gain)``.  One timbre is synthesised per distinct duration (synthesize_notes,
+        same keyword arguments; ``noise_feeds``: one per distinct duration, in order of first appearance), each distinct
+        (duration, semitones) pair is pitch-shifted once (librosa.effects.pitch_shift, track_maker.py:42) in one batched call, and
+        every note is placed at round(onset * 16000) with its gain and summed in one call (codec.shift_and_mix).  Returns the
+        fp32 track [max(onset + note length)]; no normalisation, no envelope."""
+        plan = self.track_plan(notes, time_resolution, vae_scale)
+        timbres = self.synthesize_notes(instrument_latent, condition, plan.durations, sample_steps=sample_steps,
+                                        noising_strength=noising_strength, attack=attack, before_release=before_release, sampler=sampler,
+                                        time_resolution=time_resolution, vae_scale=vae_scale, noise_feeds=noise_feeds)
+        sources = [timbres[d].waveforms[0] for d, _ in plan.pairs]
+        track = shift_and_mix(sources, [s for _, s in plan.pairs], plan.note_pair, plan.onsets, plan.gains)
+        assert track.numel() == plan.track_len
+        return track
 
 
 def shard_range(total: int, rank: int, world: int) -> Tuple[int, int]:

@@ -209,6 +209,30 @@ int ds_griffinlim_update(const float* d_rebuilt, float* d_tprev, float* d_spec, 
                          void* stream);
 
 /* ----------------------------------------------------------------------------------------
+ * Note arrangements (webUI/natural_language_guided_4/track_maker.py:42 after the per-note closure of track_maker.DiffSynth):
+ * every note is pitch-shifted, scaled, placed at its onset and summed into one track.  16 kHz throughout.  Host arrays
+ * (lengths, n_steps, onsets, offsets, gains) are read and checked before any device work, then uploaded into the workspace with
+ * one cudaMemcpyAsync, so these two calls cannot be captured in a graph.
+ * -------------------------------------------------------------------------------------- */
+/* librosa.effects.pitch_shift(y, sr=16000, n_steps=n_steps[k], bins_per_octave=12) for B items packed back to back in d_in
+   (item k: lengths[k] samples, fp32), written to d_out in the same layout: stft(n_fft 2048, hop 512, periodic Hann, centre zero
+   padding) -> librosa.phase_vocoder(rate = 2^(-n/12), hop 512) -> istft(length = round(L/rate)) -> resample from 16000/rate to
+   16000 Hz -> fix_length(L).  The resampler is a Kaiser-windowed sinc (resampy kaiser_best parameters), not librosa's default
+   soxr; n_steps == 0 skips it like librosa.resample.  |n_steps[k]| <= 24, finite.  d_ws: ds_pitch_shift_workspace bytes.  After the
+   call the workspace holds the stages at the byte offsets stage_offsets[0..3] (nullable): the STFTs (complex64 [sum T_in][1025],
+   T_in = 1 + L/512), the stretched spectra ([sum T_out][1025], T_out = ceil(T_in/rate)), the windowed iSTFT frames (fp32
+   [sum T_out][2048]) and the time-stretched signals (fp32, round(L/rate) samples each), all packed in item order. */
+int ds_pitch_shift_workspace(const long long* lengths, const double* n_steps, int B, long long* bytes, long long* stage_offsets);
+int ds_pitch_shift(const float* d_in, float* d_out, const long long* lengths, const double* n_steps, int B, void* d_ws, long long ws_bytes,
+                   void* stream);
+/* Track mix (track_maker.py's placement loop): d_track[j] = sum over notes n in input order, fp32, of
+   gains[n] * d_src[src_offsets[n] + j - onsets[n]] where 0 <= j - onsets[n] < lengths[n]; no normalisation, no envelope.  A gather
+   over track samples, bit-identical run to run.  Every onsets[n] + lengths[n] <= track_len.  d_ws: ds_mix_track_workspace bytes. */
+int ds_mix_track_workspace(const long long* lengths, const long long* onsets, int K, long long track_len, long long* bytes);
+int ds_mix_track(const float* d_src, const long long* src_offsets, const long long* lengths, const long long* onsets, const float* gains,
+                 int K, float* d_track, long long track_len, void* d_ws, long long ws_bytes, void* stream);
+
+/* ----------------------------------------------------------------------------------------
  * Image products of the decode glue (webUI/natural_language_guided_4/utils.py), batched:
  *   spectrogram_to_Gradio_image (:8-50, with tools.np_power_to_db tools.py:41-50) and phase_to_Gradio_image (:53-91)
  *   of |D| / angle(D) for D = depad_STFT(decode_stft(spec)) (:229-238): uint8 [B, 513, T, 3], flipped vertically;
