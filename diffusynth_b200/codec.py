@@ -31,7 +31,8 @@ def spectrogram_to_waveform(spec: torch.Tensor) -> torch.Tensor:
 
 def adjust_audio_length(audio, desired_length: int, original_sample_rate: Optional[int] = None, target_sample_rate: Optional[int] = None):
     """tools.adjust_audio_length (tools.py:126-151): resample when the rates differ, then crop or zero-pad the last axis.
-    Tensors stay tensors (the batched path of TextToTimbre.encode_audio), numpy arrays stay numpy arrays (drop-in use).
+    Tensors stay tensors, numpy arrays stay numpy arrays (drop-in use).  TextToTimbre.encode_audio resamples on the device instead
+    (``resample_packed``, the Kaiser-sinc filter of ``resample``).
     The reference resamples with ``librosa.core.resample`` (absent from this image, un-pinned in requirements.txt:3; its default
     ``res_type`` is a band-limited sinc method): here a polyphase FIR resampler (``scipy.signal.resample_poly``) on the host
     -- parity of this branch is UNPINNED by necessity; it is one clip of host-side preprocessing, not part of the device path."""
@@ -242,6 +243,87 @@ def shift_and_mix(sources, semitones, note_source, onsets, gains) -> torch.Tenso
     starts = np.concatenate([[0], np.cumsum(lengths)[:-1]]).astype(np.int64)
     idx = np.asarray(note_source, dtype=np.int64)
     return mix_track(shifted, starts[idx], np.asarray(lengths, dtype=np.int64)[idx], onsets, gains)
+
+
+# ---- sample-rate conversion (tools.adjust_audio_length's librosa.resample, tools.py:126-151) ----------------------------------
+MAX_RATE = 4194304                      # DS_RESAMPLE_MAX_RATE
+
+
+def _check_rates(sr, count: int, what: str) -> np.ndarray:
+    """Integer sample rates, one per item (a scalar is broadcast); an integral float is accepted."""
+    a = np.broadcast_to(np.asarray(sr, dtype=object), (count,))
+    out = np.empty(count, dtype=np.int64)
+    for k, v in enumerate(a):
+        if isinstance(v, (bool, np.bool_)) or not isinstance(v, (int, float, np.integer, np.floating)):
+            raise ValueError(f"{what} must be an integer sample rate, got {v!r}")
+        if not float(v).is_integer() or not 1 <= v <= MAX_RATE:
+            raise ValueError(f"{what} must be an integer sample rate in 1..{MAX_RATE}, got {v!r}")
+        out[k] = int(v)
+    return out
+
+
+def resample_length(length: int, orig_sr: int, target_sr: int) -> int:
+    """librosa.resample's output length: ceil(length * (target_sr / orig_sr)) in float64 (not integer ceil-division)."""
+    return int(np.ceil(length * (float(target_sr) / orig_sr)))
+
+
+@torch.no_grad()
+def resample_packed(packed: torch.Tensor, lengths, orig_sr, target_sr, out_lengths=None, normalize_peak: bool = False,
+                    out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Batched resampling of items packed back to back in one fp32 device tensor (item k: lengths[k] samples, from orig_sr[k] to
+    target_sr[k] Hz; rates: a scalar or one per item) by ds_resample.  Item k of the packed result has out_lengths[k] samples
+    (librosa's length when None): zero-padded or cropped.  ``normalize_peak`` first divides each item by its peak |x|
+    (at least 1e-12).  ``out``: an fp32 device tensor of the result's size to write into."""
+    lib = _lib.load()
+    L = np.ascontiguousarray(lengths, dtype=np.int64)
+    B = len(L)
+    o = _check_rates(orig_sr, B, "orig_sr")
+    t = _check_rates(target_sr, B, "target_sr")
+    ol = None if out_lengths is None else np.ascontiguousarray(np.broadcast_to(np.asarray(out_lengths, dtype=np.int64), (B,)))
+    packed = packed.float().contiguous()
+    assert packed.dim() == 1 and packed.numel() == int(L.sum()), "packed length must equal the sum of the item lengths"
+    ol_ptr = None if ol is None else ol.ctypes.data
+    nbytes = C.c_longlong(0)
+    check(lib.ds_resample_workspace(L.ctypes.data, o.ctypes.data, t.ctypes.data, ol_ptr, B, C.byref(nbytes)), "ds_resample_workspace")
+    total = int(ol.sum()) if ol is not None else sum(resample_length(n, a, b) for n, a, b in zip(L, o, t))
+    if out is None:
+        out = torch.empty((total,), dtype=torch.float32, device=packed.device)
+    assert out.dtype == torch.float32 and out.is_contiguous() and out.numel() == total and out.device == packed.device
+    ws = torch.empty((nbytes.value,), dtype=torch.uint8, device=packed.device)
+    check(lib.ds_resample(packed.data_ptr(), out.data_ptr(), L.ctypes.data, o.ctypes.data, t.ctypes.data, ol_ptr,
+                          1 if normalize_peak else 0, B, ws.data_ptr(), nbytes.value, ops._stream()), "ds_resample")
+    return out
+
+
+def resample(y, orig_sr, target_sr):
+    """On-device, batched ``librosa.resample(y, orig_sr=orig_sr, target_sr=target_sr, res_type="kaiser_best")`` (resampy's
+    Kaiser-windowed sinc, evaluated through a polyphase table; equal rates return the input).  ``y``: a [B, L] or [L] tensor /
+    numpy array, or a list of 1-D ones of different lengths; rates: integers, a scalar or one per item.  The output has librosa's
+    length ceil(L * target_sr / orig_sr) and the input's layout (numpy in, numpy out; fp32)."""
+    is_list = isinstance(y, (list, tuple))
+    if is_list:
+        items = list(y)
+        if not items or any(np.ndim(w) != 1 for w in items):
+            raise ValueError("expected a non-empty list of 1-D signals")
+    else:
+        if np.ndim(y) not in (1, 2):
+            raise ValueError("expected [B, L], [L] or a list of 1-D signals")
+        items = [y] if np.ndim(y) == 1 else [y[b] for b in range(y.shape[0])]
+    B = len(items)
+    o, t = _check_rates(orig_sr, B, "orig_sr"), _check_rates(target_sr, B, "target_sr")
+    if not is_list and np.ndim(y) == 2 and len(set(resample_length(y.shape[1], a, b) for a, b in zip(o, t))) > 1:
+        raise ValueError("a [B, L] input needs rates that give every row the same output length; pass a list instead")
+    is_np = isinstance(items[0], np.ndarray)
+    dev = _device() if is_np or not items[0].is_cuda else items[0].device
+    ts = [(torch.from_numpy(np.ascontiguousarray(w, dtype=np.float32)) if is_np else w).reshape(-1).to(dev, torch.float32) for w in items]
+    lengths = [x.numel() for x in ts]
+    res = resample_packed(torch.cat(ts), lengths, o, t)
+    n_out = [resample_length(n, a, b) for n, a, b in zip(lengths, o, t)]
+    if is_list:
+        parts = list(torch.split(res, n_out))
+        return [p.cpu().numpy() for p in parts] if is_np else parts
+    res = res.view(B, n_out[0]) if np.ndim(y) == 2 else res
+    return res.cpu().numpy() if is_np else res
 
 
 @torch.no_grad()

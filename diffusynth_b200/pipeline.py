@@ -11,7 +11,7 @@ import torch
 
 from . import _lib, ops, weights as W
 from ._lib import check
-from .codec import adjust_audio_length, shift_and_mix, spectrogram_to_waveform, waveform_to_spectrogram
+from .codec import SAMPLE_RATE, resample_packed, shift_and_mix, spectrogram_to_waveform, waveform_to_spectrogram
 from .sampler import DiffSynthSampler
 from .unet import ConditionedUnet
 from .vqgan import VQGAN
@@ -178,12 +178,24 @@ class TextToTimbre:
 
     # ---- timbre modification (sound2sound_with_text.py:47-269) -------------------------------------------------------
     @torch.no_grad()
-    def encode_audio(self, wave: torch.Tensor, width: int = 64) -> torch.Tensor:
-        """receive_upload_origin_audio's tensor path (:75-107): peak-normalise, crop/zero-pad to 256*(4w-1) samples, STFT
-        (1024/256, hann) -> pad_STFT -> encode_stft -> VQGAN encoder.  Returns the UN-quantised latent [B,4,128,w] (:107)."""
-        wave = wave.to(self.device, torch.float32)
-        wave = wave / wave.abs().amax(dim=-1, keepdim=True).clamp_min(1e-12)              # :75
-        wave = adjust_audio_length(wave, 256 * (4 * width - 1))                            # :80-82
+    def encode_audio(self, wave, width: int = 64, sample_rate=16000) -> torch.Tensor:
+        """receive_upload_origin_audio's tensor path (:75-107): peak-normalise, resample to 16 kHz and crop/zero-pad to
+        256*(4w-1) samples (adjust_audio_length, :80-82), STFT (1024/256, hann) -> pad_STFT -> encode_stft -> VQGAN encoder.
+        ``wave``: a [B, L] tensor / array, or a list of 1-D clips of different lengths; ``sample_rate``: an integer, or one per
+        clip.  Normalisation, resampling and the length adjustment are one ds_resample call writing the STFT's input (a 16 kHz clip
+        is copied).  Returns the UN-quantised latent [B,4,128,w] (:107)."""
+        if isinstance(wave, (list, tuple)):
+            clips = [torch.as_tensor(w) for w in wave]
+            if not clips or any(c.dim() != 1 for c in clips):
+                raise ValueError("expected a non-empty list of 1-D clips")
+            packed, lengths = torch.cat([c.to(self.device, torch.float32) for c in clips]), [c.numel() for c in clips]
+        else:
+            wave = torch.as_tensor(wave)
+            if wave.dim() != 2:
+                raise ValueError("expected a [B, L] batch or a list of 1-D clips")
+            packed, lengths = wave.to(self.device, torch.float32).reshape(-1), [wave.shape[1]] * wave.shape[0]
+        B, n = len(lengths), 256 * (4 * width - 1)
+        wave = resample_packed(packed, lengths, sample_rate, SAMPLE_RATE, out_lengths=n, normalize_peak=True).view(B, n)   # :75-82
         # pad_STFT(D) is called with its default time_resolution = 256 frames and never crops (tools.py:170-182): clips of
         # <= 3 s (width <= 64) always encode to a 64-column latent, longer ones to ``width`` columns
         spec = waveform_to_spectrogram(wave, time_resolution=max(256, 4 * width))          # :85-94

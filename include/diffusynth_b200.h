@@ -233,6 +233,26 @@ int ds_mix_track(const float* d_src, const long long* src_offsets, const long lo
                  int K, float* d_track, long long track_len, void* d_ws, long long ws_bytes, void* stream);
 
 /* ----------------------------------------------------------------------------------------
+ * Sample-rate conversion of uploaded audio (tools.adjust_audio_length, tools.py:126-151, as sound2sound_with_text.py:75-82 calls
+ * it): librosa.resample(x, orig_sr=sr_in[k], target_sr=sr_out[k], res_type="kaiser_best") for B items packed back to back in d_in
+ * (item k: lengths[k] samples, fp32), each written to d_out (packed, item k: out_lengths[k] samples, or librosa's length
+ * ceil(lengths[k] * (sr_out[k] / sr_in[k])) evaluated in float64 when out_lengths is NULL): zero past librosa's length, cropped
+ * below it (fix_length fused).  out_k[j] = sum_i xn_k[i] h(i - j * sr_in/sr_out) with pitch.cu's filter (resampy kaiser_best
+ * parameters, not librosa's default soxr); equal rates copy.  normalize_peak != 0 first divides item k by max(max|x_k|, 1e-12)
+ * (IEEE division), as the upload handler does.  Integer rates in 1..DS_RESAMPLE_MAX_RATE and lengths in 1..DS_RESAMPLE_MAX_LENGTH,
+ * so that j * (sr_in / gcd) stays in int64.  Pairs whose polyphase table has more than 2^20 coefficients (e.g. 44101 -> 16000) or
+ * whose staged window is too large evaluate the same coefficients per tap, with bit-identical results; DS_RESAMPLE_DIRECT=1 in
+ * the environment makes every pair do so (A/B timing).  Each output sums its taps in ascending input order: an item's result
+ * does not depend on the rest of the batch.  Host arrays are checked before any device work and uploaded with one
+ * cudaMemcpyAsync; 2 launches, 3 with normalize_peak, whatever B.  d_ws: ds_resample_workspace bytes. */
+#define DS_RESAMPLE_MAX_RATE 4194304LL
+#define DS_RESAMPLE_MAX_LENGTH 1099511627776LL
+int ds_resample_workspace(const long long* lengths, const long long* sr_in, const long long* sr_out, const long long* out_lengths, int B,
+                          long long* bytes);
+int ds_resample(const float* d_in, float* d_out, const long long* lengths, const long long* sr_in, const long long* sr_out,
+                const long long* out_lengths, int normalize_peak, int B, void* d_ws, long long ws_bytes, void* stream);
+
+/* ----------------------------------------------------------------------------------------
  * Image products of the decode glue (webUI/natural_language_guided_4/utils.py), batched:
  *   spectrogram_to_Gradio_image (:8-50, with tools.np_power_to_db tools.py:41-50) and phase_to_Gradio_image (:53-91)
  *   of |D| / angle(D) for D = depad_STFT(decode_stft(spec)) (:229-238): uint8 [B, 513, T, 3], flipped vertically;
