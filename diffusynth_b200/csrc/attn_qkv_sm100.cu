@@ -1,10 +1,12 @@
 // Fused  PreNorm -> to_qkv -> (softmax_d(q) * scale,  online softmax_n(k),  partial context  S = P^T V)  for the U-Net's
 // LinearCrossAttentionAdd / LinearCrossAttention (model/diffusion_components.py:148-151,263,271-289 and :171-207):
 // the 1x1 to_qkv convolution runs on tcgen05 (TMA-fed, TMEM accumulator 128 pixels x 192 channels of a head pair) and its epilogue keeps k
-// and v on chip -- they are never written to HBM: per 128-pixel tile the epilogue turns k into P = exp(k - m) (one reference m
-// per head and partial; softmax over n is shift invariant per row, so any common m is exact), stages P and V as bf16 in shared
+// and v on chip -- they are never written to HBM: per 128-pixel tile the epilogue turns k into P = exp(k - m[d]) (softmax over n is
+// shift invariant per row, so any m[d] common to the pixels of a partial is exact), stages P and V as bf16 in shared
 // memory and contracts them over the pixels with warp-level MMAs into S[d][e] (+ Z[d] = sum_n P through a column of ones);
 // q is soft-maxed over its 32 head channels in registers and written as the only per-pixel output (q').
+// The stabiliser is chosen per row d of the partial (see the epilogue), so no row can lose all of its pixels to underflow and no
+// later tile can overflow P.
 // One partial (S[32][32], Z[32], m[32]) per (sample, head, 512-pixel chunk) leaves the kernel in the format
 // attn_reduce_kernel / attn_fold_kernel already consume (ds_attn_finalize).  Replaces a to_qkv launch (which wrote 384
 // channels per pixel) and an attn_ctx_partial launch (which read them back).
@@ -34,7 +36,13 @@ static constexpr int AQ_B_BYTES = AQ_PN * AQ_BK * 2;      // 12 KB
 static constexpr int AQ_STAGE_BYTES = AQ_A_BYTES + AQ_B_BYTES;
 static constexpr int AQ_PITCH = 2 * 2 * AQ_DH + 16;       // bytes per staged P / V row (2 heads): 8 rows x 16 B hit 8 different bank groups
 static constexpr int AQ_PART = AQ_DH * AQ_DH + 2 * AQ_DH;
-static constexpr int AQ_SMEM = 1024 + AQ_STAGES * AQ_STAGE_BYTES + 2 * AQ_TILE * AQ_PITCH + AQ_PN * 4 + 256;
+static constexpr int AQ_SMEM = 1024 + AQ_STAGES * AQ_STAGE_BYTES + 2 * AQ_TILE * AQ_PITCH + AQ_PN * 4 + 256 + 7 * 2 * AQ_DH * 4;
+// Stabiliser bounds (log2 units, see the epilogue).  A row whose first-tile maximum lies more than AQ_ROW_LOW below its head's
+// takes its own stabiliser: under the head's, its largest P would be < 2^-100 and all of them could flush to 0 (ex2.approx.ftz
+// ends at 2^-126).  A later tile in which some P would exceed 2^AQ_RESCALE raises the stabiliser and rescales S and Z: P <= 2^96,
+// 512 of them times |v| < 2^22 stay inside fp32 / bf16.
+static constexpr float AQ_ROW_LOW = 100.f;
+static constexpr float AQ_RESCALE = 96.f;
 
 struct AttnQkvDev {
   int N, npix, C, num_kb, x_batch_mod, chunks, items;
@@ -65,6 +73,31 @@ __device__ __forceinline__ uint32_t pack_q(float lo, float hi) {
   return r;
 #endif
 }
+// Column maxima of a warp's 32 x 32 block (lane = pixel row, k[j] = column j): a butterfly that halves the columns a lane keeps at
+// every step (16 + 8 + 4 + 2 + 1 shuffles); lane l returns the maximum of column l over the lanes with `valid`.
+__device__ __forceinline__ float col_max32(const uint32_t (&k)[32], bool valid, int lane) {
+  float t[16];
+  const bool up16 = (lane & 16) != 0;
+#pragma unroll
+  for (int j = 0; j < 16; ++j) {
+    const float lo = valid ? __uint_as_float(k[j]) : -INFINITY, hi = valid ? __uint_as_float(k[j + 16]) : -INFINITY;
+    t[j] = fmaxf(up16 ? hi : lo, __shfl_xor_sync(0xffffffffu, up16 ? lo : hi, 16));
+  }
+#pragma unroll
+  for (int s = 8; s >= 1; s >>= 1) {
+    const bool up = (lane & s) != 0;
+#pragma unroll
+    for (int j = 0; j < s; ++j) t[j] = fmaxf(up ? t[j + s] : t[j], __shfl_xor_sync(0xffffffffu, up ? t[j] : t[j + s], s));
+  }
+  return t[0];
+}
+// named barrier that also returns whether any participating thread passed `v`
+__device__ __forceinline__ bool bar_red_or(int id, int nthreads, bool v) {
+  uint32_t r;
+  asm volatile("{\n\t.reg .pred p, q;\n\tsetp.ne.u32 p, %1, 0;\n\tbar.red.or.pred q, %2, %3, p;\n\tselp.u32 %0, 1, 0, q;\n\t}"
+               : "=r"(r) : "r"((uint32_t)v), "r"(id), "r"(nthreads) : "memory");
+  return r != 0;
+}
 __device__ __forceinline__ void sts_128(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
   asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
 }
@@ -82,7 +115,11 @@ attn_qkv_ctx_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
   uint64_t* tmem_full = empty_bar + AQ_STAGES;
   uint64_t* tmem_empty = tmem_full + 1;
   uint32_t* tmem_base_smem = reinterpret_cast<uint32_t*>(tmem_empty + 1);
-  float* s_wmax = reinterpret_cast<float*>(tmem_base_smem + 2);            // [4 lane groups][2 heads]: per-warp maxima of an item's first tile
+  // stabiliser of the item's 64 k rows (2 heads x 32 d, log2 units): column maxima per epilogue warp, m, -mb, and a rescale step
+  float* s_red = reinterpret_cast<float*>(tmem_base_smem + 4);             // [4 lane groups][64] (16-byte aligned: s_nm / s_dl are read as float4)
+  float* s_m = s_red + 4 * 2 * AQ_DH;                                      // [64] m[d]
+  float* s_nm = s_m + 2 * AQ_DH;                                           // [64] -mb[d]  (P = exp2(rl2 acc + s_nm), m = mb + tk)
+  float* s_dl = s_nm + 2 * AQ_DH;                                          // [64] increase of m in a rescaling tile
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   if (warp == 0 && lane == 0) { prefetch_tmap(&map_a); prefetch_tmap(&map_b); }
@@ -208,17 +245,19 @@ attn_qkv_ctx_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
         if (P.sbias != nullptr) t += __ldg(P.sbias + (size_t)n * P.sbias_stride + col);
         s_t[l] = l < 4 * AQ_DH ? t * kLog2e : t;
       }
-      // Stabiliser of the exponentials, one per head (log2 domain, of the bare product rl2 * acc): soft-max over n is shift invariant
-      // per row d, so ANY reference that is the same for every pixel of this partial is exact; the first tile of the item measures
-      // its own maximum and the later tiles keep it (P = exp2(rl2 acc - mh) may exceed 1 there: bf16 / fp32 have the exponent range).
-      // The per-column constant tk[d] never enters the inner loop: exp2(k - (mh + tk[d])) = exp2(rl2 acc - mh), so the partial
-      // simply reports m[d] = mh + tk[d].
-      float mh[2] = {0.f, 0.f};
+      // Stabiliser of the exponentials, one per row d of the partial (log2 domain, of the bare product rl2 acc; the per-row constant
+      // tk[d] -- bias, label key, GroupNorm mean fold -- never enters the exponent and is reported through m).  Soft-max over n is
+      // shift invariant per row, so any value that is the same for every pixel of the partial is exact.  A row takes its head's
+      // maximum over the valid pixels of the item's first tile, mh, unless its own first-tile maximum r[d] lies more than AQ_ROW_LOW
+      // below mh (a block input with a large mean-to-std ratio spreads the rows of a head apart by rl2 mean sum_c W'[d,c]); such a
+      // row takes r[d], so its largest pixel gives P = 1 and Z[d] >= 1.  Rows within range keep exactly the head value, so their
+      // P, S, Z and m are bit-identical to a per-head stabiliser.  A later tile in which some P would exceed 2^AQ_RESCALE raises
+      // the row's stabiliser to that tile's maximum and rescales S and Z, as attn_ctx_partial_kernel does.
       float c[4][4], cz[4];
 #pragma unroll
       for (int i = 0; i < 4; ++i) { cz[i] = 0.f; for (int j = 0; j < 4; ++j) c[i][j] = 0.f; }
       umma::named_bar_sync(2, 128);                              // s_t visible; the previous item's staging reads are done
-      const float tk_d = lane < 16 ? s_t[2 * AQ_DH + hl * AQ_DH + mt * 16 + lane] : 0.f;      // (s_t is rewritten by the next item's prologue)
+      const uint32_t nm_s = smem_u32(s_nm), dl_s = smem_u32(s_dl);
 
       const int nt = tiles_of(chunk);
       for (int sub = 0; sub < nt; ++sub) {
@@ -226,7 +265,8 @@ attn_qkv_ctx_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
         const bool valid = p0 + row < P.npix;                    // (false only in the ragged last tile of a sample)
         mbar_wait_warp(tmem_full, acc_phase);
         umma::fence_after();
-        // ---- k (columns 64..127) -> P = exp2(rl2 acc - mh) as bf16 rows ----
+        // ---- k (columns 64..127) -> P = exp2(rl2 acc - mb[d]) as bf16 rows ----
+        bool rescale;
         {
           uint32_t k0[32], k1[32];
           umma::ld_32x32b_x32(t_row + 64u, k0);
@@ -234,20 +274,80 @@ attn_qkv_ctx_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
           umma::ld_wait32(k0);
           umma::ld_wait32(k1);
           if (sub == 0) {
-            // first tile: maximum of the accumulator per head over the tile's pixels (rl2 > 0: max(rl2 acc) = rl2 max(acc))
-            float mx0 = -INFINITY, mx1 = -INFINITY;
-#pragma unroll
-            for (int j = 0; j < 32; ++j) { mx0 = fmaxf(mx0, __uint_as_float(k0[j])); mx1 = fmaxf(mx1, __uint_as_float(k1[j])); }
-            mx0 = warp_max(valid ? mx0 : -INFINITY);
-            mx1 = warp_max(valid ? mx1 : -INFINITY);
-            if (lane < 2) s_wmax[ew * 2 + lane] = lane == 0 ? mx0 : mx1;
+            // first tile: row maxima r[d] of acc (rl2 > 0: max(rl2 acc) = rl2 max(acc)); warps 4 and 5 (etid < 64) hold head 0 and
+            // head 1 of the pair, lane = d, so the head maximum is a warp maximum
+            const float r0 = col_max32(k0, valid, lane), r1 = col_max32(k1, valid, lane);
+            s_red[ew * 64 + lane] = r0;
+            s_red[ew * 64 + 32 + lane] = r1;
             umma::named_bar_sync(1, 128);
-            mh[0] = rl2 * fmaxf(fmaxf(s_wmax[0], s_wmax[2]), fmaxf(s_wmax[4], s_wmax[6]));
-            mh[1] = rl2 * fmaxf(fmaxf(s_wmax[1], s_wmax[3]), fmaxf(s_wmax[5], s_wmax[7]));
+            if (etid < 2 * AQ_DH) {
+              const float mx = fmaxf(fmaxf(s_red[etid], s_red[64 + etid]), fmaxf(s_red[128 + etid], s_red[192 + etid]));
+              const float mh = rl2 * warp_max(mx), mr = rl2 * mx;
+              const float mb = mr < mh - AQ_ROW_LOW ? mr : mh;
+              s_m[etid] = mb + s_t[2 * AQ_DH + etid];               // m[d] = mb[d] + tk[d]
+              s_nm[etid] = -mb;
+              s_dl[etid] = 0.f;
+            }
+            umma::named_bar_sync(1, 128);
+          }
+          // e = rl2 acc - mb in place (log2 of P), and this pixel's largest e
+          float emax = -INFINITY;
+#pragma unroll
+          for (int hh = 0; hh < 2; ++hh) {
+#pragma unroll
+            for (int j4 = 0; j4 < 8; ++j4) {
+              const float4 a = lds4(nm_s + (uint32_t)(hh * 32 + 4 * j4) * 4u);
+              const float na[4] = {a.x, a.y, a.z, a.w};
+#pragma unroll
+              for (int i = 0; i < 4; ++i) {
+                uint32_t& r = hh == 0 ? k0[4 * j4 + i] : k1[4 * j4 + i];
+                const float e = fmaf(__uint_as_float(r), rl2, na[i]);
+                emax = fmaxf(emax, e);
+                r = __float_as_uint(e);
+              }
+            }
+          }
+          rescale = sub > 0 && bar_red_or(1, 128, valid && emax > AQ_RESCALE);
+          if (rescale) {
+            // rare: some row of this tile rose more than AQ_RESCALE above its stabiliser -> raise m[d] by the tile's excess
+            // max(0, max_pix e[d]): the maximum of positive floats is the maximum of their bit patterns (s_dl is 0 here)
+            if (valid) {
+#pragma unroll
+              for (int j = 0; j < 64; ++j) {
+                const float e = __uint_as_float(j < 32 ? k0[j] : k1[j - 32]);
+                if (e > 0.f) atomicMax(reinterpret_cast<int*>(s_dl) + j, __float_as_int(e));
+              }
+            }
+            umma::named_bar_sync(1, 128);
+            if (etid < 2 * AQ_DH) {
+              const float dl = s_dl[etid];
+              s_m[etid] += dl;
+              s_nm[etid] -= dl;
+            }
+#pragma unroll
+            for (int hh = 0; hh < 2; ++hh) {
+#pragma unroll
+              for (int j4 = 0; j4 < 8; ++j4) {
+                const float4 a = lds4(dl_s + (uint32_t)(hh * 32 + 4 * j4) * 4u);
+                const float da[4] = {a.x, a.y, a.z, a.w};
+#pragma unroll
+                for (int i = 0; i < 4; ++i) {
+                  uint32_t& r = hh == 0 ? k0[4 * j4 + i] : k1[4 * j4 + i];
+                  r = __float_as_uint(__uint_as_float(r) - da[i]);
+                }
+              }
+            }
+            // S and Z so far were taken against the old m: rows d = 16 mt + g and + 8 of head hl (this thread's accumulators)
+            const int g = lane >> 2;
+            float sl, sh;
+            asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(sl) : "f"(-s_dl[hl * AQ_DH + mt * 16 + g]));
+            asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(sh) : "f"(-s_dl[hl * AQ_DH + mt * 16 + g + 8]));
+#pragma unroll
+            for (int i = 0; i < 4; ++i) { c[i][0] *= sl; c[i][1] *= sl; c[i][2] *= sh; c[i][3] *= sh; }
+            cz[0] *= sl; cz[1] *= sl; cz[2] *= sh; cz[3] *= sh;
           }
 #pragma unroll
           for (int hh = 0; hh < 2; ++hh) {
-            const float nm = -mh[hh];
 #pragma unroll
             for (int q8 = 0; q8 < 4; ++q8) {
               uint32_t o[4];
@@ -255,8 +355,8 @@ attn_qkv_ctx_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
               for (int j = 0; j < 4; ++j) {
                 const uint32_t r0 = hh == 0 ? k0[q8 * 8 + 2 * j] : k1[q8 * 8 + 2 * j], r1 = hh == 0 ? k0[q8 * 8 + 2 * j + 1] : k1[q8 * 8 + 2 * j + 1];
                 float e0, e1;
-                asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e0) : "f"(fmaf(__uint_as_float(r0), rl2, nm)));
-                asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e1) : "f"(fmaf(__uint_as_float(r1), rl2, nm)));
+                asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e0) : "f"(__uint_as_float(r0)));
+                asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e1) : "f"(__uint_as_float(r1)));
                 o[j] = valid ? pack_bf16(e0, e1) : 0u;
               }
               sts_128(sp_row + (uint32_t)(hh * 64 + q8 * 16), o[0], o[1], o[2], o[3]);
@@ -333,6 +433,7 @@ attn_qkv_ctx_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
           }
         }
         umma::named_bar_sync(2, 128);                            // P and V of this tile are staged
+        if (rescale && etid < 2 * AQ_DH) s_dl[etid] = 0.f;       // (every read of this tile's step is behind that barrier)
 
         // ---- context: S[d][e] += sum_pix P[pix][d] V[pix][e] (and Z[d] through a column of ones), head hl of the pair, d rows 16*mt.. ----
         {
@@ -355,7 +456,7 @@ attn_qkv_ctx_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
         umma::named_bar_sync(2, 128);                            // every warp is past its context MMAs: the staging rows are free
       }
       // ---- one partial per (sample, head, chunk): S rows d = 16 mt + {g, g + 8}, Z from the ones column,
-      //      m[d] = (mh + tk[d]) ln 2 in natural-log units as attn_reduce_kernel expects ----
+      //      m[d] in natural-log units as attn_reduce_kernel expects ----
       {
         float* po = P.part + (((size_t)n * AQ_HEADS + hp * 2 + hl) * P.chunks + chunk) * AQ_PART;
         const int g = lane >> 2, q = lane & 3;
@@ -366,7 +467,7 @@ attn_qkv_ctx_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
           *reinterpret_cast<float2*>(po + (d + 8) * AQ_DH + nt8 * 8 + q * 2) = make_float2(c[nt8][2], c[nt8][3]);
         }
         if (q == 0) { po[AQ_DH * AQ_DH + d] = cz[0]; po[AQ_DH * AQ_DH + d + 8] = cz[2]; }
-        if (lane < 16) po[AQ_DH * AQ_DH + AQ_DH + mt * 16 + lane] = (mh[hl] + tk_d) * kLn2;
+        if (lane < 16) po[AQ_DH * AQ_DH + AQ_DH + mt * 16 + lane] = s_m[hl * AQ_DH + mt * 16 + lane] * kLn2;
       }
     }
   }
