@@ -326,6 +326,94 @@ def resample(y, orig_sr, target_sr):
     return res.cpu().numpy() if is_np else res
 
 
+# ---- mask zoom (scipy.ndimage.zoom of the inpainting-with-text mask to the latent grid, inpaint_with_text.py) --------------------
+MAX_ZOOM_DIM = 16384                    # DS_MASK_ZOOM_MAX_DIM
+
+
+def _shapes(shapes, count: int, what: str) -> np.ndarray:
+    """[count, 2] int64 from one (rows, cols) pair or one pair per item, every dimension in 1..MAX_ZOOM_DIM."""
+    a = np.asarray(shapes, dtype=np.int64)
+    if a.shape == (2,):
+        a = np.broadcast_to(a, (count, 2))
+    if a.shape != (count, 2):
+        raise ValueError(f"{what} must be one (rows, cols) pair or one per item, got shape {a.shape}")
+    if (a < 1).any() or (a > MAX_ZOOM_DIM).any():
+        raise ValueError(f"every dimension of {what} must be in 1..{MAX_ZOOM_DIM}, got {a.tolist()}")
+    return np.ascontiguousarray(a)
+
+
+@torch.no_grad()
+def zoom_packed(packed: torch.Tensor, in_shapes, out_shapes, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Batched ``scipy.ndimage.zoom`` (order 3, mode 'constant', prefilter, grid_mode False) of 2-D items packed back to back in
+    one fp32 device tensor (item k: in_shapes[k] = (H, W), row-major) to out_shapes[k] = (h, w) (one pair, or one per item) by
+    ds_mask_zoom, computed in float64 and rounded to fp32.  ``out``: a contiguous fp32 device tensor of the result's size to
+    write into (any shape); the packed result otherwise."""
+    lib = _lib.load()
+    ins = np.asarray(in_shapes, dtype=np.int64).reshape(-1, 2)
+    B = len(ins)
+    ins = _shapes(ins, B, "in_shapes")
+    outs = _shapes(out_shapes, B, "out_shapes")
+    packed = packed.float().contiguous()
+    assert packed.dim() == 1 and packed.numel() == int((ins[:, 0] * ins[:, 1]).sum()), "packed length must equal the sum of H * W"
+    total = int((outs[:, 0] * outs[:, 1]).sum())
+    if out is None:
+        out = torch.empty((total,), dtype=torch.float32, device=packed.device)
+    assert out.dtype == torch.float32 and out.is_contiguous() and out.numel() == total and out.device == packed.device
+    nbytes = C.c_longlong(0)
+    check(lib.ds_mask_zoom_workspace(ins.ctypes.data, outs.ctypes.data, B, C.byref(nbytes)), "ds_mask_zoom_workspace")
+    ws = torch.empty((nbytes.value,), dtype=torch.uint8, device=packed.device)
+    check(lib.ds_mask_zoom(packed.data_ptr(), out.data_ptr(), ins.ctypes.data, outs.ctypes.data, B, ws.data_ptr(), nbytes.value,
+                           ops._stream()), "ds_mask_zoom")
+    return out
+
+
+def zoom(input, zoom, output=None, order=3, mode="constant", cval=0.0, prefilter=True, *, grid_mode=False):
+    """On-device, batched ``scipy.ndimage.zoom(input, zoom)`` for 2-D data with scipy's defaults; any other keyword value raises
+    NotImplementedError.  ``input``: a [H, W] or [B, H, W] tensor / numpy array (B items of one shape), or a list of 2-D ones of
+    different shapes; ``zoom``: a scalar or a (rows, cols) pair applied to every item, or for a list one per item.  Each item is
+    ``round(H * zoom_rows) x round(W * zoom_cols)`` as in scipy, and the result has the input's layout (numpy in, numpy out; fp32)."""
+    if output is not None or order != 3 or mode != "constant" or cval != 0.0 or prefilter is not True or grid_mode is not False:
+        raise NotImplementedError("only scipy.ndimage.zoom's defaults (order=3, mode='constant', cval=0, prefilter=True, "
+                                  "grid_mode=False, no output array) are implemented")
+    is_list = isinstance(input, (list, tuple))
+    if is_list:
+        items = list(input)
+        if any(np.ndim(a) != 2 for a in items):
+            raise ValueError("expected a list of 2-D arrays")
+    else:
+        if np.ndim(input) not in (2, 3):
+            raise ValueError("expected a [H, W] or [B, H, W] array, or a list of 2-D arrays")
+        items = [input] if np.ndim(input) == 2 else [input[b] for b in range(input.shape[0])]
+    B = len(items)
+    if B == 0:
+        raise ValueError("nothing to zoom: the batch is empty")
+    z = np.asarray(zoom, dtype=np.float64)
+    if z.ndim == 0:
+        z = np.full((B, 2), float(z))
+    elif z.shape == (2,):
+        z = np.broadcast_to(z, (B, 2))
+    elif is_list and z.shape == (B,):
+        z = np.repeat(z[:, None], 2, axis=1)
+    elif not (is_list and z.shape == (B, 2)):
+        raise ValueError(f"zoom must be a scalar or a (rows, cols) pair{', or one per item' if is_list else ''}, got {zoom!r}")
+    if not np.all(np.isfinite(z)) or (z <= 0).any():
+        raise ValueError(f"zoom factors must be finite and positive, got {zoom!r}")
+    ins = [tuple(int(n) for n in np.shape(a)) for a in items]
+    outs = [tuple(int(round(n * f)) for n, f in zip(s, zk)) for s, zk in zip(ins, z)]        # scipy: round(n * zoom), Python's round
+    in_shapes, out_shapes = _shapes(ins, B, "the input shape"), _shapes(outs, B, "the output shape")
+    is_np = isinstance(items[0], np.ndarray)
+    dev = _device() if is_np or not items[0].is_cuda else items[0].device
+    ts = [(torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32)) if is_np else a).reshape(-1).to(dev, torch.float32)
+          for a in items]
+    res = zoom_packed(torch.cat(ts), in_shapes, out_shapes)
+    sizes = [h * w for h, w in outs]
+    if is_list:
+        parts = [p.view(s) for p, s in zip(torch.split(res, sizes), outs)]
+        return [p.cpu().numpy() for p in parts] if is_np else parts
+    res = res.view(outs[0]) if np.ndim(input) == 2 else res.view((B,) + outs[0])
+    return res.cpu().numpy() if is_np else res
+
+
 @torch.no_grad()
 def spectrogram_images(spec: torch.Tensor):
     """[B,3,512,T] fp32 spectral representation -> (dB-magnitude image, phase image), uint8 [B,513,T,3] each: what

@@ -11,7 +11,7 @@ import torch
 
 from . import _lib, ops, weights as W
 from ._lib import check
-from .codec import SAMPLE_RATE, resample_packed, shift_and_mix, spectrogram_to_waveform, waveform_to_spectrogram
+from .codec import SAMPLE_RATE, resample_packed, shift_and_mix, spectrogram_to_waveform, waveform_to_spectrogram, zoom_packed
 from .sampler import DiffSynthSampler
 from .unet import ConditionedUnet
 from .vqgan import VQGAN
@@ -229,6 +229,63 @@ class TextToTimbre:
         s.graph_tail, s.final_only = (self._tail_factory if decode else None), True
         imgs, _ = s.img_guided_sample(self.unet, (B, self.channels, self.height, width), strength, guide, return_tensor=True,
                                       condition=cond.to(self.device), sampler=sampler, initial_noise=init, seed=seed)
+        latents = imgs[-1]
+        if not decode:
+            self.last_launches = s.last_graph_launches
+            return Timbres(latents, None, None, None)
+        return self._decode(s, latents)
+
+    # ---- inpainting with text (inpaint_with_text.py:140-333) ----------------------------------------------------------
+    @torch.no_grad()
+    def inpaint(self, guide_latent: torch.Tensor, mask, cond: torch.Tensor, uncond: Optional[torch.Tensor], steps: int = 20,
+                cfg_scale: float = 6, noising_strength: float = 1.0, sampler: str = "ddim", seed: Optional[int] = None,
+                noise_feed: Optional[torch.Tensor] = None, decode: bool = True) -> Timbres:
+        """Regenerate the masked part of an upload from text: the mask is zoomed to the latent grid (scipy.ndimage.zoom with its
+        defaults, no threshold), then inpaint_sample with classifier-free guidance (:229-231) and the same VQ -> decoder -> iSTFT
+        tail as text-to-timbre, in one graph launch for the whole batch.
+        ``guide_latent``: [1 or B, 4, 128, w], e.g. from encode_audio.  ``mask``: 1 keeps the upload, 0 regenerates; in the
+        spectrogram's orientation (row 0 = lowest frequency, last axis = time; flip an image-oriented mask first) on any grid,
+        e.g. 513 x T as InputBatch2Encode_STFT renders it after np.flipud, or 512 x 4w; one 2-D array / tensor for every row, a
+        [B, H, W] one, or a list of B 2-D ones of any shapes.  All masks go through ONE ds_mask_zoom into the [B, 1, 128, w]
+        mask the sampling graph reads.  The sampler is respaced to ``steps`` (cached per (batch, steps)), as generate does."""
+        B = cond.shape[0]
+        if guide_latent.dim() != 4 or guide_latent.shape[0] not in (1, B) or tuple(guide_latent.shape[1:3]) != (self.channels, self.height):
+            raise ValueError(f"guide_latent must be [1 or {B}, {self.channels}, {self.height}, w], got {tuple(guide_latent.shape)}")
+        width = guide_latent.shape[-1]
+        if isinstance(mask, (list, tuple)):
+            items = [torch.as_tensor(m) for m in mask]
+            if len(items) != B or any(m.dim() != 2 for m in items):
+                raise ValueError(f"a list mask must hold {B} 2-D arrays")
+        else:
+            m = torch.as_tensor(mask)
+            if m.dim() == 2:
+                items = [m]
+            elif m.dim() == 3 and m.shape[0] == B:
+                items = list(m)
+            else:
+                raise ValueError(f"mask must be 2-D, [{B}, H, W] or a list of {B} 2-D arrays, got shape {tuple(m.shape)}")
+        zoomed = torch.empty((len(items), 1, self.height, width), dtype=torch.float32, device=self.device)
+        zoom_packed(torch.cat([m.to(self.device, torch.float32).reshape(-1) for m in items]), [tuple(m.shape) for m in items],
+                    (self.height, width), out=zoomed)
+        key = ("inpaint", B, steps)
+        s = self._samplers.get(key)
+        if s is None:
+            s = DiffSynthSampler(self.timesteps, height=self.height, channels=self.channels, noise_strategy=self.noise_strategy,
+                                 mute=True, device=str(self.device), max_batchsize=B)
+            s.respace(list(np.linspace(0, self.timesteps - 1, steps, dtype=np.int32)))
+            self._samplers[key] = s
+        s.activate_classifier_free_guidance(cfg_scale, uncond)
+        guide = guide_latent.to(self.device, torch.float32)
+        if guide.shape[0] == 1 and B > 1:
+            guide = guide.repeat(B, 1, 1, 1)
+        init = None
+        s.noise_feed = None
+        if noise_feed is not None:
+            init = noise_feed[0][:B].to(self.device, torch.float32)
+            s.noise_feed = noise_feed[1:]
+        s.graph_tail, s.final_only = (self._tail_factory if decode else None), True
+        imgs, _ = s.inpaint_sample(self.unet, (B, self.channels, self.height, width), noising_strength, guide, zoomed, return_tensor=True,
+                                   condition=cond.to(self.device), sampler=sampler, initial_noise=init, seed=seed)
         latents = imgs[-1]
         if not decode:
             self.last_launches = s.last_graph_launches

@@ -253,6 +253,22 @@ int ds_resample(const float* d_in, float* d_out, const long long* lengths, const
                 const long long* out_lengths, int normalize_peak, int B, void* d_ws, long long ws_bytes, void* stream);
 
 /* ----------------------------------------------------------------------------------------
+ * Mask zoom for inpainting with text (webUI/natural_language_guided_4/inpaint_with_text.py: the spectrogram mask is shrunk to the
+ * latent grid): scipy.ndimage.zoom(a, (h/H, w/W)) with scipy's defaults (order 3, mode 'constant', prefilter, grid_mode False)
+ * for B 2-D fp32 arrays packed back to back in d_in (item k: in_shapes[2k] x in_shapes[2k+1], row-major), each written to d_out
+ * (packed, item k: out_shapes[2k] x out_shapes[2k+1]).  Separable: the cubic B-spline prefilter (mirror boundary) and the
+ * interpolation at x = o * (n-1)/(out-1) run along the rows' axis, then along the columns' axis, in float64 as scipy does; the
+ * result is rounded once to fp32.  Every dimension in 1..DS_MASK_ZOOM_MAX_DIM, so that every element and byte offset of up to
+ * 2^31 items fits in int64.  Each output sums in a fixed order: an item's result does not depend on the rest of the batch.  Host
+ * arrays are checked before any device work and uploaded with one cudaMemcpyAsync; 2 launches whatever B.
+ * d_ws: ds_mask_zoom_workspace bytes.
+ * -------------------------------------------------------------------------------------- */
+#define DS_MASK_ZOOM_MAX_DIM 16384LL
+int ds_mask_zoom_workspace(const long long* in_shapes, const long long* out_shapes, int B, long long* bytes);
+int ds_mask_zoom(const float* d_in, float* d_out, const long long* in_shapes, const long long* out_shapes, int B, void* d_ws,
+                 long long ws_bytes, void* stream);
+
+/* ----------------------------------------------------------------------------------------
  * Image products of the decode glue (webUI/natural_language_guided_4/utils.py), batched:
  *   spectrogram_to_Gradio_image (:8-50, with tools.np_power_to_db tools.py:41-50) and phase_to_Gradio_image (:53-91)
  *   of |D| / angle(D) for D = depad_STFT(decode_stft(spec)) (:229-238): uint8 [B, 513, T, 3], flipped vertically;
