@@ -45,6 +45,10 @@ class ConvGemmArgs(C.Structure):
     ]
 
 
+class ConvGemmPlanInfo(C.Structure):
+    _fields_ = [(n, C.c_int32) for n in ("BK", "BN", "cg", "pair_flat", "epi", "two_per_sm", "nacc", "sps", "stages", "num_tiles", "grid")]
+
+
 _P, _I, _L, _F = C.c_void_p, C.c_int, C.c_longlong, C.c_float
 _SIGNATURES = {
     "ds_last_error": (C.c_char_p, []),
@@ -54,6 +58,7 @@ _SIGNATURES = {
     "ds_conv_gemm": (_I, [C.POINTER(ConvGemmArgs), _P]),
     "ds_conv_gemm_reference": (_I, [C.POINTER(ConvGemmArgs), _P]),
     "ds_conv_gemm_stats_slots": (_I, [C.POINTER(ConvGemmArgs)]),
+    "ds_conv_gemm_plan": (_I, [C.POINTER(ConvGemmArgs), C.POINTER(ConvGemmPlanInfo)]),
     "ds_ddim_step": (_I, [_P, _P, _P, _P, _P, _P, _L, _P]),
     "ds_q_sample": (_I, [_P, _P, _P, _P, _L, _L, _P]),
     "ds_mask_blend": (_I, [_P, _P, _P, _I, _P, _P, _I, _I, _L, _P]),

@@ -963,15 +963,64 @@ static void fill_dev(const ds_conv_gemm_args* a, ConvGemmDev& P) {
   memcpy(P.taps, a->taps, sizeof(P.taps));
 }
 
-static int conv_gemm_launch(const ds_conv_gemm_args* a, cudaStream_t stream) {
+// Every launch decision of one call: the tile schedule (fill_dev), the epilogue specialisation, the residency (two CTAs per SM),
+// the pipeline depth and the grid.  conv_gemm_launch launches exactly this plan and ds_conv_gemm_plan reports it.
+struct LaunchPlan { int epi; bool two_per_sm; size_t smem; int grid; };
+
+static int plan_launch(const ds_conv_gemm_args* a, ConvGemmDev& P, LaunchPlan& L) {
   int rc = validate(a);
+  if (rc) return rc;
+  fill_dev(a, P);
+  // epilogue specialisation (see the kernel): the main path needs a 16-bit output whose every chunk is full
+  int epi = 0;
+  if (a->d_out && !a->d_out_f32_nchw && a->Cout == a->Cout_pad && !(P.dbg & 1) && !knobs().generic_epi) {
+    if (a->act == 0) epi = a->d_residual ? 3 : (!a->d_e1 && !a->d_sbias && !a->d_stats_in) ? 4 : 1;
+    else if (!a->d_residual && a->d_e1 && a->d_stats_in && !a->d_sbias) epi = 2;      // ConvNeXt conv1: fold + GELU, no per-sample bias
+  }
+  // two resident CTAs per SM for the plain 1x1 convolutions whose accumulator pair fits half of the tensor memory (see the kernel)
+  // (BN <= 128: each CTA keeps its double-buffered accumulator in half of the tensor memory; BN <= 256: a single accumulator per CTA,
+  // the other CTA's work covers the wait between a tile's MMAs and its epilogue)
+  const size_t fixed_bytes = smem_fixed_bytes(a);
+  const size_t half_budget = fixed_bytes < 111 * 1024 ? 111 * 1024 - fixed_bytes : 0;
+  const bool two_per_sm = epi == 4 && P.cg == 1 && a->ntaps == 1 && half_budget >= 2 * ((size_t)P.stage_a_bytes + P.stage_b_bytes);
+  P.nacc = (two_per_sm && 2 * a->BN > 256) ? 1 : 2;
+  const size_t budget = two_per_sm ? half_budget : smem_budget(a);
+  // K-blocks per stage: one barrier round trip per stage costs a few hundred cycles on the single MMA-issuing thread, so every
+  // stage should carry >= ~384 cycles of tensor work (BK/16 MMAs of BN/2 cycles each per K-block) while >= 4 stages still fit.
+  P.sps = 1;
+  {
+    const size_t sub = (size_t)P.stage_a_bytes + P.stage_b_bytes;
+    const int cyc = (a->BK / 16) * (a->BN / 2);
+    const int max_sps = two_per_sm ? 1 : knobs().max_sps;          // 4: the producer keeps at most 4 table entries in registers
+    const int min_stages = knobs().min_stages;    // 3: three stages already saturate the pipeline (measured); deeper rings buy nothing
+    const int cyc_target = knobs().sps_cyc;       // 768: measured, two barrier round trips per ~768 MMA cycles keep the single issuing thread off the critical path
+    while (P.sps < max_sps && P.sps * cyc < cyc_target && P.sps < P.num_kb && (size_t)(P.sps + 1) * sub * min_stages <= budget) ++P.sps;
+  }
+  const size_t stage_bytes = (size_t)P.sps * ((size_t)P.stage_a_bytes + P.stage_b_bytes);
+  int stages = (int)(budget / stage_bytes);
+  if (stages > kMaxStages) stages = kMaxStages;
+  if (knobs().max_stages >= 2 && knobs().max_stages < stages) stages = knobs().max_stages;      // (-DDS_CONV_DEBUG experiment knob)
+  // (the ring spans tiles of the persistent loop: small-K convs prefetch several tiles ahead, so it is never clamped to K)
+  DS_REQUIRE(stages >= 2, "ds_conv_gemm: epilogue tables leave no room for a 2-stage pipeline (Cout_pad=%d ncls=%d)", a->Cout_pad, a->ncls);
+  P.stages = stages;
+  L.epi = epi;
+  L.two_per_sm = two_per_sm;
+  L.smem = fixed_bytes + stages * stage_bytes;
+  const int slots = two_per_sm ? 2 * num_sms() : num_sms();
+  L.grid = P.num_tiles < slots ? P.num_tiles : slots;
+  if (P.cg == 2) { const int pairs = num_sms() / 2; L.grid = 2 * (P.num_tiles < pairs ? P.num_tiles : pairs); }
+  return DS_OK;
+}
+
+static int conv_gemm_launch(const ds_conv_gemm_args* a, cudaStream_t stream) {
+  ConvGemmDev P;
+  LaunchPlan L;
+  int rc = plan_launch(a, P, L);
   if (rc) return rc;
   EncodeTiledFn encode = get_encode_fn();
   DS_REQUIRE(encode != nullptr, "ds_conv_gemm: cuTensorMapEncodeTiled entry point not available");
 
   TmaMaps maps;          // per call (host threads may launch concurrently); unused slots are copies of a valid map (prefetch-safe)
-  ConvGemmDev P;
-  fill_dev(a, P);
   const CUtensorMapSwizzle swz = a->BK == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
 
   for (int s = 0; s < 2; ++s) {
@@ -1005,43 +1054,8 @@ static int conv_gemm_launch(const ds_conv_gemm_args* a, cudaStream_t stream) {
     DS_REQUIRE(r == CUDA_SUCCESS, "ds_conv_gemm: cuTensorMapEncodeTiled(B) failed with %d (K=%lld Cout_pad=%d)", (int)r, K, a->Cout_pad);
   }
 
-  // epilogue specialisation (see the kernel): the main path needs a 16-bit output whose every chunk is full
-  int epi = 0;
-  if (a->d_out && !a->d_out_f32_nchw && a->Cout == a->Cout_pad && !(P.dbg & 1) && !knobs().generic_epi) {
-    if (a->act == 0) epi = a->d_residual ? 3 : (!a->d_e1 && !a->d_sbias && !a->d_stats_in) ? 4 : 1;
-    else if (!a->d_residual && a->d_e1 && a->d_stats_in && !a->d_sbias) epi = 2;      // ConvNeXt conv1: fold + GELU, no per-sample bias
-  }
-  // two resident CTAs per SM for the plain 1x1 convolutions whose accumulator pair fits half of the tensor memory (see the kernel)
-  // (BN <= 128: each CTA keeps its double-buffered accumulator in half of the tensor memory; BN <= 256: a single accumulator per CTA,
-  // the other CTA's work covers the wait between a tile's MMAs and its epilogue)
-  const size_t fixed_bytes = smem_fixed_bytes(a);
-  const size_t half_budget = fixed_bytes < 111 * 1024 ? 111 * 1024 - fixed_bytes : 0;
-  const bool two_per_sm = epi == 4 && P.cg == 1 && a->ntaps == 1 && half_budget >= 2 * ((size_t)P.stage_a_bytes + P.stage_b_bytes);
-  P.nacc = (two_per_sm && 2 * a->BN > 256) ? 1 : 2;
-  const size_t budget = two_per_sm ? half_budget : smem_budget(a);
-  // K-blocks per stage: one barrier round trip per stage costs a few hundred cycles on the single MMA-issuing thread, so every
-  // stage should carry >= ~384 cycles of tensor work (BK/16 MMAs of BN/2 cycles each per K-block) while >= 4 stages still fit.
-  P.sps = 1;
-  {
-    const size_t sub = (size_t)P.stage_a_bytes + P.stage_b_bytes;
-    const int cyc = (a->BK / 16) * (a->BN / 2);
-    const int max_sps = two_per_sm ? 1 : knobs().max_sps;          // 4: the producer keeps at most 4 table entries in registers
-    const int min_stages = knobs().min_stages;    // 3: three stages already saturate the pipeline (measured); deeper rings buy nothing
-    const int cyc_target = knobs().sps_cyc;       // 768: measured, two barrier round trips per ~768 MMA cycles keep the single issuing thread off the critical path
-    while (P.sps < max_sps && P.sps * cyc < cyc_target && P.sps < P.num_kb && (size_t)(P.sps + 1) * sub * min_stages <= budget) ++P.sps;
-  }
-  const size_t stage_bytes = (size_t)P.sps * ((size_t)P.stage_a_bytes + P.stage_b_bytes);
-  int stages = (int)(budget / stage_bytes);
-  if (stages > kMaxStages) stages = kMaxStages;
-  if (knobs().max_stages >= 2 && knobs().max_stages < stages) stages = knobs().max_stages;      // (-DDS_CONV_DEBUG experiment knob)
-  // (the ring spans tiles of the persistent loop: small-K convs prefetch several tiles ahead, so it is never clamped to K)
-  DS_REQUIRE(stages >= 2, "ds_conv_gemm: epilogue tables leave no room for a 2-stage pipeline (Cout_pad=%d ncls=%d)", a->Cout_pad, a->ncls);
-  P.stages = stages;
-  const size_t smem = fixed_bytes + stages * stage_bytes;
-
-  const int slots = two_per_sm ? 2 * num_sms() : num_sms();
-  int grid = P.num_tiles < slots ? P.num_tiles : slots;
-  if (P.cg == 2) { const int pairs = num_sms() / 2; grid = 2 * (P.num_tiles < pairs ? P.num_tiles : pairs); }
+  const int epi = L.epi, grid = L.grid;
+  const size_t smem = L.smem;
   static unsigned long long* dbg_buf = nullptr;
   P.dbg_buf = nullptr;
   if (P.dbg & 64) {
@@ -1166,6 +1180,17 @@ extern "C" int ds_conv_gemm(const ds_conv_gemm_args* args, void* stream) {
 }
 extern "C" int ds_conv_gemm_reference(const ds_conv_gemm_args* args, void* stream) {
   return ds::conv_gemm_reference_launch(args, reinterpret_cast<cudaStream_t>(stream));
+}
+extern "C" int ds_conv_gemm_plan(const ds_conv_gemm_args* a, ds_conv_gemm_plan_info* info) {
+  DS_REQUIRE(info != nullptr, "ds_conv_gemm_plan: null info");
+  ds::ConvGemmDev P;
+  ds::LaunchPlan L;
+  const int rc = ds::plan_launch(a, P, L);
+  if (rc) return rc;
+  info->BK = a->BK; info->BN = a->BN; info->cg = P.cg; info->pair_flat = P.pair_flat; info->epi = L.epi;
+  info->two_per_sm = L.two_per_sm ? 1 : 0; info->nacc = P.nacc; info->sps = P.sps; info->stages = P.stages;
+  info->num_tiles = P.num_tiles; info->grid = L.grid;
+  return ds::DS_OK;
 }
 extern "C" int ds_conv_gemm_stats_slots(const ds_conv_gemm_args* a) {
   if (!a || a->Hb <= 0 || a->Wb <= 0 || a->BN <= 0) return -1;

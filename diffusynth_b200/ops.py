@@ -13,7 +13,7 @@ from typing import List, Optional, Sequence, Tuple
 import torch
 
 from . import _lib
-from ._lib import ConvGemmArgs, check
+from ._lib import ConvGemmArgs, ConvGemmPlanInfo, check
 
 
 
@@ -298,6 +298,16 @@ def conv_cost(a: ConvGemmArgs, pc: PackedConv) -> Tuple[str, float, float]:
         by += out_px * a.Cout * 2.0
     fam = "conv3x3" if (pc.kind == "s1" and a.ntaps == 9) else "conv1x1" if pc.kind == "s1" else "conv4x4s2" if pc.kind == "down" else "convT4x4s2"
     return fam, flops, by
+
+
+def conv_plan(a: ConvGemmArgs) -> dict:
+    """The launch ds_conv_gemm makes for this argument block (ds_conv_gemm_plan; host only), plus the mean number of work items
+    per CTA (per CTA pair when cg = 2)."""
+    info = ConvGemmPlanInfo()
+    check(_lib.load().ds_conv_gemm_plan(C.byref(a), C.byref(info)), "ds_conv_gemm_plan")
+    plan = {name: getattr(info, name) for name, _ in ConvGemmPlanInfo._fields_}
+    plan["items_per_cta"] = plan["num_tiles"] / (plan["grid"] // plan["cg"])
+    return plan
 
 
 def run_conv(a: ConvGemmArgs, reference: bool = False) -> None:

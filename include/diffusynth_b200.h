@@ -117,6 +117,22 @@ int ds_conv_gemm_stats_slots(const ds_conv_gemm_args* args);
 /* Same contract on plain CUDA cores; exists only to cross-check the tcgen05 kernel in tests. */
 int ds_conv_gemm_reference(const ds_conv_gemm_args* args, void* stream);
 
+/* The launch ds_conv_gemm would make for these arguments (host only, launches nothing; ds_conv_gemm launches from the same
+   computation).  A work item is one 128-pixel M-tile x BN-channel N-tile (cg = 1) or a pair of M-tiles on a two-CTA cluster
+   (cg = 2); the grid's CTAs (CTA pairs) walk the items with a stride of grid (grid / 2). */
+typedef struct ds_conv_gemm_plan_info {
+  int32_t BK, BN;           /* K block and N tile (as given in the arguments) */
+  int32_t cg;               /* CTAs per MMA: 1, or 2 (cta_group::2 pairs) */
+  int32_t pair_flat;        /* cg = 2 pairs run over the flattened (sample, M-tile) index (odd M-tiles per sample) */
+  int32_t epi;              /* epilogue variant: 0 generic (fp32 / ragged output), 1 fold, 2 fold + GELU, 3 + residual, 4 bias only */
+  int32_t two_per_sm;       /* two resident CTAs per SM (plain 1x1 convolutions) */
+  int32_t nacc;             /* tensor-memory accumulators per CTA: 2 (double-buffered) or 1 */
+  int32_t sps, stages;      /* K-blocks per pipeline stage, pipeline stages */
+  int32_t num_tiles;        /* work items */
+  int32_t grid;             /* CTAs launched */
+} ds_conv_gemm_plan_info;
+int ds_conv_gemm_plan(const ds_conv_gemm_args* args, ds_conv_gemm_plan_info* info);
+
 /* ----------------------------------------------------------------------------------------
  * Sampler step kernels (model/DiffSynthSampler.py).
  * -------------------------------------------------------------------------------------- */
@@ -138,7 +154,11 @@ int ds_mask_blend(const float* d_guide, const float* d_noise, const float* d_mas
  * U-Net pieces that are not GEMMs (model/diffusion_components.py, model/diffusion.py).
  * -------------------------------------------------------------------------------------- */
 /* ConvNextBlock.ds_conv (:118,131) + time-embedding bias (:133-136) + partials of net[0] GroupNorm (:121).
-   src_batch_mod > 0: sample n reads sample n % src_batch_mod of source 0 (source 1 is indexed by n). */
+   src_batch_mod > 0: sample n reads sample n % src_batch_mod of source 0 (source 1 is indexed by n).
+   out = act16(bias + sum over the 49 taps of x * w), accumulated in fp32.  Two kernels, whose weights differ:
+     H >= 16: warp-level tensor cores on 16-row tiles; the weights are rounded to the 16-bit operand type first.
+     H <  16: packed fp32 FMA on 8-row tiles; the weights stay fp32.
+   The (sum, sumsq) partials are of the fp32 values before the 16-bit rounding. */
 int ds_dwconv7(const void* d_src0, const void* d_src1, int C0, int C1, int src_batch_mod, const float* d_weight,
                const float* d_tbias, long long tbias_stride, void* d_out, void* d_stats, float eps, int N, int H, int W, void* stream);
 int ds_dwconv7_stats_slots(int C, int H, int W);

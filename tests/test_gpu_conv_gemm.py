@@ -23,20 +23,39 @@ def _run(pc, srcs, N, H, W, reference=False, **kw):
     return st
 
 
+# Small jobs (these are all far below the 148 SMs) run narrow N tiles and one work item per CTA: (BN, cg, pair_flat) each case
+# runs, from the planner query.  Wide N tiles and persistent runs of many items per CTA: tests/test_gpu_conv_scale.py.
+PLAIN_PLANS = {
+    (64, 64, 3, 16, 8, 2): (32, 2, 1),
+    (96, 192, 3, 32, 16, 2): (64, 2, 0),
+    (128, 96, 1, 16, 16, 3): (32, 1, 0),
+    (192, 384, 3, 16, 8, 1): (64, 1, 0),
+    (192, 384, 3, 16, 8, 4): (64, 2, 1),
+    (128, 96, 3, 16, 24, 3): (32, 1, 0),
+    (64, 768, 1, 16, 8, 2): (64, 1, 0),
+    (96, 96, 3, 128, 64, 2): (96, 2, 0),
+    (32, 32, 3, 128, 24, 1): (32, 2, 0),
+    (64, 48, 3, 20, 12, 2): (48, 1, 0),
+    (96, 192, 3, 64, 32, 2): (64, 2, 0),
+    (64, 64, 3, 20, 40, 3): (32, 1, 0),
+    (128, 256, 3, 128, 64, 1): (64, 2, 0),
+}
+
+
 @pytest.mark.parametrize("cin,cout,k,H,W,N", [
-    (64, 64, 3, 16, 8, 2),        # BK=64 (SWIZZLE_128B), one tile per sample
+    (64, 64, 3, 16, 8, 2),        # BK=64 (SWIZZLE_128B), one tile per sample: the two-CTA pair spans both samples
     (96, 192, 3, 32, 16, 2),      # BK=32 (SWIZZLE_64B), 4 m-tiles
     (128, 96, 1, 16, 16, 3),      # 1x1
-    (192, 384, 3, 16, 8, 1),      # two n-tiles (BN=192)
+    (192, 384, 3, 16, 8, 1),      # six narrow n-tiles (BN=64), one CTA per tile
     (192, 384, 3, 16, 8, 4),      # one M-tile per sample: the two-CTA pairs span consecutive samples
     (128, 96, 3, 16, 24, 3),      # three M-tiles per sample, odd sample count: falls back to one CTA per tile
-    (64, 768, 1, 16, 8, 2),       # BN=256, three n-tiles
-    (96, 96, 3, 128, 64, 2),      # full-resolution level-0 shape, 64 m-tiles per sample (persistent loop)
+    (64, 768, 1, 16, 8, 2),       # 1x1 with twelve narrow n-tiles (BN=64), two CTAs per SM
+    (96, 96, 3, 128, 64, 2),      # full-resolution level-0 shape, 64 m-tiles per sample
     (32, 32, 3, 128, 24, 1),      # width not a multiple of the preferred tile
     (64, 48, 3, 20, 12, 2),       # ragged: partial tiles in both directions
     (96, 192, 3, 64, 32, 2),      # BK=32 with several K-blocks per stage
     (64, 64, 3, 20, 40, 3),       # ragged, W > 32
-    (128, 256, 3, 128, 64, 1),    # BK=64, BN=256, 64 tiles per sample
+    (128, 256, 3, 128, 64, 1),    # BK=64, 64 tiles per sample, four n-tiles: up to two items per CTA pair
 ])
 def test_plain_conv(cin, cout, k, H, W, N):
     from diffusynth_b200 import ops
@@ -44,6 +63,9 @@ def test_plain_conv(cin, cout, k, H, W, N):
     w, b = cases.randn((cout, cin, k, k), 2) * (1.0 / (cin * k * k) ** 0.5), cases.randn((cout,), 3)
     pc = ops.pack_conv_s1(w, b)
     out = torch.zeros((N, H, W, cout), dtype=ops.ACT, device="cuda")
+    a, _, _ = ops.conv_args(pc.to("cuda"), nhwc(x), None, N, H, W, out=out)
+    plan = ops.conv_plan(a)
+    assert (plan["BN"], plan["cg"], plan["pair_flat"]) == PLAIN_PLANS[(cin, cout, k, H, W, N)]
     _run(pc, [nhwc(x)], N, H, W, out=out)
     ref = F.conv2d(bf(x), bf(w), b, padding=k // 2)
     assert rel(nchw(out), ref) < TOL
