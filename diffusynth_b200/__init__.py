@@ -7,7 +7,7 @@ Importing the compute classes needs a CUDA build of torch; there is no CPU fallb
 from . import weights  # noqa: F401  (pure-python parameter inventory; safe everywhere)
 
 __all__ = ["weights", "DiffSynthSampler", "ConditionedUnet", "VQGAN", "VectorQuantizerEMA", "Decoder", "Encoder",
-           "TextToTimbre", "TextEncoder", "spectrogram_to_waveform", "waveform_to_spectrogram", "pitch_shift", "mix_track"]
+           "TextToTimbre", "TextEncoder", "spectrogram_to_waveform", "waveform_to_spectrogram", "pitch_shift", "mix_track", "mix_arrangement"]
 
 
 def __getattr__(name):
@@ -28,7 +28,7 @@ def __getattr__(name):
         return TextToTimbre
     if name in ("spectrogram_to_waveform", "waveform_to_spectrogram", "encodeBatch2GradioOutput_STFT", "InputBatch2Encode_STFT",
                 "spectrogram_images", "latent_images", "latent_representation_to_Gradio_image", "griffinlim",
-                "pitch_shift", "mix_track", "shift_and_mix"):
+                "pitch_shift", "mix_track", "mix_arrangement", "shift_and_mix"):
         from . import codec
         return getattr(codec, name)
     raise AttributeError(name)

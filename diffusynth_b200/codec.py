@@ -234,15 +234,59 @@ def mix_track(packed: torch.Tensor, src_offsets, lengths, onsets, gains, track_l
     return track
 
 
-def shift_and_mix(sources, semitones, note_source, onsets, gains) -> torch.Tensor:
+def _check_peak(target_peak) -> float:
+    """None (no normalisation) -> 0.0; otherwise a finite peak > 0."""
+    if target_peak is None:
+        return 0.0
+    p = float(target_peak)
+    if not np.isfinite(p) or p <= 0.0 or not np.isfinite(np.float32(p)):
+        raise ValueError(f"target_peak must be None or a finite value > 0, got {target_peak}")
+    return p
+
+
+@torch.no_grad()
+def mix_arrangement(packed: torch.Tensor, src_offsets, lengths, onsets, gains, fade_out, target_peak: Optional[float] = None,
+                    track_len: Optional[int] = None) -> torch.Tensor:
+    """mix_track with a linear fade over the last fade_out[n] samples of every note (clamped to the note; 0 = none) and, when
+    ``target_peak`` is given, the track scaled on the device so that max |track| == target_peak (ds_mix_arrangement).  Notes
+    without a fade are summed exactly as mix_track sums them.  Summed in note order, bit-identical run to run."""
+    lib = _lib.load()
+    off = np.ascontiguousarray(src_offsets, dtype=np.int64)
+    L = np.ascontiguousarray(lengths, dtype=np.int64)
+    on = np.ascontiguousarray(onsets, dtype=np.int64)
+    g = np.ascontiguousarray(gains, dtype=np.float32)
+    fade = np.ascontiguousarray(fade_out, dtype=np.int64)
+    peak = _check_peak(target_peak)
+    if np.any(fade < 0):
+        raise ValueError(f"fade_out must be >= 0, got {fade_out}")
+    K = len(L)
+    if track_len is None:
+        track_len = int((on + L).max())
+    nbytes = C.c_longlong(0)
+    check(lib.ds_mix_arrangement_workspace(L.ctypes.data, on.ctypes.data, fade.ctypes.data, K, peak, int(track_len), C.byref(nbytes)),
+          "ds_mix_arrangement_workspace")
+    packed = packed.float().contiguous()
+    ws = torch.empty((nbytes.value,), dtype=torch.uint8, device=packed.device)
+    track = torch.empty((int(track_len),), dtype=torch.float32, device=packed.device)
+    check(lib.ds_mix_arrangement(packed.data_ptr(), off.ctypes.data, L.ctypes.data, on.ctypes.data, g.ctypes.data, fade.ctypes.data, K,
+                                 peak, track.data_ptr(), int(track_len), ws.data_ptr(), nbytes.value, ops._stream()), "ds_mix_arrangement")
+    return track
+
+
+def shift_and_mix(sources, semitones, note_source, onsets, gains, fades=None, target_peak: Optional[float] = None) -> torch.Tensor:
     """The arrangement stage after synthesis: every source (1-D fp32 device tensor) is pitch-shifted by its semitones in ONE batched
     call, then note n -- source note_source[n] at sample onsets[n], scaled by gains[n] -- is mixed in ONE call.  Two library
-    calls plus their workspace queries, whatever the number of notes."""
+    calls plus their workspace queries, whatever the number of notes.  ``fades`` (per note, in samples) or ``target_peak``
+    mix through mix_arrangement; without either, through mix_track."""
     lengths = [int(s.numel()) for s in sources]
     shifted = pitch_shift_packed(torch.cat([s.reshape(-1) for s in sources]), lengths, semitones)
     starts = np.concatenate([[0], np.cumsum(lengths)[:-1]]).astype(np.int64)
     idx = np.asarray(note_source, dtype=np.int64)
-    return mix_track(shifted, starts[idx], np.asarray(lengths, dtype=np.int64)[idx], onsets, gains)
+    note_len = np.asarray(lengths, dtype=np.int64)[idx]
+    if fades is None and target_peak is None:
+        return mix_track(shifted, starts[idx], note_len, onsets, gains)
+    fades = np.zeros(len(idx), dtype=np.int64) if fades is None else fades
+    return mix_arrangement(shifted, starts[idx], note_len, onsets, gains, fades, target_peak)
 
 
 # ---- sample-rate conversion (tools.adjust_audio_length's librosa.resample, tools.py:126-151) ----------------------------------

@@ -238,6 +238,77 @@ pitch_mix_kernel(const float* __restrict__ src, float* __restrict__ track, long 
   }
 }
 
+// ---- arrangement mix: pitch_mix_kernel's gather with a linear fade over the last fade_n samples of every note (fade_n =
+// min(fade_out[n], len[n]), clamped on the host) and, when `peak` is non-null, one max |track| partial per tile.  A sample before
+// the ramp takes pitch_mix_kernel's exact fmaf(gain, src, acc), so a fade-free note has no envelope multiply at all.  Every thread
+// owns ARR_SPT samples 256 apart and walks the tile's notes once for all of them (a note's metadata is loaded once per thread, not
+// once per sample); each sample still sums its notes in input order, as pitch_mix_kernel does.  256 threads per block.
+constexpr int ARR_SPT = MIX_TILE / 256;
+__global__ void __launch_bounds__(256)
+pitch_arrange_kernel(const float* __restrict__ src, float* __restrict__ track, long long track_len, const int* __restrict__ tile_ptr,
+                     const int* __restrict__ tile_notes, const long long* __restrict__ src_off, const long long* __restrict__ len,
+                     const long long* __restrict__ onset, const float* __restrict__ gain, const long long* __restrict__ fade,
+                     float* __restrict__ peak) {
+  pdl_enter();
+  __shared__ float red[8];
+  const int p0 = __ldg(tile_ptr + blockIdx.x), p1 = __ldg(tile_ptr + blockIdx.x + 1);
+  const long long j0 = (long long)blockIdx.x * MIX_TILE + threadIdx.x;
+  float acc[ARR_SPT];
+#pragma unroll
+  for (int k = 0; k < ARR_SPT; ++k) acc[k] = 0.f;
+  for (int p = p0; p < p1; ++p) {
+    const int n = __ldg(tile_notes + p);
+    const long long on = __ldg(onset + n), L = __ldg(len + n), F = __ldg(fade + n);   // (samples past track_len have r >= L)
+    const float g = __ldg(gain + n);
+    const float* sn = src + __ldg(src_off + n);
+#pragma unroll
+    for (int k = 0; k < ARR_SPT; ++k) {
+      const long long r = j0 + 256 * k - on;
+      if (r < 0 || r >= L) continue;
+      const float s = __ldg(sn + r);
+      const long long left = L - r;                                       // 1 on the note's last sample
+      if (left > F) acc[k] = fmaf(g, s, acc[k]);
+      else acc[k] = fmaf(g * ((float)left / (float)F), s, acc[k]);
+    }
+  }
+  float pk = 0.f;
+#pragma unroll
+  for (int k = 0; k < ARR_SPT; ++k) {
+    const long long j = j0 + 256 * k;
+    if (j < track_len) {
+      track[j] = acc[k];
+      pk = fmaxf(pk, fabsf(acc[k]));
+    }
+  }
+  if (!peak) return;
+  pk = warp_max(pk);
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = pk;
+  __syncthreads();
+  if (threadIdx.x < 32) {
+    pk = warp_max(threadIdx.x < 8 ? red[threadIdx.x] : 0.f);
+    if (threadIdx.x == 0) peak[blockIdx.x] = pk;
+  }
+}
+
+// ---- peak normalisation: every block reduces the n_tiles partials (a maximum: exact in any order), then scales its grid-stride
+// share of the track by target / max in place.  An all-zero track stays zero.
+__global__ void __launch_bounds__(512)
+pitch_peak_scale_kernel(float* __restrict__ track, long long track_len, const float* __restrict__ peak, int n_tiles, float target) {
+  pdl_enter();
+  __shared__ float red[16];
+  float m = 0.f;
+  for (int t = threadIdx.x; t < n_tiles; t += blockDim.x) m = fmaxf(m, __ldg(peak + t));
+  m = warp_max(m);
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = m;
+  __syncthreads();
+  m = red[0];
+  for (int w = 1; w < (int)(blockDim.x >> 5); ++w) m = fmaxf(m, red[w]);
+  if (m == 0.f) return;
+  const float sc = target / m;
+  for (long long j = blockIdx.x * (long long)blockDim.x + threadIdx.x; j < track_len; j += (long long)gridDim.x * blockDim.x)
+    track[j] *= sc;
+}
+
 // I0(x) by its power series sum ((x/2)^k / k!)^2 (converged to double precision for the beta used here)
 double bessel_i0(double x) {
   double term = 1.0, sum = 1.0;
@@ -312,16 +383,24 @@ void make_plan(const long long* lengths, const double* n_steps, int B, PitchPlan
 struct MixPlan {
   std::vector<int> tile_ptr, tile_notes;
   size_t off_notes = 0, off_src = 0, off_len = 0, off_onset = 0, off_gain = 0, bytes = 0;
+  size_t off_fade = 0, off_peak = 0;          // arrangement mix only: the clamped fades, then the per-tile peak partials
   int n_tiles = 0;
 };
 
-int check_mix_args(const long long* lengths, const long long* onsets, int K, long long track_len, const char* who) {
+// fade_out (nullable) and target_peak are the arrangement mix's: fades >= 0, a finite target_peak >= 0; src_offsets (nullable:
+// the workspace queries do not take them) >= 0.
+int check_mix_args(const long long* lengths, const long long* onsets, int K, long long track_len, const char* who,
+                   const long long* fade_out = nullptr, float target_peak = 0.f, const long long* src_offsets = nullptr) {
   DS_REQUIRE(lengths && onsets && K > 0 && track_len > 0, "%s: lengths and onsets must be non-null, K > 0 and track_len > 0", who);
+  DS_REQUIRE(std::isfinite(target_peak) && target_peak >= 0.f, "%s: target_peak %g (must be finite and >= 0)", who, (double)target_peak);
   for (int n = 0; n < K; ++n) {
     DS_REQUIRE(lengths[n] > 0, "%s: note %d has length %lld (must be > 0)", who, n, lengths[n]);
     DS_REQUIRE(onsets[n] >= 0, "%s: note %d has onset %lld (must be >= 0)", who, n, onsets[n]);
     DS_REQUIRE(onsets[n] + lengths[n] <= track_len, "%s: note %d ends at %lld, past the track length %lld", who, n,
                onsets[n] + lengths[n], track_len);
+    DS_REQUIRE(!fade_out || fade_out[n] >= 0, "%s: note %d has fade_out %lld (must be >= 0)", who, n, fade_out ? fade_out[n] : 0LL);
+    DS_REQUIRE(!src_offsets || src_offsets[n] >= 0, "%s: note %d has source offset %lld (must be >= 0)", who, n,
+               src_offsets ? src_offsets[n] : 0LL);
   }
   return DS_OK;
 }
@@ -343,6 +422,15 @@ void make_mix_plan(const long long* lengths, const long long* onsets, int K, lon
   p.off_len = o;   o = align256(o + (size_t)K * sizeof(long long));
   p.off_onset = o; o = align256(o + (size_t)K * sizeof(long long));
   p.off_gain = o;  o = align256(o + (size_t)K * sizeof(float));
+  p.bytes = o;
+}
+
+// make_mix_plan's layout followed by the K clamped fades and, when normalising, one peak partial per tile
+void make_arrangement_plan(const long long* lengths, const long long* onsets, int K, long long track_len, bool normalise, MixPlan& p) {
+  make_mix_plan(lengths, onsets, K, track_len, p);
+  size_t o = p.bytes;
+  p.off_fade = o; o = align256(o + (size_t)K * sizeof(long long));
+  p.off_peak = o; if (normalise) o = align256(o + (size_t)p.n_tiles * sizeof(float));
   p.bytes = o;
 }
 
@@ -448,6 +536,55 @@ int ds_mix_track(const float* d_src, const long long* src_off, const long long* 
   DS_CHECK_CUDA(launch_pdl(pitch_mix_kernel, dim3((unsigned)p.n_tiles), dim3(256), (size_t)0, st, d_src, d_track, track_len,
                            (const int*)ws, (const int*)(ws + p.off_notes), (const long long*)(ws + p.off_src),
                            (const long long*)(ws + p.off_len), (const long long*)(ws + p.off_onset), (const float*)(ws + p.off_gain)));
+  DS_CHECK_CUDA(cudaGetLastError());
+  return DS_OK;
+}
+
+int ds_mix_arrangement_workspace(const long long* lengths, const long long* onsets, const long long* fade_out, int K, float target_peak,
+                                 long long track_len, long long* bytes) {
+  DS_REQUIRE(bytes && fade_out, "ds_mix_arrangement_workspace: bytes and fade_out must be non-null");
+  int rc = check_mix_args(lengths, onsets, K, track_len, "ds_mix_arrangement_workspace", fade_out, target_peak);
+  if (rc) return rc;
+  MixPlan p;
+  make_arrangement_plan(lengths, onsets, K, track_len, target_peak > 0.f, p);
+  *bytes = (long long)p.bytes;
+  return DS_OK;
+}
+
+int ds_mix_arrangement(const float* d_src, const long long* src_offsets, const long long* lengths, const long long* onsets,
+                       const float* gains, const long long* fade_out, int K, float target_peak, float* d_track, long long track_len,
+                       void* d_ws, long long ws_bytes, void* stream) {
+  DS_REQUIRE(d_src && d_track && d_ws && src_offsets && gains && fade_out,
+             "ds_mix_arrangement: d_src, d_track, d_ws, src_offsets, gains and fade_out must be non-null");
+  int rc = check_mix_args(lengths, onsets, K, track_len, "ds_mix_arrangement", fade_out, target_peak, src_offsets);
+  if (rc) return rc;
+  const bool normalise = target_peak > 0.f;
+  MixPlan p;
+  make_arrangement_plan(lengths, onsets, K, track_len, normalise, p);
+  DS_REQUIRE(ws_bytes >= (long long)p.bytes, "ds_mix_arrangement: workspace of %lld bytes, %zu needed", ws_bytes, p.bytes);
+  std::vector<uint8_t> host(p.off_peak, 0);                 // everything but the partials, which the mix kernel writes
+  memcpy(host.data(), p.tile_ptr.data(), p.tile_ptr.size() * sizeof(int));
+  memcpy(host.data() + p.off_notes, p.tile_notes.data(), p.tile_notes.size() * sizeof(int));
+  memcpy(host.data() + p.off_src, src_offsets, (size_t)K * sizeof(long long));
+  memcpy(host.data() + p.off_len, lengths, (size_t)K * sizeof(long long));
+  memcpy(host.data() + p.off_onset, onsets, (size_t)K * sizeof(long long));
+  memcpy(host.data() + p.off_gain, gains, (size_t)K * sizeof(float));
+  long long* fade = (long long*)(host.data() + p.off_fade);
+  for (int n = 0; n < K; ++n) fade[n] = fade_out[n] < lengths[n] ? fade_out[n] : lengths[n];
+  cudaStream_t st = (cudaStream_t)stream;
+  uint8_t* ws = (uint8_t*)d_ws;
+  float* peak = normalise ? (float*)(ws + p.off_peak) : nullptr;
+  DS_CHECK_CUDA(cudaMemcpyAsync(ws, host.data(), host.size(), cudaMemcpyHostToDevice, st));
+  DS_CHECK_CUDA(launch_pdl(pitch_arrange_kernel, dim3((unsigned)p.n_tiles), dim3(256), (size_t)0, st, d_src, d_track, track_len,
+                           (const int*)ws, (const int*)(ws + p.off_notes), (const long long*)(ws + p.off_src),
+                           (const long long*)(ws + p.off_len), (const long long*)(ws + p.off_onset), (const float*)(ws + p.off_gain),
+                           (const long long*)(ws + p.off_fade), peak));
+  if (normalise) {
+    long long blocks = (track_len + 511) / 512;
+    if (blocks > 2LL * num_sms()) blocks = 2LL * num_sms();
+    DS_CHECK_CUDA(launch_pdl(pitch_peak_scale_kernel, dim3((unsigned)blocks), dim3(512), (size_t)0, st, d_track, track_len,
+                             (const float*)peak, p.n_tiles, target_peak));
+  }
   DS_CHECK_CUDA(cudaGetLastError());
   return DS_OK;
 }

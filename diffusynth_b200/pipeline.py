@@ -36,6 +36,19 @@ class TrackPlan:
     track_len: int               # max(onset + length)
 
 
+@dataclass
+class ArrangementPlan:
+    rows: list                   # distinct (track, duration (s)): tracks in order, durations in order of first appearance
+    widths: list                 # per row: latent width
+    items: list                  # distinct (index into rows, semitones), in order of first appearance
+    note_item: list              # per note (tracks in order, then notes in order): index into items
+    onsets: list                 # per note: onset in samples
+    gains: list                  # per note: note gain * track gain
+    fades: list                  # per note: fade-out of its track in samples
+    lengths: list                # per note: samples of its waveform, 256 * (4 * width - 1)
+    track_len: int               # max(onset + length) over every track
+
+
 class _Tail:
     """quantiser -> decoder -> STFT+ decode + iSTFT (text2sound.py:128-134, utils.py:224-241) as a fixed launch sequence on
     static buffers, so that it is captured in the same CUDA graph as the sampling loop: ``src`` is the loop's final-latent
@@ -354,12 +367,22 @@ class TextToTimbre:
         duration -- hence equal latent width -- are batched into ONE graph launch (SURVEY 8f item 1).  Returns one ``Timbres`` per
         note, in input order.  ``noise_feeds`` (tests): per note a host noise tensor [count, 1, C, H, 64]."""
         widths = [self.note_width(d, time_resolution, vae_scale) for d in durations_sec]
+        return self._synthesize_rows([instrument_latent] * len(widths), [condition] * len(widths), widths, sample_steps, noising_strength,
+                                     attack, before_release, sampler, time_resolution, vae_scale, noise_feeds)
+
+    def _synthesize_rows(self, latents, conditions, widths, sample_steps, noising_strength, attack, before_release, sampler, time_resolution,
+                         vae_scale, noise_feeds) -> list:
+        """Rows of equal width -- whatever their instrument latent [1,4,128,64] and condition [1,512] -- as ONE batched graph launch
+        per distinct width (each row of the batch carries its own guide and condition).  Returns one ``Timbres`` per row, in order;
+        ``noise_feeds``: None or one per row."""
         out = [None] * len(widths)
         for w in sorted(set(widths)):
             idx = [i for i, ww in enumerate(widths) if ww == w]
             feed = torch.cat([noise_feeds[i] for i in idx], dim=1) if noise_feeds is not None else None
-            t = self._synthesize_group(instrument_latent, condition, w, len(idx), sample_steps, noising_strength, attack, before_release,
-                                       sampler, time_resolution, vae_scale, feed)
+            guide = torch.cat([latents[i].to(self.device, torch.float32) for i in idx])
+            cond = torch.cat([conditions[i].to(self.device) for i in idx])
+            t = self._synthesize_group(guide, cond, w, len(idx), sample_steps, noising_strength, attack, before_release, sampler,
+                                       time_resolution, vae_scale, feed)
             for b, i in enumerate(idx):
                 out[i] = Timbres(t.latents[b:b + 1], t.quantized[b:b + 1], t.spectrograms[b:b + 1], t.waveforms[b:b + 1])
         return out
@@ -402,6 +425,67 @@ class TextToTimbre:
                                         time_resolution=time_resolution, vae_scale=vae_scale, noise_feeds=noise_feeds)
         sources = [timbres[d].waveforms[0] for d, _ in plan.pairs]
         track = shift_and_mix(sources, [s for _, s in plan.pairs], plan.note_pair, plan.onsets, plan.gains)
+        assert track.numel() == plan.track_len
+        return track
+
+    @staticmethod
+    def arrangement_plan(tracks, time_resolution: int = 256, vae_scale: int = 4, sample_rate: int = 16000) -> ArrangementPlan:
+        """Host side of render_arrangement: ``tracks`` of ``(instrument_latent, condition, notes, gain, fade_out_sec)`` -> track_plan
+        per track, joined: the synthesis rows (one per distinct (track, duration)) and their widths, the pitch items (one per
+        distinct (row, semitones)), and per note in mix order (tracks in order, notes in order) its item, onset, gain (note gain *
+        track gain), fade (round(fade_out_sec * 16000) samples) and length; the track length is the end of the last note."""
+        if len(tracks) == 0:
+            raise ValueError("an arrangement needs at least one track")
+        rows, widths, items, note_item, onsets, gains, fades, lengths = [], [], [], [], [], [], [], []
+        for k, (_, _, notes, gain, fade_sec) in enumerate(tracks):
+            if len(notes) == 0:
+                raise ValueError(f"track {k} has no notes")
+            if not np.isfinite(float(fade_sec)) or float(fade_sec) < 0:
+                raise ValueError(f"track {k}: fade_out_sec must be finite and >= 0, got {fade_sec}")
+            fade = int(round(float(fade_sec) * sample_rate))
+            p = TextToTimbre.track_plan(notes, time_resolution, vae_scale, sample_rate)
+            r0, i0 = len(rows), len(items)
+            rows += [(k, d) for d in p.durations]
+            widths += [TextToTimbre.note_width(d, time_resolution, vae_scale) for d in p.durations]
+            items += [(r0 + d, semi) for d, semi in p.pairs]
+            note_item += [i0 + i for i in p.note_pair]
+            onsets += p.onsets
+            gains += [g * float(gain) for g in p.gains]
+            fades += [fade] * len(p.onsets)
+            lengths += p.lengths
+        track_len = max(o + n for o, n in zip(onsets, lengths))
+        return ArrangementPlan(rows, widths, items, note_item, onsets, gains, fades, lengths, track_len)
+
+    @torch.no_grad()
+    def render_arrangement(self, tracks, sample_steps: int = 20, noising_strength: float = 1.0, attack: float = 0.5,
+                           before_release: float = 0.5, sampler: str = "ddim", target_peak: Optional[float] = None,
+                           time_resolution: int = 256, vae_scale: int = 4, noise_feeds=None) -> torch.Tensor:
+        """Several instruments rendered into one piece on the device: track_maker.DiffSynth over several Tracks, summed.  ``tracks``
+        is a list of ``(instrument_latent [1,4,128,64], condition [1,512], notes, gain, fade_out_sec)``, ``notes`` as render_track
+        takes them.  The (track, duration) rows of ALL tracks are synthesised with one graph launch per distinct width, each row
+        with its own instrument latent and condition; every distinct (row, semitones) item is pitch-shifted in one call; every note
+        is placed with its gain times its track's gain, faded out linearly over the last fade_out_sec of its waveform, and summed
+        in one call (ds_mix_arrangement).  ``target_peak``: None, or max |result| after a peak normalisation on the device.
+        ``noise_feeds`` (tests): one per row (arrangement_plan), in row order.  Returns the fp32 piece [max(onset + note length)]."""
+        if target_peak is not None and not (np.isfinite(float(target_peak)) and float(target_peak) > 0.0):
+            raise ValueError(f"target_peak must be None or a finite value > 0, got {target_peak}")
+        plan = self.arrangement_plan(tracks, time_resolution, vae_scale)
+        latents, conditions = [], []
+        for k, (lat, cond, _, _, _) in enumerate(tracks):
+            if tuple(lat.shape) != (1, self.channels, self.height, 64):
+                raise ValueError(f"track {k}: instrument_latent must be [1, {self.channels}, {self.height}, 64], got {tuple(lat.shape)}")
+            if cond.dim() != 2 or cond.shape[0] != 1:
+                raise ValueError(f"track {k}: condition must be [1, L], got {tuple(cond.shape)}")
+            latents.append(lat)
+            conditions.append(cond)
+        if len({c.shape[1] for c in conditions}) != 1:
+            raise ValueError("every track's condition must have the same length")
+        timbres = self._synthesize_rows([latents[k] for k, _ in plan.rows], [conditions[k] for k, _ in plan.rows], plan.widths,
+                                        sample_steps, noising_strength, attack, before_release, sampler, time_resolution, vae_scale,
+                                        noise_feeds)
+        sources = [timbres[r].waveforms[0] for r, _ in plan.items]
+        track = shift_and_mix(sources, [s for _, s in plan.items], plan.note_item, plan.onsets, plan.gains, fades=plan.fades,
+                              target_peak=target_peak)
         assert track.numel() == plan.track_len
         return track
 

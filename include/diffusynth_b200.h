@@ -251,6 +251,19 @@ int ds_pitch_shift(const float* d_in, float* d_out, const long long* lengths, co
 int ds_mix_track_workspace(const long long* lengths, const long long* onsets, int K, long long track_len, long long* bytes);
 int ds_mix_track(const float* d_src, const long long* src_offsets, const long long* lengths, const long long* onsets, const float* gains,
                  int K, float* d_track, long long track_len, void* d_ws, long long ws_bytes, void* stream);
+/* Arrangement mix (several tracks summed into one piece): ds_mix_track with a linear fade at the end of every note and optional
+   peak normalisation.  d_track[j] = sum over notes n in input order, fp32, of gains[n] * env_n(i) * d_src[src_offsets[n] + i],
+   i = j - onsets[n], 0 <= i < L = lengths[n]; with F = min(fade_out[n], L), env_n(i) = 1 for i < L - F and (L - i) / F after (1/F on
+   the last sample).  A note with fade_out[n] == 0 is summed exactly as ds_mix_track sums it: a fade-free call is bit-identical to
+   ds_mix_track.  target_peak > 0 then scales the track in place by target_peak / max|d_track| (computed on the device: no host
+   synchronisation; an all-zero track stays zero; bit-identical run to run); 0 leaves it unscaled.  fade_out[n] >= 0, finite
+   target_peak >= 0, src_offsets[n] >= 0, every onsets[n] + lengths[n] <= track_len.  d_ws: ds_mix_arrangement_workspace bytes,
+   which include one peak partial per 1024 track samples when target_peak > 0. */
+int ds_mix_arrangement_workspace(const long long* lengths, const long long* onsets, const long long* fade_out, int K, float target_peak,
+                                 long long track_len, long long* bytes);
+int ds_mix_arrangement(const float* d_src, const long long* src_offsets, const long long* lengths, const long long* onsets,
+                       const float* gains, const long long* fade_out, int K, float target_peak, float* d_track, long long track_len,
+                       void* d_ws, long long ws_bytes, void* stream);
 
 /* ----------------------------------------------------------------------------------------
  * Sample-rate conversion of uploaded audio (tools.adjust_audio_length, tools.py:126-151, as sound2sound_with_text.py:75-82 calls
