@@ -99,6 +99,8 @@ _SIGNATURES = {
     "ds_resample": (_I, [_P, _P, _P, _P, _P, _P, _I, _I, _P, _L, _P]),
     "ds_mask_zoom_workspace": (_I, [_P, _P, _I, _P]),
     "ds_mask_zoom": (_I, [_P, _P, _P, _P, _I, _P, _L, _P]),
+    "ds_morph_rows_workspace": (_I, [_I, _I, _L, _L, _I, _P]),
+    "ds_morph_rows": (_I, [_P, _P, _P, _P, _I, _I, _L, _L, _I, _P, _P, _P, _L, _P]),
     "ds_spec_images": (_I, [_P, _P, _P, _P, _I, _I, _P]),
     "ds_latent_image": (_I, [_P, _P, _P, _I, _I, _I, _P]),
     "ds_text_embed_ln": (_I, [_P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _F, _P]),

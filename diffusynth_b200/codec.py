@@ -411,6 +411,35 @@ def zoom_packed(packed: torch.Tensor, in_shapes, out_shapes, out: Optional[torch
     return out
 
 
+MORPH_PATHS = {"linear": 0, "slerp": 1}                # DS_MORPH_LINEAR, DS_MORPH_SLERP
+
+
+@torch.no_grad()
+def morph_rows(e0: torch.Tensor, e1: torch.Tensor, c0: torch.Tensor, c1: torch.Tensor, frames: int, path: str = "slerp"):
+    """The initial-noise and condition rows of P timbre morphs of ``frames`` frames each, by one ds_morph_rows call: endpoints
+    ``e0``, ``e1`` [P, n] and conditions ``c0``, ``c1`` [P, L] (fp32 device tensors of any shape whose leading axis is P) ->
+    (noise [P*frames, n], conditions [P*frames, L]), row p*frames + k = frame k of sequence p at a = k / (frames - 1).
+    ``path``: "linear" (the reference's generate_linear_noise, bit for bit) or "slerp" (spherical, conditions stay linear)."""
+    if path not in MORPH_PATHS:
+        raise ValueError(f"path must be one of {sorted(MORPH_PATHS)}, got {path!r}")
+    lib = _lib.load()
+    P = e0.shape[0]
+    e0, e1 = e0.float().reshape(P, -1).contiguous(), e1.float().reshape(P, -1).contiguous()
+    c0, c1 = c0.float().reshape(P, -1).contiguous(), c1.float().reshape(P, -1).contiguous()
+    if e1.shape != e0.shape or c1.shape != c0.shape or c0.shape[0] != P:
+        raise ValueError(f"endpoints must be [P, n] / [P, L] pairs of one P, got {tuple(e0.shape)}, {tuple(e1.shape)}, "
+                         f"{tuple(c0.shape)}, {tuple(c1.shape)}")
+    n, L, N, mode = e0.shape[1], c0.shape[1], int(frames), MORPH_PATHS[path]
+    nbytes = C.c_longlong(0)
+    check(lib.ds_morph_rows_workspace(P, N, n, L, mode, C.byref(nbytes)), "ds_morph_rows_workspace")
+    noise = torch.empty((P * N, n), dtype=torch.float32, device=e0.device)
+    cond = torch.empty((P * N, L), dtype=torch.float32, device=e0.device)
+    ws = torch.empty((max(nbytes.value, 1),), dtype=torch.uint8, device=e0.device)
+    check(lib.ds_morph_rows(e0.data_ptr(), e1.data_ptr(), c0.data_ptr(), c1.data_ptr(), P, N, n, L, mode, noise.data_ptr(),
+                            cond.data_ptr(), ws.data_ptr(), nbytes.value, ops._stream()), "ds_morph_rows")
+    return noise, cond
+
+
 def zoom(input, zoom, output=None, order=3, mode="constant", cval=0.0, prefilter=True, *, grid_mode=False):
     """On-device, batched ``scipy.ndimage.zoom(input, zoom)`` for 2-D data with scipy's defaults; any other keyword value raises
     NotImplementedError.  ``input``: a [H, W] or [B, H, W] tensor / numpy array (B items of one shape), or a list of 2-D ones of

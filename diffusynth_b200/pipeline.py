@@ -11,7 +11,8 @@ import torch
 
 from . import _lib, ops, weights as W
 from ._lib import check
-from .codec import SAMPLE_RATE, resample_packed, shift_and_mix, spectrogram_to_waveform, waveform_to_spectrogram, zoom_packed
+from .codec import MORPH_PATHS, SAMPLE_RATE, morph_rows, resample_packed, shift_and_mix, spectrogram_to_waveform, waveform_to_spectrogram, \
+    zoom_packed
 from .sampler import DiffSynthSampler
 from .unet import ConditionedUnet
 from .vqgan import VQGAN
@@ -23,6 +24,7 @@ class Timbres:
     quantized: torch.Tensor      # [B,4,128,W]
     spectrograms: torch.Tensor   # [B,3,512,4W]
     waveforms: torch.Tensor      # [B, 256*(4W-1)]
+    initial_noise: Optional[torch.Tensor] = None     # [B,4,128,64] train-width noise each row started from (generate / morph)
 
 
 @dataclass
@@ -148,14 +150,18 @@ class TextToTimbre:
 
     def sampler_for(self, batch: int, steps: int, cfg_scale: float, uncond: Optional[torch.Tensor]) -> DiffSynthSampler:
         """text2sound.py:96-106: fresh sampler, CFG activated, respaced to ``steps`` (cached per (batch, steps))."""
-        key = (batch, steps)
+        s = self._respaced_sampler((batch, steps), batch, steps)
+        s.activate_classifier_free_guidance(cfg_scale, uncond)
+        return s
+
+    def _respaced_sampler(self, key, batch: int, n_steps: int) -> DiffSynthSampler:
+        """A sampler of ``batch`` rows respaced to ``n_steps`` as text2sound.py:96-106 builds it, cached under ``key``."""
         s = self._samplers.get(key)
         if s is None:
             s = DiffSynthSampler(self.timesteps, height=self.height, channels=self.channels, noise_strategy=self.noise_strategy,
                                  mute=True, device=str(self.device), max_batchsize=batch)
-            s.respace(list(np.linspace(0, self.timesteps - 1, steps, dtype=np.int32)))
+            s.respace(list(np.linspace(0, self.timesteps - 1, n_steps, dtype=np.int32)))
             self._samplers[key] = s
-        s.activate_classifier_free_guidance(cfg_scale, uncond)
         return s
 
     @torch.no_grad()
@@ -172,21 +178,83 @@ class TextToTimbre:
     def generate(self, cond: torch.Tensor, uncond: Optional[torch.Tensor], steps: int = 20, cfg_scale: float = 6, width: int = 64,
                  sampler: str = "ddim", seed: Optional[int] = None, noise_feed: Optional[torch.Tensor] = None,
                  decode: bool = True) -> Timbres:
+        """``noise_feed``: host or device draws [K, >=B, 4, 128, 64], draw 0 the initial noise and 1.. the per-step draws (K = 1:
+        the initial noise only, e.g. ``[timbres.initial_noise]`` to re-create a timbre; later draws then come from the RNG).  The
+        result's ``initial_noise`` is each row's train-width noise."""
         B = cond.shape[0]
         s = self.sampler_for(B, steps, cfg_scale, uncond)
         s.noise_feed = noise_feed
         init = None
         if noise_feed is not None:
             init = noise_feed[0][:B].to(self.device, torch.float32)
-            s.noise_feed = noise_feed[1:]
+            s.noise_feed = noise_feed[1:] if len(noise_feed) > 1 else None
         s.graph_tail, s.final_only = (self._tail_factory if decode else None), True
         imgs, _ = s.sample(self.unet, (B, self.channels, self.height, width), return_tensor=True, condition=cond.to(self.device),
                            sampler=sampler, initial_noise=init, seed=seed)
         latents = imgs[-1]
         if not decode:
             self.last_launches = s.last_graph_launches
-            return Timbres(latents, None, None, None)
-        return self._decode(s, latents)       # quantiser (text2sound.py:128), decoder (utils.py:224), iSTFT (utils.py:229-241): same graph
+            return Timbres(latents, None, None, None, s.last_reference_noise)
+        out = self._decode(s, latents)        # quantiser (text2sound.py:128), decoder (utils.py:224), iSTFT (utils.py:229-241): same graph
+        out.initial_noise = s.last_reference_noise
+        return out
+
+    # ---- timbre morphs (DiffSynthSampler.interpolate, model/DiffSynthSampler.py:224-269, from the pipeline) ------------------
+    @torch.no_grad()
+    def invert(self, latents: torch.Tensor, cond: torch.Tensor, uncond: Optional[torch.Tensor] = None, steps: int = 20,
+               cfg_scale: float = 1.0) -> torch.Tensor:
+        """DDIM inversion of latents [B,4,128,64] (e.g. encode_audio's) under their conditions [B, L]: the noises [B,4,128,64]
+        from which generate / morph re-create them, in one graph launch for the batch (DiffSynthSampler.ddim_invert, a port
+        extension).  The sampler is respaced to ``steps`` as generate's is (cached per batch and step count)."""
+        if latents.dim() != 4 or tuple(latents.shape[1:]) != (self.channels, self.height, 64):
+            raise ValueError(f"latents must be [B, {self.channels}, {self.height}, 64], got {tuple(latents.shape)}")
+        B = latents.shape[0]
+        if cond.dim() != 2 or cond.shape[0] != B:
+            raise ValueError(f"cond must be [{B}, L], got {tuple(cond.shape)}")
+        s = self._respaced_sampler(("invert", B, steps), B, steps)
+        s.activate_classifier_free_guidance(cfg_scale, uncond)
+        s.final_only = True
+        imgs, _ = s.ddim_invert(self.unet, latents, cond.to(self.device), return_tensor=True)
+        self.last_launches = s.last_graph_launches
+        return imgs[-1]
+
+    def _morph_endpoints(self, first_noise, second_noise, first_cond, second_cond, frames, path):
+        """Shape checks of morph (no device work): [P,4,128,64] / [4,128,64] noises and [P, L] / [L] conditions -> 4-D and 2-D views."""
+        if self.noise_strategy != "repeat":
+            raise ValueError(f"morph needs the 'repeat' noise strategy, not {self.noise_strategy!r}")
+        if path not in MORPH_PATHS:
+            raise ValueError(f"path must be one of {sorted(MORPH_PATHS)}, got {path!r}")
+        if isinstance(frames, bool) or int(frames) != frames or frames < 2:
+            raise ValueError(f"frames must be an integer >= 2, got {frames!r}")
+        nz = (self.channels, self.height, 64)
+        e = [x.unsqueeze(0) if x.dim() == 3 else x for x in (first_noise, second_noise)]
+        c = [x.unsqueeze(0) if x.dim() == 1 else x for x in (first_cond, second_cond)]
+        for x in e:
+            if x.dim() != 4 or tuple(x.shape[1:]) != nz:
+                raise ValueError(f"endpoint noises must be [P, {nz[0]}, {nz[1]}, {nz[2]}] or [{nz[0]}, {nz[1]}, {nz[2]}], got {tuple(x.shape)}")
+        for x in c:
+            if x.dim() != 2 or not x.is_floating_point():
+                raise ValueError(f"endpoint conditions must be floating [P, L] or [L], got {tuple(x.shape)} {x.dtype}")
+        if len({x.shape[0] for x in e + c}) != 1 or c[0].shape[1] != c[1].shape[1]:
+            raise ValueError(f"endpoints disagree: noises {[tuple(x.shape) for x in e]}, conditions {[tuple(x.shape) for x in c]}")
+        return e[0], e[1], c[0], c[1]
+
+    @torch.no_grad()
+    def morph(self, first_noise: torch.Tensor, second_noise: torch.Tensor, first_cond: torch.Tensor, second_cond: torch.Tensor,
+              uncond: Optional[torch.Tensor], frames: int, path: str = "slerp", steps: int = 20, cfg_scale: float = 6, width: int = 64,
+              sampler: str = "ddim", seed: Optional[int] = None, decode: bool = True) -> Timbres:
+        """P timbre morphs of ``frames`` frames each: frame k of sequence p starts from the noise between first_noise[p] and
+        second_noise[p] at a = k / (frames - 1) (``path`` "slerp", or "linear" = the reference's interpolate) under the linearly
+        interpolated condition, and the P * frames rows sample with classifier-free guidance and decode through the usual VQ ->
+        decoder -> iSTFT tail in ONE graph launch.  Endpoint noises are train-width noises [P,4,128,64] (``Timbres.initial_noise``
+        of generate, or invert of an upload); a [4,128,64] noise / [L] condition is P = 1.  Rows are sequence-major; the result's
+        initial_noise holds the rows' noises."""
+        e0, e1, c0, c1 = self._morph_endpoints(first_noise, second_noise, first_cond, second_cond, frames, path)
+        dev = self.device
+        noise, cond = morph_rows(e0.to(dev), e1.to(dev), c0.to(dev), c1.to(dev), int(frames), path)      # one ds_morph_rows
+        rows = noise.view(1, noise.shape[0], self.channels, self.height, 64)
+        return self.generate(cond, uncond, steps=steps, cfg_scale=cfg_scale, width=width, sampler=sampler, seed=seed, noise_feed=rows,
+                             decode=decode)
 
 
     # ---- timbre modification (sound2sound_with_text.py:47-269) -------------------------------------------------------
@@ -223,13 +291,7 @@ class TextToTimbre:
         B = cond.shape[0]
         width = guide_latent.shape[-1]
         n_steps = int(steps / strength)
-        key = ("modify", B, n_steps)
-        s = self._samplers.get(key)
-        if s is None:
-            s = DiffSynthSampler(self.timesteps, height=self.height, channels=self.channels, noise_strategy=self.noise_strategy,
-                                 mute=True, device=str(self.device), max_batchsize=B)
-            s.respace(list(np.linspace(0, self.timesteps - 1, n_steps, dtype=np.int32)))
-            self._samplers[key] = s
+        s = self._respaced_sampler(("modify", B, n_steps), B, n_steps)
         s.activate_classifier_free_guidance(cfg_scale, uncond)
         guide = guide_latent.to(self.device, torch.float32)
         if guide.shape[0] == 1 and B > 1:
@@ -280,13 +342,7 @@ class TextToTimbre:
         zoomed = torch.empty((len(items), 1, self.height, width), dtype=torch.float32, device=self.device)
         zoom_packed(torch.cat([m.to(self.device, torch.float32).reshape(-1) for m in items]), [tuple(m.shape) for m in items],
                     (self.height, width), out=zoomed)
-        key = ("inpaint", B, steps)
-        s = self._samplers.get(key)
-        if s is None:
-            s = DiffSynthSampler(self.timesteps, height=self.height, channels=self.channels, noise_strategy=self.noise_strategy,
-                                 mute=True, device=str(self.device), max_batchsize=B)
-            s.respace(list(np.linspace(0, self.timesteps - 1, steps, dtype=np.int32)))
-            self._samplers[key] = s
+        s = self._respaced_sampler(("inpaint", B, steps), B, steps)
         s.activate_classifier_free_guidance(cfg_scale, uncond)
         guide = guide_latent.to(self.device, torch.float32)
         if guide.shape[0] == 1 and B > 1:

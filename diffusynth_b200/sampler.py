@@ -2,7 +2,8 @@
 
 Same constructor, same public methods and return values:
 ``respace``, ``activate_classifier_free_guidance``, ``q_sample``, ``sample``, ``img_guided_sample``,
-``inpaint_sample``, ``interpolate`` -> ``(imgs: list[steps+1], initial_noise)``.
+``inpaint_sample``, ``interpolate`` -> ``(imgs: list[steps+1], initial_noise)``; ``ddim_invert`` is a port extension (DDIM inversion,
+no reference entry) in the same convention.
 
 What runs where:
   * schedule tables / respacing: numpy float64 on the host, as in the reference (:55-57,169-222);
@@ -80,6 +81,8 @@ class DiffSynthSampler:
         self.graph_tail = None
         self.last_tail = None
         self.final_only = False
+        # 'repeat' strategy: the train-width noise [B,C,H,train_width] the last p_sample_loop re-laid into its initial noise
+        self.last_reference_noise: Optional[torch.Tensor] = None
 
     # ---- schedule (host, float64) -----------------------------------------------------------
     def define_beta_schedule(self):
@@ -209,8 +212,9 @@ class DiffSynthSampler:
         return out
 
     @torch.no_grad()
-    def ddim_sample(self, model, x, t, condition=None, ddim_eta=0.0):
-        """One reverse step (:297-345) for a generic callable model; the update is the fused kernel."""
+    def ddim_sample(self, model, x, t, condition=None, ddim_eta=0.0, coef=None):
+        """One reverse step (:297-345) for a generic callable model; the update is the fused kernel.  ``coef``: the step's 8
+        ds_ddim_step coefficients instead of _coef(t, ddim_eta), with no noise draw (sigma must be 0; ddim_invert)."""
         B = x.shape[0]
         ti = int(t.reshape(-1)[0])
         mapped = torch.full((B,), self.timestep_map[ti], device=x.device, dtype=torch.long)
@@ -220,11 +224,15 @@ class DiffSynthSampler:
             u = self.unconditional_condition.unsqueeze(0).repeat(*([B] + [1] * len(self.unconditional_condition.shape)))
             out = model(torch.cat([x] * 2), torch.cat([mapped] * 2), torch.cat([u.to(condition.device), condition])).float().contiguous()
             eps_u, eps_c = out[:B], out[B:]
-        z, _ = self.get_deterministic_noise_tensor(B, x.shape[3])
-        coef = torch.tensor(self._coef(ti, ddim_eta), dtype=torch.float32, device=x.device)
+        z = None
+        if coef is None:
+            z, _ = self.get_deterministic_noise_tensor(B, x.shape[3])
+            z = z.contiguous()
+            coef = self._coef(ti, ddim_eta)
+        coef = torch.tensor(coef, dtype=torch.float32, device=x.device)
         xin = x.float().contiguous()
         nxt = torch.empty_like(xin)
-        ops.ddim_step(eps_u, eps_c, xin, z.contiguous(), coef, nxt)
+        ops.ddim_step(eps_u, eps_c, xin, z, coef, nxt)
         return nxt
 
     def p_sample(self, model, x, t, condition=None, sampler="ddim"):
@@ -277,6 +285,9 @@ class DiffSynthSampler:
         B, Wd = shape[0], shape[3]
         if initial_noise is not None:
             initial_noise = initial_noise.to(self.device, torch.float32)
+        elif self.noise_strategy == "repeat":
+            initial_noise = self._draw(B)           # the draw get_deterministic_noise_tensor_repeat would make, kept below
+        self.last_reference_noise = initial_noise if self.noise_strategy == "repeat" else None
         initial_noise, _ = self.get_deterministic_noise_tensor(B, Wd, reference_noise=initial_noise)
         initial_noise = initial_noise.contiguous()
         assert tuple(initial_noise.shape) == shape, "initial_noise.shape != shape"
@@ -330,7 +341,8 @@ class DiffSynthSampler:
             imgs.append(img)
         return imgs
 
-    def _run_graph_loop(self, model, shape, img, steps, eta, condition, guide_img, initial_noise, masks, inpaint):
+    def _run_graph_loop(self, model, shape, img, steps, eta, condition, guide_img, initial_noise, masks, inpaint, coef=None):
+        """``coef``: per-step ds_ddim_step coefficients instead of _coef(i, eta), with no per-step noise draw (ddim_invert)."""
         B, Cc, H, Wd = shape
         cfg_on = self.CFG != 1.0
         n_iter = len(steps)
@@ -345,7 +357,9 @@ class DiffSynthSampler:
             self._graphs[key] = loop
         # per-call inputs (device buffers the graph reads)
         loop.imgs[0].copy_(img)
-        coef = [self._coef(i, eta) for i in steps]
+        draw_steps = coef is None
+        if coef is None:
+            coef = [self._coef(i, eta) for i in steps]
         loop.coef.copy_(torch.tensor(coef, dtype=torch.float32))
         loop.ttab.copy_(torch.tensor([self.timestep_map[i] for i in steps], dtype=torch.long))
         cond = condition.to(self.device, loop.cond.dtype)          # fp32 [B, L] text conditions, or int64 [B] class labels
@@ -355,7 +369,7 @@ class DiffSynthSampler:
             loop.cond.copy_(torch.cat([u, cond]))
         else:
             loop.cond.copy_(cond)
-        if eta > 0 or self.faithful_rng:
+        if draw_steps and (eta > 0 or self.faithful_rng):
             for k in range(n_iter):
                 z, _ = self.get_deterministic_noise_tensor(B, Wd)
                 if eta > 0:
@@ -397,6 +411,47 @@ class DiffSynthSampler:
         linear_noise = self.generate_linear_noise(shape, variance, first_endpoint=first_endpoint, second_endpoint=second_endpoint)
         return self.p_sample_loop(model, shape, initial_noise=linear_noise, start_noise_level_ratio=1.0, end_noise_level_ratio=0.0,
                                   return_tensor=return_tensor, condition=condition, sampler=sampler)
+
+    def _invert_coef(self, t: int) -> List[float]:
+        """ds_ddim_step coefficients of inversion step t (x_t -> x_next): [sqrt(1-a_t), sqrt(a_t), sqrt(a_next), sqrt(1-a_next), 0,
+        CFG, 0, 0] from alphas_cumprod / alphas_cumprod_next, evaluated as _coef is (f64 table -> fp32 -> fp32 math)."""
+        at = torch.tensor(self.alphas_cumprod[t]).float()
+        an = torch.tensor(self.alphas_cumprod_next[t]).float()
+        return [float(torch.sqrt(1. - at)), float(torch.sqrt(at)), float(torch.sqrt(an)), float(torch.sqrt(1. - an)), 0.0,
+                float(self.CFG), 0.0, 0.0]
+
+    @torch.no_grad()
+    def ddim_invert(self, model, x0, condition, return_tensor=True):
+        """DDIM inversion (a port extension: the reference has no entry for it): the latents ``x0`` [B,C,H,train_width] are run
+        through the respaced timesteps in ASCENDING order, step t mapping x_t to sqrt(a_next) x0_pred + sqrt(1 - a_next) eps with the
+        schedule's alphas_cumprod_next (0 after the last step, so the result is the model's noise prediction), under the active
+        classifier-free guidance.  With a ConditionedUnet the steps run through the same captured graph as sample() (no tail).
+        Returns ``(imgs, None)``: imgs[0] = x0, imgs[k] after k steps, imgs[-1] the noise; numpy after imgs[0] unless return_tensor.
+        Only the 'repeat' strategy at the train width is supported."""
+        if self.noise_strategy != "repeat":
+            raise NotImplementedError("ddim_invert supports the 'repeat' noise strategy only")
+        shape = tuple(int(s) for s in x0.shape)
+        if len(shape) != 4 or shape[1:] != (self.channels, self.height, self.train_width):
+            raise ValueError(f"x0 must be [B, {self.channels}, {self.height}, {self.train_width}], got {shape}")
+        if condition is None:
+            raise ValueError("ddim_invert needs a condition")
+        steps = list(range(0, self.num_timesteps))
+        coef = [self._invert_coef(i) for i in steps]
+        img = x0.to(self.device, torch.float32).contiguous()
+        if isinstance(model, ConditionedUnet):
+            tail, self.graph_tail = self.graph_tail, None
+            try:
+                imgs = self._run_graph_loop(model, shape, img, steps, 0.0, condition, None, None, None, False, coef=coef)
+            finally:
+                self.graph_tail = tail
+        else:
+            imgs = [img]
+            for i, c in zip(steps, coef):
+                imgs.append(self.ddim_sample(model, imgs[-1], torch.full((shape[0],), i, device=self.device, dtype=torch.long),
+                                             condition=condition, coef=c))
+        if not return_tensor:
+            imgs = [imgs[0]] + [im.cpu().numpy() for im in imgs[1:]]
+        return imgs, None
 
     def img_guided_sample(self, model, shape, noising_strength, guide_img, return_tensor=False, condition=None, sampler="ddim",
                           initial_noise=None, seed=None):

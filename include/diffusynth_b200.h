@@ -302,6 +302,28 @@ int ds_mask_zoom(const float* d_in, float* d_out, const long long* in_shapes, co
                  long long ws_bytes, void* stream);
 
 /* ----------------------------------------------------------------------------------------
+ * Timbre morph rows (model/DiffSynthSampler.py:224-269, generate_linear_noise with both endpoints, as interpolate uses it, batched):
+ * P sequences x N frames (N >= 2), row p*N + k = frame k of sequence p, a = k / (N - 1).  d_e0 / d_e1: endpoint noises [P, n] fp32
+ * (n % 4 == 0; n = 4*128*64 for the repeat strategy's train-width noise), d_c0 / d_c1: endpoint conditions [P, L] fp32.  Writes
+ * d_noise [P*N, n] and d_cond [P*N, L].
+ *   DS_MORPH_LINEAR (:170-174): fl(fl(a e1) + fl((1 - a) e0)) with a, 1 - a evaluated in double and rounded to fp32 (as torch
+ *     rounds a Python scalar), no FMA contraction: bit-identical to generate_linear_noise.
+ *   DS_MORPH_SLERP (no reference entry): theta = acos(clamp(<e0,e1> / (|e0| |e1|), -1, 1)) per sequence from a float64 reduction in
+ *     a fixed order; row = fl(w0 e0 + w1 e1), w0 = sin((1 - a) theta) / sin theta, w1 = sin(a theta) / sin theta, in float64.  A
+ *     sequence with sin theta < 1e-6 (identical or antipodal endpoints) or a zero endpoint takes the linear rows.  Frames 0 and
+ *     N - 1 equal the endpoints exactly.
+ * Conditions always take the linear expression, except that an element equal in both endpoints is copied as it is (so equal
+ * conditions give every frame exactly that condition).  A sequence's rows do not depend on P (bit for bit) and repeat run to run.  Every
+ * argument is checked before any device work, including P * N * max(n, L) in int64; no host synchronisation.  Launches: 1 (linear),
+ * 2 (slerp).  d_ws: ds_morph_rows_workspace bytes (0 for the linear path, where d_ws may be NULL).
+ * -------------------------------------------------------------------------------------- */
+#define DS_MORPH_LINEAR 0
+#define DS_MORPH_SLERP 1
+int ds_morph_rows_workspace(int P, int N, long long n, long long L, int path, long long* bytes);
+int ds_morph_rows(const float* d_e0, const float* d_e1, const float* d_c0, const float* d_c1, int P, int N, long long n, long long L,
+                  int path, float* d_noise, float* d_cond, void* d_ws, long long ws_bytes, void* stream);
+
+/* ----------------------------------------------------------------------------------------
  * Image products of the decode glue (webUI/natural_language_guided_4/utils.py), batched:
  *   spectrogram_to_Gradio_image (:8-50, with tools.np_power_to_db tools.py:41-50) and phase_to_Gradio_image (:53-91)
  *   of |D| / angle(D) for D = depad_STFT(decode_stft(spec)) (:229-238): uint8 [B, 513, T, 3], flipped vertically;
