@@ -73,6 +73,45 @@ def _device():
     return torch.device("cuda", torch.cuda.current_device())
 
 
+def _layout(x, item_dim: int, what: str = "unsupported layout"):
+    """Host side of _pack: a list of ``item_dim``-D arrays / tensors (1-D signals, 2-D masks), one of them, or a batch of them
+    along a leading axis -> (the arrays to pack, each item's shape, the layout for _unpack).  ValueError(``what``) for any other
+    number of axes, and for an empty batch."""
+    if isinstance(x, (list, tuple)):
+        parts, kind = list(x), "list"
+        shapes = [tuple(np.shape(a)) for a in parts]
+        if any(len(s) != item_dim for s in shapes):
+            raise ValueError(what)
+    else:
+        s = tuple(np.shape(x))
+        if len(s) not in (item_dim, item_dim + 1):
+            raise ValueError(what)
+        parts, kind = [x], "one" if len(s) == item_dim else "batch"
+        shapes = [s] if kind == "one" else [s[1:]] * s[0]
+    if not shapes:
+        raise ValueError("nothing to do: the batch is empty")
+    return parts, shapes, (kind, isinstance(parts[0], np.ndarray))
+
+
+def _pack(parts, device=None) -> torch.Tensor:
+    """The arrays / tensors of _layout back to back in one fp32 tensor on ``device`` (by default the first one's CUDA device, else
+    the current one)."""
+    ts = [torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32)) if isinstance(a, np.ndarray) else torch.as_tensor(a) for a in parts]
+    dev = device if device is not None else ts[0].device if ts[0].is_cuda else _device()
+    ts = [t.reshape(-1).to(dev, torch.float32) for t in ts]
+    return torch.cat(ts) if len(ts) > 1 else ts[0]
+
+
+def _unpack(out: torch.Tensor, shapes, layout):
+    """A packed result whose items have ``shapes``, in the layout _layout read: a list, one item or a batch (numpy in, numpy out)."""
+    kind, is_np = layout
+    if kind == "list":
+        parts = [p.view(s) for p, s in zip(torch.split(out, [int(np.prod(s)) for s in shapes]), shapes)]
+        return [p.cpu().numpy() for p in parts] if is_np else parts
+    res = out.view(shapes[0] if kind == "one" else (len(shapes),) + tuple(shapes[0]))
+    return res.cpu().numpy() if is_np else res
+
+
 def decode_stft(encoded_D: np.ndarray) -> np.ndarray:
     """tools.decode_stft (:334-345): [3, F, T] (log1p magnitude, cos, sin) -> complex [F, T], evaluated by ds_decode_stft in the
     precision of the input (float32 -> complex64, float64 -> complex128), like numpy."""
@@ -189,26 +228,8 @@ def pitch_shift(waves, n_steps):
     with librosa's default STFT arguments; the resampler is a Kaiser-windowed sinc (resampy kaiser_best) instead of librosa's soxr.
     ``waves``: a [B, L] or [L] tensor / numpy array, or a list of 1-D ones of different lengths; ``n_steps``: a scalar or one per
     item, finite, |n_steps| <= 24.  Returns the same layout (numpy in, numpy out; fp32)."""
-    is_list = isinstance(waves, (list, tuple))
-    items = list(waves) if is_list else None
-    if not is_list:
-        arr = waves
-        if arr.ndim == 1:
-            items = [arr]
-        else:
-            assert arr.ndim == 2, "expected [B, L], [L] or a list of 1-D signals"
-            items = [arr[b] for b in range(arr.shape[0])]
-    is_np = isinstance(items[0], np.ndarray)
-    dev = _device() if is_np or not items[0].is_cuda else items[0].device
-    ts = [(torch.from_numpy(np.ascontiguousarray(w, dtype=np.float32)) if is_np else w).reshape(-1).to(dev, torch.float32)
-          for w in items]
-    lengths = [t.numel() for t in ts]
-    out = pitch_shift_packed(torch.cat(ts), lengths, n_steps)
-    parts = list(torch.split(out, lengths))
-    if is_list:
-        return [p.cpu().numpy() for p in parts] if is_np else parts
-    res = out.view(len(lengths), lengths[0]) if waves.ndim == 2 else out
-    return res.cpu().numpy() if is_np else res
+    parts, shapes, layout = _layout(waves, 1, "expected [B, L], [L] or a list of 1-D signals")
+    return _unpack(pitch_shift_packed(_pack(parts), [n for n, in shapes], n_steps), shapes, layout)
 
 
 @torch.no_grad()
@@ -216,6 +237,13 @@ def mix_track(packed: torch.Tensor, src_offsets, lengths, onsets, gains, track_l
     """Place and sum notes into one fp32 track (ds_mix_track): note n is ``packed[src_offsets[n] : src_offsets[n] + lengths[n]]``
     times gains[n], starting at sample onsets[n]; notes may share a source.  Summed in note order, bit-identical run to run.
     ``track_len`` defaults to the end of the last note."""
+    return _mix(packed, src_offsets, lengths, onsets, gains, track_len)
+
+
+def _mix(packed: torch.Tensor, src_offsets, lengths, onsets, gains, track_len, fade: Optional[np.ndarray] = None,
+         peak: float = 0.0) -> torch.Tensor:
+    """mix_track (``fade`` None: ds_mix_track) or mix_arrangement (int64 ``fade``: ds_mix_arrangement, whose extra arguments are
+    the fades before the note count and the peak after it): host arrays, workspace query, allocation, launch."""
     lib = _lib.load()
     off = np.ascontiguousarray(src_offsets, dtype=np.int64)
     L = np.ascontiguousarray(lengths, dtype=np.int64)
@@ -224,13 +252,14 @@ def mix_track(packed: torch.Tensor, src_offsets, lengths, onsets, gains, track_l
     K = len(L)
     if track_len is None:
         track_len = int((on + L).max())
+    name, fk = ("ds_mix_track", (K,)) if fade is None else ("ds_mix_arrangement", (fade.ctypes.data, K, peak))
     nbytes = C.c_longlong(0)
-    check(lib.ds_mix_track_workspace(L.ctypes.data, on.ctypes.data, K, int(track_len), C.byref(nbytes)), "ds_mix_track_workspace")
+    check(getattr(lib, name + "_workspace")(L.ctypes.data, on.ctypes.data, *fk, int(track_len), C.byref(nbytes)), name + "_workspace")
     packed = packed.float().contiguous()
     ws = torch.empty((nbytes.value,), dtype=torch.uint8, device=packed.device)
     track = torch.empty((int(track_len),), dtype=torch.float32, device=packed.device)
-    check(lib.ds_mix_track(packed.data_ptr(), off.ctypes.data, L.ctypes.data, on.ctypes.data, g.ctypes.data, K, track.data_ptr(),
-                           int(track_len), ws.data_ptr(), nbytes.value, ops._stream()), "ds_mix_track")
+    check(getattr(lib, name)(packed.data_ptr(), off.ctypes.data, L.ctypes.data, on.ctypes.data, g.ctypes.data, *fk, track.data_ptr(),
+                             int(track_len), ws.data_ptr(), nbytes.value, ops._stream()), name)
     return track
 
 
@@ -250,27 +279,11 @@ def mix_arrangement(packed: torch.Tensor, src_offsets, lengths, onsets, gains, f
     """mix_track with a linear fade over the last fade_out[n] samples of every note (clamped to the note; 0 = none) and, when
     ``target_peak`` is given, the track scaled on the device so that max |track| == target_peak (ds_mix_arrangement).  Notes
     without a fade are summed exactly as mix_track sums them.  Summed in note order, bit-identical run to run."""
-    lib = _lib.load()
-    off = np.ascontiguousarray(src_offsets, dtype=np.int64)
-    L = np.ascontiguousarray(lengths, dtype=np.int64)
-    on = np.ascontiguousarray(onsets, dtype=np.int64)
-    g = np.ascontiguousarray(gains, dtype=np.float32)
     fade = np.ascontiguousarray(fade_out, dtype=np.int64)
     peak = _check_peak(target_peak)
     if np.any(fade < 0):
         raise ValueError(f"fade_out must be >= 0, got {fade_out}")
-    K = len(L)
-    if track_len is None:
-        track_len = int((on + L).max())
-    nbytes = C.c_longlong(0)
-    check(lib.ds_mix_arrangement_workspace(L.ctypes.data, on.ctypes.data, fade.ctypes.data, K, peak, int(track_len), C.byref(nbytes)),
-          "ds_mix_arrangement_workspace")
-    packed = packed.float().contiguous()
-    ws = torch.empty((nbytes.value,), dtype=torch.uint8, device=packed.device)
-    track = torch.empty((int(track_len),), dtype=torch.float32, device=packed.device)
-    check(lib.ds_mix_arrangement(packed.data_ptr(), off.ctypes.data, L.ctypes.data, on.ctypes.data, g.ctypes.data, fade.ctypes.data, K,
-                                 peak, track.data_ptr(), int(track_len), ws.data_ptr(), nbytes.value, ops._stream()), "ds_mix_arrangement")
-    return track
+    return _mix(packed, src_offsets, lengths, onsets, gains, track_len, fade, peak)
 
 
 def shift_and_mix(sources, semitones, note_source, onsets, gains, fades=None, target_peak: Optional[float] = None) -> torch.Tensor:
@@ -344,30 +357,13 @@ def resample(y, orig_sr, target_sr):
     Kaiser-windowed sinc, evaluated through a polyphase table; equal rates return the input).  ``y``: a [B, L] or [L] tensor /
     numpy array, or a list of 1-D ones of different lengths; rates: integers, a scalar or one per item.  The output has librosa's
     length ceil(L * target_sr / orig_sr) and the input's layout (numpy in, numpy out; fp32)."""
-    is_list = isinstance(y, (list, tuple))
-    if is_list:
-        items = list(y)
-        if not items or any(np.ndim(w) != 1 for w in items):
-            raise ValueError("expected a non-empty list of 1-D signals")
-    else:
-        if np.ndim(y) not in (1, 2):
-            raise ValueError("expected [B, L], [L] or a list of 1-D signals")
-        items = [y] if np.ndim(y) == 1 else [y[b] for b in range(y.shape[0])]
-    B = len(items)
-    o, t = _check_rates(orig_sr, B, "orig_sr"), _check_rates(target_sr, B, "target_sr")
-    if not is_list and np.ndim(y) == 2 and len(set(resample_length(y.shape[1], a, b) for a, b in zip(o, t))) > 1:
+    parts, shapes, layout = _layout(y, 1, "expected [B, L], [L] or a list of 1-D signals")
+    lengths = [n for n, in shapes]
+    o, t = _check_rates(orig_sr, len(lengths), "orig_sr"), _check_rates(target_sr, len(lengths), "target_sr")
+    n_out = [(resample_length(n, a, b),) for n, a, b in zip(lengths, o, t)]
+    if layout[0] == "batch" and len(set(n_out)) > 1:
         raise ValueError("a [B, L] input needs rates that give every row the same output length; pass a list instead")
-    is_np = isinstance(items[0], np.ndarray)
-    dev = _device() if is_np or not items[0].is_cuda else items[0].device
-    ts = [(torch.from_numpy(np.ascontiguousarray(w, dtype=np.float32)) if is_np else w).reshape(-1).to(dev, torch.float32) for w in items]
-    lengths = [x.numel() for x in ts]
-    res = resample_packed(torch.cat(ts), lengths, o, t)
-    n_out = [resample_length(n, a, b) for n, a, b in zip(lengths, o, t)]
-    if is_list:
-        parts = list(torch.split(res, n_out))
-        return [p.cpu().numpy() for p in parts] if is_np else parts
-    res = res.view(B, n_out[0]) if np.ndim(y) == 2 else res
-    return res.cpu().numpy() if is_np else res
+    return _unpack(resample_packed(_pack(parts), lengths, o, t), n_out, layout)
 
 
 # ---- mask zoom (scipy.ndimage.zoom of the inpainting-with-text mask to the latent grid, inpaint_with_text.py) --------------------
@@ -448,18 +444,8 @@ def zoom(input, zoom, output=None, order=3, mode="constant", cval=0.0, prefilter
     if output is not None or order != 3 or mode != "constant" or cval != 0.0 or prefilter is not True or grid_mode is not False:
         raise NotImplementedError("only scipy.ndimage.zoom's defaults (order=3, mode='constant', cval=0, prefilter=True, "
                                   "grid_mode=False, no output array) are implemented")
-    is_list = isinstance(input, (list, tuple))
-    if is_list:
-        items = list(input)
-        if any(np.ndim(a) != 2 for a in items):
-            raise ValueError("expected a list of 2-D arrays")
-    else:
-        if np.ndim(input) not in (2, 3):
-            raise ValueError("expected a [H, W] or [B, H, W] array, or a list of 2-D arrays")
-        items = [input] if np.ndim(input) == 2 else [input[b] for b in range(input.shape[0])]
-    B = len(items)
-    if B == 0:
-        raise ValueError("nothing to zoom: the batch is empty")
+    parts, ins, layout = _layout(input, 2, "expected a [H, W] or [B, H, W] array, or a list of 2-D arrays")
+    B, is_list = len(ins), layout[0] == "list"
     z = np.asarray(zoom, dtype=np.float64)
     if z.ndim == 0:
         z = np.full((B, 2), float(z))
@@ -471,20 +457,9 @@ def zoom(input, zoom, output=None, order=3, mode="constant", cval=0.0, prefilter
         raise ValueError(f"zoom must be a scalar or a (rows, cols) pair{', or one per item' if is_list else ''}, got {zoom!r}")
     if not np.all(np.isfinite(z)) or (z <= 0).any():
         raise ValueError(f"zoom factors must be finite and positive, got {zoom!r}")
-    ins = [tuple(int(n) for n in np.shape(a)) for a in items]
     outs = [tuple(int(round(n * f)) for n, f in zip(s, zk)) for s, zk in zip(ins, z)]        # scipy: round(n * zoom), Python's round
     in_shapes, out_shapes = _shapes(ins, B, "the input shape"), _shapes(outs, B, "the output shape")
-    is_np = isinstance(items[0], np.ndarray)
-    dev = _device() if is_np or not items[0].is_cuda else items[0].device
-    ts = [(torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32)) if is_np else a).reshape(-1).to(dev, torch.float32)
-          for a in items]
-    res = zoom_packed(torch.cat(ts), in_shapes, out_shapes)
-    sizes = [h * w for h, w in outs]
-    if is_list:
-        parts = [p.view(s) for p, s in zip(torch.split(res, sizes), outs)]
-        return [p.cpu().numpy() for p in parts] if is_np else parts
-    res = res.view(outs[0]) if np.ndim(input) == 2 else res.view((B,) + outs[0])
-    return res.cpu().numpy() if is_np else res
+    return _unpack(zoom_packed(_pack(parts), in_shapes, out_shapes), outs, layout)
 
 
 @torch.no_grad()

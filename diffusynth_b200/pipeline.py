@@ -11,8 +11,8 @@ import torch
 
 from . import _lib, ops, weights as W
 from ._lib import check
-from .codec import MORPH_PATHS, SAMPLE_RATE, morph_rows, resample_packed, shift_and_mix, spectrogram_to_waveform, waveform_to_spectrogram, \
-    zoom_packed
+from .codec import MORPH_PATHS, SAMPLE_RATE, _layout, _pack, morph_rows, resample_packed, shift_and_mix, spectrogram_to_waveform, \
+    waveform_to_spectrogram, zoom_packed
 from .sampler import DiffSynthSampler
 from .unet import ConditionedUnet
 from .vqgan import VQGAN
@@ -24,7 +24,7 @@ class Timbres:
     quantized: torch.Tensor      # [B,4,128,W]
     spectrograms: torch.Tensor   # [B,3,512,4W]
     waveforms: torch.Tensor      # [B, 256*(4W-1)]
-    initial_noise: Optional[torch.Tensor] = None     # [B,4,128,64] train-width noise each row started from (generate / morph)
+    initial_noise: Optional[torch.Tensor] = None     # [B,4,128,64] train-width noise each row started from
 
 
 @dataclass
@@ -130,13 +130,33 @@ class TextToTimbre:
         assert t is not None and t.src.shape[0] == batch and t.src.shape[3] == width, "no generate() call with this shape yet"
         return t if isinstance(t, _Tail) else _Tail(self.vqgan, t.src)
 
-    def _decode(self, s: DiffSynthSampler, latents: torch.Tensor) -> Timbres:
-        """Results of the tail that ran inside the sampler's graph (copied out of its static buffers)."""
+    def _run(self, s: DiffSynthSampler, call, B: int, noise_feed, decode: bool) -> Timbres:
+        """One sampling call of B rows on ``s`` (guidance already active): ``call(initial_noise)`` runs the sampler's entry point;
+        ``noise_feed`` as generate takes it.  With ``decode`` the quantiser (text2sound.py:128), decoder (utils.py:224) and iSTFT
+        (utils.py:229-241) run in the sampling graph and their results are copied out of its static buffers."""
+        init = None
+        s.noise_feed = None
+        if noise_feed is not None:
+            init = noise_feed[0][:B].to(self.device, torch.float32)
+            s.noise_feed = noise_feed[1:] if len(noise_feed) > 1 else None
+        s.graph_tail, s.final_only = (self._tail_factory if decode else None), True
+        imgs, _ = call(init)
+        self.last_launches = s.last_graph_launches
+        if not decode:
+            return Timbres(imgs[-1], None, None, None, s.last_reference_noise)
         t = s.last_tail
         self._last_tail = t
-        self.last_launches = s.last_graph_launches
         self.vqgan._vq_vae.last_indices = t.idx.clone()
-        return Timbres(latents, t.q.clone(), t.spec.clone(), t.wave.clone())
+        return Timbres(imgs[-1], t.q.clone(), t.spec.clone(), t.wave.clone(), s.last_reference_noise)
+
+    def _rows(self, x: torch.Tensor, B: int, what: str, trailing: tuple) -> torch.Tensor:
+        """``x`` [1 or B, *trailing] (a name in ``trailing``: any size) on the device as B rows: one row is repeated."""
+        if x.dim() != 1 + len(trailing) or x.shape[0] not in (1, B) or \
+                any(isinstance(t, int) and n != t for n, t in zip(x.shape[1:], trailing)):
+            dims = ", ".join(str(t) for t in trailing)
+            raise ValueError(f"{what} must be [{'1' if B == 1 else f'1 or {B}'}, {dims}], got {tuple(x.shape)}")
+        x = x.to(self.device)
+        return x.repeat(B, *([1] * len(trailing))) if x.shape[0] < B else x
 
     @classmethod
     def random_init(cls, device="cuda", seed: int = 0, perturb_norm: bool = False, batch_invariant: bool = False) -> "TextToTimbre":
@@ -150,18 +170,19 @@ class TextToTimbre:
 
     def sampler_for(self, batch: int, steps: int, cfg_scale: float, uncond: Optional[torch.Tensor]) -> DiffSynthSampler:
         """text2sound.py:96-106: fresh sampler, CFG activated, respaced to ``steps`` (cached per (batch, steps))."""
-        s = self._respaced_sampler((batch, steps), batch, steps)
-        s.activate_classifier_free_guidance(cfg_scale, uncond)
-        return s
+        return self._respaced_sampler((batch, steps), batch, steps, cfg_scale, uncond)
 
-    def _respaced_sampler(self, key, batch: int, n_steps: int) -> DiffSynthSampler:
-        """A sampler of ``batch`` rows respaced to ``n_steps`` as text2sound.py:96-106 builds it, cached under ``key``."""
+    def _respaced_sampler(self, key, batch: int, n_steps: int, cfg_scale: float, uncond: Optional[torch.Tensor],
+                          noise_strategy: Optional[str] = None) -> DiffSynthSampler:
+        """A sampler of ``batch`` rows respaced to ``n_steps`` as text2sound.py:96-106 builds it (``noise_strategy``: the pipeline's
+        by default), cached under ``key``, with classifier-free guidance activated."""
         s = self._samplers.get(key)
         if s is None:
-            s = DiffSynthSampler(self.timesteps, height=self.height, channels=self.channels, noise_strategy=self.noise_strategy,
-                                 mute=True, device=str(self.device), max_batchsize=batch)
+            s = DiffSynthSampler(self.timesteps, height=self.height, channels=self.channels, mute=True, device=str(self.device),
+                                 max_batchsize=batch, noise_strategy=noise_strategy or self.noise_strategy)
             s.respace(list(np.linspace(0, self.timesteps - 1, n_steps, dtype=np.int32)))
             self._samplers[key] = s
+        s.activate_classifier_free_guidance(cfg_scale, uncond)
         return s
 
     @torch.no_grad()
@@ -183,21 +204,9 @@ class TextToTimbre:
         result's ``initial_noise`` is each row's train-width noise."""
         B = cond.shape[0]
         s = self.sampler_for(B, steps, cfg_scale, uncond)
-        s.noise_feed = noise_feed
-        init = None
-        if noise_feed is not None:
-            init = noise_feed[0][:B].to(self.device, torch.float32)
-            s.noise_feed = noise_feed[1:] if len(noise_feed) > 1 else None
-        s.graph_tail, s.final_only = (self._tail_factory if decode else None), True
-        imgs, _ = s.sample(self.unet, (B, self.channels, self.height, width), return_tensor=True, condition=cond.to(self.device),
-                           sampler=sampler, initial_noise=init, seed=seed)
-        latents = imgs[-1]
-        if not decode:
-            self.last_launches = s.last_graph_launches
-            return Timbres(latents, None, None, None, s.last_reference_noise)
-        out = self._decode(s, latents)        # quantiser (text2sound.py:128), decoder (utils.py:224), iSTFT (utils.py:229-241): same graph
-        out.initial_noise = s.last_reference_noise
-        return out
+        return self._run(s, lambda init: s.sample(self.unet, (B, self.channels, self.height, width), return_tensor=True,
+                                                  condition=cond.to(self.device), sampler=sampler, initial_noise=init, seed=seed),
+                         B, noise_feed, decode)
 
     # ---- timbre morphs (DiffSynthSampler.interpolate, model/DiffSynthSampler.py:224-269, from the pipeline) ------------------
     @torch.no_grad()
@@ -211,8 +220,7 @@ class TextToTimbre:
         B = latents.shape[0]
         if cond.dim() != 2 or cond.shape[0] != B:
             raise ValueError(f"cond must be [{B}, L], got {tuple(cond.shape)}")
-        s = self._respaced_sampler(("invert", B, steps), B, steps)
-        s.activate_classifier_free_guidance(cfg_scale, uncond)
+        s = self._respaced_sampler(("invert", B, steps), B, steps, cfg_scale, uncond)
         s.final_only = True
         imgs, _ = s.ddim_invert(self.unet, latents, cond.to(self.device), return_tensor=True)
         self.last_launches = s.last_graph_launches
@@ -266,17 +274,14 @@ class TextToTimbre:
         clip.  Normalisation, resampling and the length adjustment are one ds_resample call writing the STFT's input (a 16 kHz clip
         is copied).  Returns the UN-quantised latent [B,4,128,w] (:107)."""
         if isinstance(wave, (list, tuple)):
-            clips = [torch.as_tensor(w) for w in wave]
-            if not clips or any(c.dim() != 1 for c in clips):
+            if not wave or any(np.ndim(c) != 1 for c in wave):
                 raise ValueError("expected a non-empty list of 1-D clips")
-            packed, lengths = torch.cat([c.to(self.device, torch.float32) for c in clips]), [c.numel() for c in clips]
-        else:
-            wave = torch.as_tensor(wave)
-            if wave.dim() != 2:
-                raise ValueError("expected a [B, L] batch or a list of 1-D clips")
-            packed, lengths = wave.to(self.device, torch.float32).reshape(-1), [wave.shape[1]] * wave.shape[0]
-        B, n = len(lengths), 256 * (4 * width - 1)
-        wave = resample_packed(packed, lengths, sample_rate, SAMPLE_RATE, out_lengths=n, normalize_peak=True).view(B, n)   # :75-82
+        elif np.ndim(wave) != 2:
+            raise ValueError("expected a [B, L] batch or a list of 1-D clips")
+        parts, shapes, _ = _layout(wave, 1)
+        B, n = len(shapes), 256 * (4 * width - 1)
+        wave = resample_packed(_pack(parts, self.device), [L for L, in shapes], sample_rate, SAMPLE_RATE, out_lengths=n,
+                               normalize_peak=True).view(B, n)                                             # :75-82
         # pad_STFT(D) is called with its default time_resolution = 256 frames and never crops (tools.py:170-182): clips of
         # <= 3 s (width <= 64) always encode to a 64-column latent, longer ones to ``width`` columns
         spec = waveform_to_spectrogram(wave, time_resolution=max(256, 4 * width))          # :85-94
@@ -289,26 +294,14 @@ class TextToTimbre:
         """sound2sound_sample (:126-269): respace to int(steps/strength) (:185), img_guided_sample(noising_strength=strength,
         guide_img=latent.repeat(B)) (:194-203), then the same VQ -> decoder -> iSTFT tail as text-to-timbre."""
         B = cond.shape[0]
-        width = guide_latent.shape[-1]
+        guide = self._rows(guide_latent, B, "guide_latent", (self.channels, self.height, "w")).float()
+        width = guide.shape[-1]
         n_steps = int(steps / strength)
-        s = self._respaced_sampler(("modify", B, n_steps), B, n_steps)
-        s.activate_classifier_free_guidance(cfg_scale, uncond)
-        guide = guide_latent.to(self.device, torch.float32)
-        if guide.shape[0] == 1 and B > 1:
-            guide = guide.repeat(B, 1, 1, 1)
-        init = None
-        s.noise_feed = None
-        if noise_feed is not None:
-            init = noise_feed[0][:B].to(self.device, torch.float32)
-            s.noise_feed = noise_feed[1:]
-        s.graph_tail, s.final_only = (self._tail_factory if decode else None), True
-        imgs, _ = s.img_guided_sample(self.unet, (B, self.channels, self.height, width), strength, guide, return_tensor=True,
-                                      condition=cond.to(self.device), sampler=sampler, initial_noise=init, seed=seed)
-        latents = imgs[-1]
-        if not decode:
-            self.last_launches = s.last_graph_launches
-            return Timbres(latents, None, None, None)
-        return self._decode(s, latents)
+        s = self._respaced_sampler(("modify", B, n_steps), B, n_steps, cfg_scale, uncond)
+        return self._run(s, lambda init: s.img_guided_sample(self.unet, (B, self.channels, self.height, width), strength, guide,
+                                                             return_tensor=True, condition=cond.to(self.device), sampler=sampler,
+                                                             initial_noise=init, seed=seed),
+                         B, noise_feed, decode)
 
     # ---- inpainting with text (inpaint_with_text.py:140-333) ----------------------------------------------------------
     @torch.no_grad()
@@ -324,83 +317,27 @@ class TextToTimbre:
         [B, H, W] one, or a list of B 2-D ones of any shapes.  All masks go through ONE ds_mask_zoom into the [B, 1, 128, w]
         mask the sampling graph reads.  The sampler is respaced to ``steps`` (cached per (batch, steps)), as generate does."""
         B = cond.shape[0]
-        if guide_latent.dim() != 4 or guide_latent.shape[0] not in (1, B) or tuple(guide_latent.shape[1:3]) != (self.channels, self.height):
-            raise ValueError(f"guide_latent must be [1 or {B}, {self.channels}, {self.height}, w], got {tuple(guide_latent.shape)}")
-        width = guide_latent.shape[-1]
+        guide = self._rows(guide_latent, B, "guide_latent", (self.channels, self.height, "w")).float()
+        width = guide.shape[-1]
         if isinstance(mask, (list, tuple)):
-            items = [torch.as_tensor(m) for m in mask]
-            if len(items) != B or any(m.dim() != 2 for m in items):
+            if len(mask) != B or any(np.ndim(m) != 2 for m in mask):
                 raise ValueError(f"a list mask must hold {B} 2-D arrays")
-        else:
-            m = torch.as_tensor(mask)
-            if m.dim() == 2:
-                items = [m]
-            elif m.dim() == 3 and m.shape[0] == B:
-                items = list(m)
-            else:
-                raise ValueError(f"mask must be 2-D, [{B}, H, W] or a list of {B} 2-D arrays, got shape {tuple(m.shape)}")
-        zoomed = torch.empty((len(items), 1, self.height, width), dtype=torch.float32, device=self.device)
-        zoom_packed(torch.cat([m.to(self.device, torch.float32).reshape(-1) for m in items]), [tuple(m.shape) for m in items],
-                    (self.height, width), out=zoomed)
-        s = self._respaced_sampler(("inpaint", B, steps), B, steps)
-        s.activate_classifier_free_guidance(cfg_scale, uncond)
-        guide = guide_latent.to(self.device, torch.float32)
-        if guide.shape[0] == 1 and B > 1:
-            guide = guide.repeat(B, 1, 1, 1)
-        init = None
-        s.noise_feed = None
-        if noise_feed is not None:
-            init = noise_feed[0][:B].to(self.device, torch.float32)
-            s.noise_feed = noise_feed[1:]
-        s.graph_tail, s.final_only = (self._tail_factory if decode else None), True
-        imgs, _ = s.inpaint_sample(self.unet, (B, self.channels, self.height, width), noising_strength, guide, zoomed, return_tensor=True,
-                                   condition=cond.to(self.device), sampler=sampler, initial_noise=init, seed=seed)
-        latents = imgs[-1]
-        if not decode:
-            self.last_launches = s.last_graph_launches
-            return Timbres(latents, None, None, None)
-        return self._decode(s, latents)
+        elif not (np.ndim(mask) == 2 or np.ndim(mask) == 3 and np.shape(mask)[0] == B):
+            raise ValueError(f"mask must be 2-D, [{B}, H, W] or a list of {B} 2-D arrays, got shape {tuple(np.shape(mask))}")
+        parts, shapes, _ = _layout(mask, 2)
+        zoomed = torch.empty((len(shapes), 1, self.height, width), dtype=torch.float32, device=self.device)
+        zoom_packed(_pack(parts, self.device), shapes, (self.height, width), out=zoomed)
+        s = self._respaced_sampler(("inpaint", B, steps), B, steps, cfg_scale, uncond)
+        return self._run(s, lambda init: s.inpaint_sample(self.unet, (B, self.channels, self.height, width), noising_strength, guide,
+                                                          zoomed, return_tensor=True, condition=cond.to(self.device), sampler=sampler,
+                                                          initial_noise=init, seed=seed),
+                         B, noise_feed, decode)
 
 
     # ---- per-note synthesis for arrangements (track_maker.py:228-283) ---------------------------------------------------
     @staticmethod
     def note_width(duration_sec: float, time_resolution: int = 256, vae_scale: int = 4) -> int:
         return int(time_resolution * ((duration_sec + 1) / 4) / vae_scale)                                    # track_maker.py:245
-
-    @torch.no_grad()
-    def _synthesize_group(self, instrument_latent, condition, width: int, B: int, sample_steps, noising_strength, attack, before_release,
-                          sampler, time_resolution, vae_scale, noise_feed) -> Timbres:
-        """B notes of one width as ONE batched inpainting run (one graph launch): every note is an independent sample of the batch
-        (own noise rows), exactly what B separate calls of the reference's per-note closure compute."""
-        # the reference builds a fresh sampler per note (:248-249); here it is cached per (step count, batch) so that the captured
-        # graph of a (width, steps, batch) triple is reused by every later group of that shape instead of being re-captured
-        key = ("note", sample_steps, B)
-        s = self._samplers.get(key)
-        if s is None:
-            s = DiffSynthSampler(self.timesteps, height=self.height, channels=self.channels, noise_strategy="repeat", mute=True,
-                                 device=str(self.device), max_batchsize=B)                                     # :248
-            s.respace(list(np.linspace(0, self.timesteps - 1, sample_steps, dtype=np.int32)))                  # :249
-            self._samplers[key] = s
-        s.activate_classifier_free_guidance(1.0, None)
-        s.noise_feed = None
-        s.graph_tail, s.final_only = self._tail_factory, True
-        mask = torch.zeros((B, 1, self.height, width), dtype=torch.float32, device=self.device)                # :252-254
-        mask[:, :, :, :int(time_resolution * (attack / 4) / vae_scale)] = 1.0
-        mask[:, :, :, -int(time_resolution * ((before_release + 1) / 4) / vae_scale):] = 1.0
-        init = None
-        if noise_feed is not None:
-            init = noise_feed[0][:B].to(self.device, torch.float32)
-            s.noise_feed = noise_feed[1:]
-        guide = instrument_latent.to(self.device, torch.float32)
-        if guide.shape[0] == 1 and B > 1:
-            guide = guide.repeat(B, 1, 1, 1)
-        cond = condition.to(self.device)
-        if cond.shape[0] == 1 and B > 1:
-            cond = cond.repeat(B, 1)
-        imgs, _ = s.inpaint_sample(self.unet, (B, self.channels, self.height, width), noising_strength, guide, mask, return_tensor=True,
-                                   condition=cond, sampler=sampler, initial_noise=init,
-                                   use_dynamic_mask=True, end_noise_level_ratio=0.0, mask_flexivity=1.0)       # :257-269
-        return self._decode(s, imgs[-1])       # quantiser :275, decoder + iSTFT :277-283, inside the group's graph
 
     @torch.no_grad()
     def synthesize_note(self, instrument_latent: torch.Tensor, condition: torch.Tensor, duration_sec: float, sample_steps: int = 20,
@@ -411,9 +348,8 @@ class TextToTimbre:
         ``condition`` [1,512] the empty-prompt embedding the reference passes (:231-233; no classifier-free guidance here);
         attack and tail are frozen by a mask that shrinks over the steps (``use_dynamic_mask``, mask_flexivity 1.0).
         The width ``int(256 * ((duration + 1) / 4) / 4)`` is arbitrary, odd levels included (pad_to_match)."""
-        width = self.note_width(duration_sec, time_resolution, vae_scale)
-        return self._synthesize_group(instrument_latent, condition, width, 1, sample_steps, noising_strength, attack, before_release,
-                                      sampler, time_resolution, vae_scale, noise_feed)
+        return self.synthesize_notes(instrument_latent, condition, [duration_sec], sample_steps, noising_strength, attack, before_release,
+                                     sampler, time_resolution, vae_scale, None if noise_feed is None else [noise_feed])[0]
 
     @torch.no_grad()
     def synthesize_notes(self, instrument_latent: torch.Tensor, condition: torch.Tensor, durations_sec, sample_steps: int = 20,
@@ -428,19 +364,31 @@ class TextToTimbre:
 
     def _synthesize_rows(self, latents, conditions, widths, sample_steps, noising_strength, attack, before_release, sampler, time_resolution,
                          vae_scale, noise_feeds) -> list:
-        """Rows of equal width -- whatever their instrument latent [1,4,128,64] and condition [1,512] -- as ONE batched graph launch
-        per distinct width (each row of the batch carries its own guide and condition).  Returns one ``Timbres`` per row, in order;
+        """Rows of equal width -- whatever their instrument latent [1,4,128,64] and condition [1,512] -- as ONE batched inpainting
+        run (one graph launch) per distinct width: every row is an independent sample of the batch (own guide, condition and noise
+        rows), exactly what separate calls of the reference's per-note closure compute.  Returns one ``Timbres`` per row, in order;
         ``noise_feeds``: None or one per row."""
         out = [None] * len(widths)
         for w in sorted(set(widths)):
             idx = [i for i, ww in enumerate(widths) if ww == w]
-            feed = torch.cat([noise_feeds[i] for i in idx], dim=1) if noise_feeds is not None else None
-            guide = torch.cat([latents[i].to(self.device, torch.float32) for i in idx])
-            cond = torch.cat([conditions[i].to(self.device) for i in idx])
-            t = self._synthesize_group(guide, cond, w, len(idx), sample_steps, noising_strength, attack, before_release, sampler,
-                                       time_resolution, vae_scale, feed)
+            B = len(idx)
+            guide = torch.cat([self._rows(latents[i], 1, "instrument_latent", (self.channels, self.height, 64)) for i in idx]).float()
+            cond = torch.cat([self._rows(conditions[i], 1, "condition", ("L",)) for i in idx])
+            feed = None if noise_feeds is None else noise_feeds[idx[0]] if B == 1 else torch.cat([noise_feeds[i] for i in idx], dim=1)
+            # the reference builds a fresh sampler per note (:248-249); here it is cached per (step count, batch) so that the captured
+            # graph of a (width, steps, batch) triple is reused by every later group of that shape instead of being re-captured
+            s = self._respaced_sampler(("note", sample_steps, B), B, sample_steps, 1.0, None, noise_strategy="repeat")
+            mask = torch.zeros((B, 1, self.height, w), dtype=torch.float32, device=self.device)                # :252-254
+            mask[:, :, :, :int(time_resolution * (attack / 4) / vae_scale)] = 1.0
+            mask[:, :, :, -int(time_resolution * ((before_release + 1) / 4) / vae_scale):] = 1.0
+            # :257-269, then the quantiser (:275), decoder and iSTFT (:277-283) inside the group's graph
+            t = self._run(s, lambda init: s.inpaint_sample(self.unet, (B, self.channels, self.height, w), noising_strength, guide, mask,
+                                                           return_tensor=True, condition=cond, sampler=sampler, initial_noise=init,
+                                                           use_dynamic_mask=True, end_noise_level_ratio=0.0, mask_flexivity=1.0),
+                          B, feed, True)
             for b, i in enumerate(idx):
-                out[i] = Timbres(t.latents[b:b + 1], t.quantized[b:b + 1], t.spectrograms[b:b + 1], t.waveforms[b:b + 1])
+                out[i] = Timbres(t.latents[b:b + 1], t.quantized[b:b + 1], t.spectrograms[b:b + 1], t.waveforms[b:b + 1],
+                                 t.initial_noise[b:b + 1])
         return out
 
     @staticmethod
@@ -475,14 +423,8 @@ class TextToTimbre:
         (duration, semitones) pair is pitch-shifted once (librosa.effects.pitch_shift, track_maker.py:42) in one batched call, and
         every note is placed at round(onset * 16000) with its gain and summed in one call (codec.shift_and_mix).  Returns the
         fp32 track [max(onset + note length)]; no normalisation, no envelope."""
-        plan = self.track_plan(notes, time_resolution, vae_scale)
-        timbres = self.synthesize_notes(instrument_latent, condition, plan.durations, sample_steps=sample_steps,
-                                        noising_strength=noising_strength, attack=attack, before_release=before_release, sampler=sampler,
-                                        time_resolution=time_resolution, vae_scale=vae_scale, noise_feeds=noise_feeds)
-        sources = [timbres[d].waveforms[0] for d, _ in plan.pairs]
-        track = shift_and_mix(sources, [s for _, s in plan.pairs], plan.note_pair, plan.onsets, plan.gains)
-        assert track.numel() == plan.track_len
-        return track
+        return self._render([(instrument_latent, condition, notes, 1.0, 0.0)], sample_steps, noising_strength, attack, before_release,
+                            sampler, time_resolution, vae_scale, noise_feeds, fades=False, target_peak=None)
 
     @staticmethod
     def arrangement_plan(tracks, time_resolution: int = 256, vae_scale: int = 4, sample_rate: int = 16000) -> ArrangementPlan:
@@ -525,6 +467,13 @@ class TextToTimbre:
         ``noise_feeds`` (tests): one per row (arrangement_plan), in row order.  Returns the fp32 piece [max(onset + note length)]."""
         if target_peak is not None and not (np.isfinite(float(target_peak)) and float(target_peak) > 0.0):
             raise ValueError(f"target_peak must be None or a finite value > 0, got {target_peak}")
+        return self._render(tracks, sample_steps, noising_strength, attack, before_release, sampler, time_resolution, vae_scale,
+                            noise_feeds, fades=True, target_peak=target_peak)
+
+    def _render(self, tracks, sample_steps, noising_strength, attack, before_release, sampler, time_resolution, vae_scale, noise_feeds,
+                fades: bool, target_peak: Optional[float]) -> torch.Tensor:
+        """render_arrangement's body: the plan, one synthesis launch per distinct width, one pitch shift and one mix.  ``fades``
+        False (render_track) mixes through ds_mix_track, without the tracks' fades."""
         plan = self.arrangement_plan(tracks, time_resolution, vae_scale)
         latents, conditions = [], []
         for k, (lat, cond, _, _, _) in enumerate(tracks):
@@ -540,8 +489,8 @@ class TextToTimbre:
                                         sample_steps, noising_strength, attack, before_release, sampler, time_resolution, vae_scale,
                                         noise_feeds)
         sources = [timbres[r].waveforms[0] for r, _ in plan.items]
-        track = shift_and_mix(sources, [s for _, s in plan.items], plan.note_item, plan.onsets, plan.gains, fades=plan.fades,
-                              target_peak=target_peak)
+        track = shift_and_mix(sources, [s for _, s in plan.items], plan.note_item, plan.onsets, plan.gains,
+                              fades=plan.fades if fades else None, target_peak=target_peak)
         assert track.numel() == plan.track_len
         return track
 

@@ -71,7 +71,7 @@ class DiffSynthSampler:
         self.noise_feed: Optional[torch.Tensor] = None     # [K, >=B, C, H, train_width]; consumed in draw order
         self._feed_pos = 0
         # The reference draws the per-step noise even when eta == 0 (:340), which advances the global RNG; True reproduces that RNG
-        # state after sample() at the cost of n_iter discarded randn launches (TextToTimbre turns it off for throughput runs).
+        # state after sample() at the cost of n_iter discarded randn launches (TextToTimbre leaves it on).
         self.faithful_rng = True
         self._graphs: Dict[tuple, "_GraphLoop"] = {}
         self.last_graph_launches = 0

@@ -75,6 +75,16 @@ def test_invalid_arguments_fail_without_a_gpu():
     assert lib.ds_conv_gemm(C.byref(a), None) == -1 and b"BK" in lib.ds_last_error()
 
 
+def test_modify_rejects_a_guide_of_other_rows_before_the_device():
+    from diffusynth_b200 import TextToTimbre
+    pipe = TextToTimbre.__new__(TextToTimbre)
+    pipe.channels, pipe.height = 4, 128
+    cond = torch.zeros(2, 512)
+    for guide in (torch.zeros(3, 4, 128, 64), torch.zeros(2, 3, 128, 64), torch.zeros(4, 128, 64)):
+        with pytest.raises(ValueError):
+            pipe.modify(guide, cond, None)
+
+
 def test_noise_layout_column_map_matches_oracle():
     from diffusynth_b200.sampler import _column_map
     base = torch.arange(64).float().view(1, 1, 1, 64)

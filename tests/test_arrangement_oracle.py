@@ -133,3 +133,17 @@ def test_render_arrangement_rejects_bad_input_before_synthesis():
     for peak in (0.0, -1.0, float("nan")):
         with pytest.raises(ValueError):
             pipe.render_arrangement([(lat, cond, notes, 1.0, 0.0)], target_peak=peak)
+
+
+def test_render_track_rejects_bad_input_before_synthesis():
+    from diffusynth_b200 import TextToTimbre
+    pipe = TextToTimbre.__new__(TextToTimbre)
+    pipe.channels, pipe.height = 4, 128
+
+    def no_synthesis(*a):
+        raise AssertionError("synthesis reached")
+    pipe._synthesize_rows = no_synthesis
+    lat, cond, notes = torch.zeros(1, 4, 128, 64), torch.zeros(1, 512), [(0.0, 1.0, 0, 1.0)]
+    for args in ((lat[:, :3], cond, notes), (lat, torch.zeros(512), notes), (lat, cond, [])):
+        with pytest.raises(ValueError):
+            pipe.render_track(*args)

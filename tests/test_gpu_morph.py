@@ -98,6 +98,28 @@ def test_generated_initial_noise_recreates_the_timbre(pipe, width):
     assert torch.equal(c.initial_noise.cpu(), draws[0])
 
 
+@pytest.mark.parametrize("entry", ["modify", "inpaint", "synthesize_note"])
+def test_one_draw_feed_runs_like_the_full_feed(pipe, entry):
+    """A feed of draw 0 alone, as generate takes it: the step draws come from the RNG, and DDIM multiplies them by sigma = 0, so
+    the result is the full feed's; initial_noise is draw 0 either way."""
+    steps, B = 2, (1 if entry == "synthesize_note" else 2)
+    guide = cases.vq_latents(B=1, seed=66).cuda()
+    cond, uncond = W.synthetic_conditions(B, L)
+    draws = W.host_noise(6, 1 + 2 * steps, B)                         # enough step draws for modify's int(steps / 0.5)
+    mask = np.ones((513, 257), np.float32)
+    mask[100:300, 60:180] = 0.0
+
+    def run(feed):
+        if entry == "modify":
+            return pipe.modify(guide, cond.cuda(), uncond.cuda(), steps=steps, strength=0.5, noise_feed=feed)
+        if entry == "inpaint":
+            return pipe.inpaint(guide, mask, cond.cuda(), uncond.cuda(), steps=steps, noise_feed=feed)
+        return pipe.synthesize_note(guide, cond.cuda(), 0.9, sample_steps=steps, noise_feed=feed)
+    full, one = run(draws), run([draws[0]])
+    assert torch.equal(one.latents, full.latents) and torch.equal(one.waveforms, full.waveforms)
+    assert torch.equal(one.initial_noise.cpu(), draws[0]) and torch.equal(full.initial_noise.cpu(), draws[0])
+
+
 def _small_unet(use_engine):
     from diffusynth_b200 import ConditionedUnet
     cfg, sd, _, _, cond = cases.unet_case("small_w16")

@@ -65,12 +65,12 @@ def main() -> int:
 
     pipe = TextToTimbre.random_init(device="cuda", seed=0)
     groups = [0]
-    inner = pipe._synthesize_group
+    inner = pipe._run
 
-    def counted(*args, **kw):                                                   # one _synthesize_group = one graph launch
+    def counted(*args, **kw):                                                   # one _run = one graph launch
         groups[0] += 1
         return inner(*args, **kw)
-    pipe._synthesize_group = counted
+    pipe._run = counted
 
     def arrangement():
         return pipe.render_arrangement(tracks, sample_steps=a.steps, target_peak=0.9)
