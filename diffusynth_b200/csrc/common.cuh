@@ -7,6 +7,7 @@
 #include <cstdio>
 #include <cstring>
 #include <cstdlib>
+#include <vector>
 
 namespace ds {
 
@@ -46,6 +47,55 @@ inline int num_sms() {
   }
   return n;
 }
+
+// Blocks of `block` threads for n work items: ceil(n / block), at most per_sm per SM (grid-stride kernels) and at least 1.
+inline unsigned grid_for(long long n, int block, int per_sm) {
+  long long b = (n + block - 1) / block;
+  const long long cap = (long long)num_sms() * per_sm;
+  if (b > cap) b = cap;
+  return (unsigned)(b > 0 ? b : 1);
+}
+
+inline size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
+
+// ---- workspace of a ragged-batch entry point ------------------------------------------------------------------------------
+// stage() places a host array after the previous one, at its type's alignment, in one block at the start of the workspace, and
+// returns its byte offset; reserve(), called after the last stage(), places device-only scratch after that block.  The block and
+// every scratch buffer start 256-byte aligned; `bytes` is the workspace size.  The arrays are read only by upload(), so they must
+// stay alive and unchanged until then (a workspace query plans the same way and never uploads).  upload() gathers them into a
+// pageable host block and copies it with one cudaMemcpyAsync.  From a pageable source the copy is staged before the call returns,
+// so the block may be freed at once; for the same reason these uploads are never made under stream capture, where the copy would
+// read the freed block at every replay.
+struct Workspace {
+  struct Array { size_t off; const void* src; size_t n; };
+  std::vector<Array> arrays;
+  size_t staged = 0, bytes = 0;
+
+  template <typename T>
+  size_t stage(const T* src, size_t count) {
+    const size_t o = (staged + alignof(T) - 1) / alignof(T) * alignof(T);
+    arrays.push_back({o, src, count * sizeof(T)});
+    staged = o + count * sizeof(T);
+    bytes = align256(staged);
+    return o;
+  }
+  size_t reserve(size_t n) {
+    const size_t o = bytes;
+    bytes = align256(o + n);
+    return o;
+  }
+  cudaError_t upload(void* ws, cudaStream_t stream) const {
+    std::vector<uint8_t> host(staged, 0);
+    for (const Array& a : arrays)
+      if (a.n) memcpy(host.data() + a.off, a.src, a.n);
+    return cudaMemcpyAsync(ws, host.data(), staged, cudaMemcpyHostToDevice, stream);
+  }
+};
+
+// resampy's kaiser_best filter (pitch.cu, resample.cu): 64 zero crossings per side, roll-off and Kaiser beta
+constexpr double kPi = 3.14159265358979323846;
+constexpr int RS_ZEROS = 64;
+constexpr double RS_ROLLOFF = 0.9475937167399596, RS_BETA = 14.769656459379492;
 
 // ---- programmatic dependent launch ------------------------------------------------------------------------------
 // Every hot-path kernel is launched with cudaLaunchAttributeProgrammaticStreamSerialization: its blocks may be scheduled while
@@ -128,6 +178,16 @@ __device__ __forceinline__ float warp_max(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
   return v;
+}
+
+// item of a global index in a ragged batch: the k with off[k] <= g < off[k+1] (off is a prefix array of B+1 entries, off[0] = 0)
+__device__ __forceinline__ int find_item(const long long* __restrict__ off, int B, long long g) {
+  int lo = 0, hi = B - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (__ldg(off + mid) <= g) lo = mid; else hi = mid - 1;
+  }
+  return lo;
 }
 
 // Reduce (sum, sumsq) partials to (mean, rstd).  Called by a full warp; every lane returns the result.

@@ -492,9 +492,7 @@ int ds_dwconv7_stats_slots(int C, int H, int W) {
 int ds_stem_im2col(const float* d_x, void* d_col, int N, int Cin, int H, int W, void* stream) {
   DS_REQUIRE(d_x && d_col && N > 0 && Cin > 0 && Cin <= 4 && H > 0 && W > 0, "ds_stem_im2col: bad arguments");
   const long long total = (long long)N * H * W * 7;
-  long long g = (total + 255) / 256;
-  const long long cap = (long long)num_sms() * 16;
-  DS_CHECK_CUDA(launch_pdl(stem_im2col_kernel, dim3((int)(g < cap ? g : cap)), dim3(256), (size_t)(0), (cudaStream_t)stream, d_x, (act_t*)d_col, Cin, H, W, total));
+  DS_CHECK_CUDA(launch_pdl(stem_im2col_kernel, dim3(grid_for(total, 256, 16)), dim3(256), (size_t)(0), (cudaStream_t)stream, d_x, (act_t*)d_col, Cin, H, W, total));
   DS_CHECK_CUDA(cudaGetLastError());
   return DS_OK;
 }

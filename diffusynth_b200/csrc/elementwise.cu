@@ -356,12 +356,6 @@ __global__ void sinusoidal_kernel(const long long* __restrict__ t, float* __rest
   }
 }
 
-static inline int grid_for(long long n, int block, int per_sm = 8) {
-  long long g = (n + block - 1) / block;
-  long long cap = (long long)num_sms() * per_sm;
-  return (int)(g < 1 ? 1 : (g > cap ? cap : g));
-}
-
 }  // namespace ds
 
 using namespace ds;
@@ -373,7 +367,7 @@ extern "C" {
 int ds_ddim_step(const float* d_eps_u, const float* d_eps_c, const float* d_x, const float* d_z, const float* d_coef,
                  float* d_out, long long n, void* stream) {
   DS_REQUIRE(d_eps_c && d_x && d_coef && d_out && n > 0 && n % 4 == 0, "ds_ddim_step: bad arguments (n=%lld must be a positive multiple of 4)", n);
-  DS_CHECK_CUDA(launch_pdl(ddim_step_kernel, dim3(grid_for(n / 4, 256)), dim3(256), (size_t)(0), (cudaStream_t)stream, 
+  DS_CHECK_CUDA(launch_pdl(ddim_step_kernel, dim3(grid_for(n / 4, 256, 8)), dim3(256), (size_t)(0), (cudaStream_t)stream, 
       (const float4*)d_eps_u, (const float4*)d_eps_c, (const float4*)d_x, (const float4*)d_z, d_coef, (float4*)d_out, n / 4));
   DS_CHECK_CUDA(cudaGetLastError());
   return DS_OK;
@@ -383,7 +377,7 @@ int ds_q_sample(const float* d_x0, const float* d_noise, const float* d_coef, fl
                 void* stream) {
   DS_REQUIRE(d_x0 && d_noise && d_coef && d_out && n > 0 && n % 4 == 0, "ds_q_sample: bad arguments");
   DS_REQUIRE(per_sample >= 0 && per_sample % 4 == 0 && (per_sample == 0 || n % per_sample == 0), "ds_q_sample: per_sample=%lld must divide n=%lld and be a multiple of 4", per_sample, n);
-  DS_CHECK_CUDA(launch_pdl(q_sample_kernel, dim3(grid_for(n / 4, 256)), dim3(256), (size_t)(0), (cudaStream_t)stream, (const float4*)d_x0, (const float4*)d_noise, d_coef,
+  DS_CHECK_CUDA(launch_pdl(q_sample_kernel, dim3(grid_for(n / 4, 256, 8)), dim3(256), (size_t)(0), (cudaStream_t)stream, (const float4*)d_x0, (const float4*)d_noise, d_coef,
                                                                           (float4*)d_out, n / 4, per_sample / 4));
   DS_CHECK_CUDA(cudaGetLastError());
   return DS_OK;
@@ -394,7 +388,7 @@ int ds_mask_blend(const float* d_guide, const float* d_noise, const float* d_mas
   DS_REQUIRE(d_guide && d_noise && d_mask && d_coef && d_img && B > 0 && C > 0 && hw > 0, "ds_mask_blend: bad arguments");
   DS_REQUIRE(mask_channels == 1 || mask_channels == C, "ds_mask_blend: mask_channels=%d must be 1 or C=%d", mask_channels, C);
   const long long total = (long long)B * C * hw;
-  DS_CHECK_CUDA(launch_pdl(mask_blend_kernel, dim3(grid_for(total, 256)), dim3(256), (size_t)(0), (cudaStream_t)stream, d_guide, d_noise, d_mask, d_coef, d_img, C, mask_channels, hw, total));
+  DS_CHECK_CUDA(launch_pdl(mask_blend_kernel, dim3(grid_for(total, 256, 8)), dim3(256), (size_t)(0), (cudaStream_t)stream, d_guide, d_noise, d_mask, d_coef, d_img, C, mask_channels, hw, total));
   DS_CHECK_CUDA(cudaGetLastError());
   return DS_OK;
 }
@@ -402,7 +396,7 @@ int ds_mask_blend(const float* d_guide, const float* d_noise, const float* d_mas
 int ds_add_channel_bias(void* d_x, const float* d_bias, long long bias_stride, int N, int C, long long hw, void* stream) {
   DS_REQUIRE(d_x && d_bias && N > 0 && C > 0 && C % 2 == 0 && hw > 0 && bias_stride >= 0, "ds_add_channel_bias: bad arguments");
   const long long per = hw * C / 2, total = per * N;
-  DS_CHECK_CUDA(launch_pdl(add_channel_bias_kernel, dim3(grid_for(total, 256)), dim3(256), (size_t)(0), (cudaStream_t)stream, (act_t*)d_x, d_bias, bias_stride, C, per, total));
+  DS_CHECK_CUDA(launch_pdl(add_channel_bias_kernel, dim3(grid_for(total, 256, 8)), dim3(256), (size_t)(0), (cudaStream_t)stream, (act_t*)d_x, d_bias, bias_stride, C, per, total));
   DS_CHECK_CUDA(cudaGetLastError());
   return DS_OK;
 }
@@ -410,9 +404,9 @@ int ds_add_channel_bias(void* d_x, const float* d_bias, long long bias_stride, i
 int ds_nchw_f32_to_nhwc_bf16(const float* d_in, void* d_out, int N, int C, int Cp, long long hw, void* stream) {
   DS_REQUIRE(d_in && d_out && N > 0 && C > 0 && Cp >= C && hw > 0, "ds_nchw_f32_to_nhwc_bf16: bad arguments");
   if (Cp % 8 == 0 && reinterpret_cast<uintptr_t>(d_out) % 16 == 0)
-    DS_CHECK_CUDA(launch_pdl(nchw_f32_to_nhwc_vec_kernel, dim3(grid_for((long long)N * hw, 256)), dim3(256), (size_t)(0), (cudaStream_t)stream, d_in, (uint4*)d_out, C, Cp / 8, hw, (long long)N * hw));
+    DS_CHECK_CUDA(launch_pdl(nchw_f32_to_nhwc_vec_kernel, dim3(grid_for((long long)N * hw, 256, 8)), dim3(256), (size_t)(0), (cudaStream_t)stream, d_in, (uint4*)d_out, C, Cp / 8, hw, (long long)N * hw));
   else
-    DS_CHECK_CUDA(launch_pdl(nchw_f32_to_nhwc_bf16_kernel, dim3(grid_for((long long)N * hw * Cp, 256)), dim3(256), (size_t)(0), (cudaStream_t)stream, 
+    DS_CHECK_CUDA(launch_pdl(nchw_f32_to_nhwc_bf16_kernel, dim3(grid_for((long long)N * hw * Cp, 256, 8)), dim3(256), (size_t)(0), (cudaStream_t)stream, 
         d_in, (act_t*)d_out, C, Cp, hw, (long long)N * hw));
   DS_CHECK_CUDA(cudaGetLastError());
   return DS_OK;
@@ -421,7 +415,7 @@ int ds_nchw_f32_to_nhwc_bf16(const float* d_in, void* d_out, int N, int C, int C
 int ds_nhwc_bf16_to_nchw_f32(const void* d_in, float* d_out, int N, int C, int Cp, long long hw, void* stream) {
   DS_REQUIRE(d_in && d_out && N > 0 && C > 0 && Cp >= C && hw > 0, "ds_nhwc_bf16_to_nchw_f32: bad arguments");
   const long long total = (long long)N * C * hw;
-  DS_CHECK_CUDA(launch_pdl(nhwc_bf16_to_nchw_f32_kernel, dim3(grid_for(total, 256)), dim3(256), (size_t)(0), (cudaStream_t)stream, (const act_t*)d_in, d_out, C, Cp, hw, total));
+  DS_CHECK_CUDA(launch_pdl(nhwc_bf16_to_nchw_f32_kernel, dim3(grid_for(total, 256, 8)), dim3(256), (size_t)(0), (cudaStream_t)stream, (const act_t*)d_in, d_out, C, Cp, hw, total));
   DS_CHECK_CUDA(cudaGetLastError());
   return DS_OK;
 }
@@ -480,7 +474,7 @@ int ds_gn_act(const void* d_x, void* d_out, const void* d_part, int chunks, cons
 
 int ds_add_bf16(const void* d_a, const void* d_b, void* d_out, long long n, void* stream) {
   DS_REQUIRE(d_a && d_b && d_out && n > 0 && n % 8 == 0, "ds_add_bf16: bad arguments");
-  DS_CHECK_CUDA(launch_pdl(add_bf16_kernel, dim3(grid_for(n / 8, 256)), dim3(256), (size_t)(0), (cudaStream_t)stream, (const uint4*)d_a, (const uint4*)d_b, (uint4*)d_out, n / 8));
+  DS_CHECK_CUDA(launch_pdl(add_bf16_kernel, dim3(grid_for(n / 8, 256, 8)), dim3(256), (size_t)(0), (cudaStream_t)stream, (const uint4*)d_a, (const uint4*)d_b, (uint4*)d_out, n / 8));
   DS_CHECK_CUDA(cudaGetLastError());
   return DS_OK;
 }
@@ -488,7 +482,7 @@ int ds_add_bf16(const void* d_a, const void* d_b, void* d_out, long long n, void
 int ds_decoder_head(const float* d_a, const float* d_b, float* d_out, int N, long long hw, void* stream) {
   DS_REQUIRE(d_a && d_out && N > 0 && hw > 0, "ds_decoder_head: bad arguments");
   const long long total = (long long)N * 3 * hw;
-  DS_CHECK_CUDA(launch_pdl(decoder_head_kernel, dim3(grid_for(total, 256)), dim3(256), (size_t)(0), (cudaStream_t)stream, d_a, d_b, d_out, hw, total));
+  DS_CHECK_CUDA(launch_pdl(decoder_head_kernel, dim3(grid_for(total, 256, 8)), dim3(256), (size_t)(0), (cudaStream_t)stream, d_a, d_b, d_out, hw, total));
   DS_CHECK_CUDA(cudaGetLastError());
   return DS_OK;
 }
@@ -506,13 +500,13 @@ int ds_linear(const float* d_in, long long in_stride, const float* d_w, const fl
 
 int ds_embedding_gather(const float* d_table, const long long* d_ids, float* d_out, int N, int D, int rows, void* stream) {
   DS_REQUIRE(d_table && d_ids && d_out && N > 0 && D > 0 && rows > 0, "ds_embedding_gather: bad arguments");
-  DS_CHECK_CUDA(launch_pdl(embedding_gather_kernel, dim3(grid_for((long long)N * D, 256)), dim3(256), (size_t)0, (cudaStream_t)stream, d_table, d_ids, d_out, N, D, rows));
+  DS_CHECK_CUDA(launch_pdl(embedding_gather_kernel, dim3(grid_for((long long)N * D, 256, 8)), dim3(256), (size_t)0, (cudaStream_t)stream, d_table, d_ids, d_out, N, D, rows));
   return DS_OK;
 }
 
 int ds_sinusoidal_embedding(const long long* d_t, float* d_out, int N, int dim, void* stream) {
   DS_REQUIRE(d_t && d_out && N > 0 && dim >= 4 && dim % 2 == 0, "ds_sinusoidal_embedding: bad arguments");
-  DS_CHECK_CUDA(launch_pdl(sinusoidal_kernel, dim3(grid_for((long long)N * dim / 2, 128)), dim3(128), (size_t)(0), (cudaStream_t)stream, d_t, d_out, N, dim));
+  DS_CHECK_CUDA(launch_pdl(sinusoidal_kernel, dim3(grid_for((long long)N * dim / 2, 128, 8)), dim3(128), (size_t)(0), (cudaStream_t)stream, d_t, d_out, N, dim));
   DS_CHECK_CUDA(cudaGetLastError());
   return DS_OK;
 }

@@ -169,10 +169,7 @@ int ds_latent_image(const float* d_lat, void* d_img, void* d_minmax, int B, int 
   latent_minmax_kernel<<<B * 4, 256, 0, st>>>(d_lat, reinterpret_cast<float2*>(d_minmax), (long long)H * W);
   DS_CHECK_CUDA(cudaGetLastError());
   const long long total = (long long)B * 8 * H * W;
-  long long blocks = (total + 255) / 256;
-  const long long cap = (long long)num_sms() * 32;
-  if (blocks > cap) blocks = cap;
-  latent_image_kernel<<<(unsigned)blocks, 256, 0, st>>>(d_lat, reinterpret_cast<const float2*>(d_minmax), reinterpret_cast<unsigned char*>(d_img), B, H, W);
+  latent_image_kernel<<<grid_for(total, 256, 32), 256, 0, st>>>(d_lat, reinterpret_cast<const float2*>(d_minmax), reinterpret_cast<unsigned char*>(d_img), B, H, W);
   DS_CHECK_CUDA(cudaGetLastError());
   return DS_OK;
 }

@@ -273,21 +273,17 @@ int ds_stft_encode(const float* d_wave, long long L, float* d_spec, int B, int T
    tools.encode_stft (:320-331): the inverse mapping.  is_double selects float64 (numpy computes in the precision of its input). */
 int ds_decode_stft(const void* d_enc, void* d_out, long long plane, int is_double, void* stream) {
   DS_REQUIRE(d_enc && d_out && plane > 0, "ds_decode_stft: bad arguments");
-  long long blocks = (plane + 255) / 256;
-  const long long cap = (long long)num_sms() * 16;
-  if (blocks > cap) blocks = cap;
-  if (is_double) decode_stft_kernel<double><<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>((const double*)d_enc, (double*)d_out, plane);
-  else decode_stft_kernel<float><<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>((const float*)d_enc, (float*)d_out, plane);
+  const unsigned blocks = grid_for(plane, 256, 16);
+  if (is_double) decode_stft_kernel<double><<<blocks, 256, 0, (cudaStream_t)stream>>>((const double*)d_enc, (double*)d_out, plane);
+  else decode_stft_kernel<float><<<blocks, 256, 0, (cudaStream_t)stream>>>((const float*)d_enc, (float*)d_out, plane);
   DS_CHECK_CUDA(cudaGetLastError());
   return DS_OK;
 }
 int ds_encode_stft(const void* d_D, void* d_out, long long plane, int is_double, void* stream) {
   DS_REQUIRE(d_D && d_out && plane > 0, "ds_encode_stft: bad arguments");
-  long long blocks = (plane + 255) / 256;
-  const long long cap = (long long)num_sms() * 16;
-  if (blocks > cap) blocks = cap;
-  if (is_double) encode_stft_kernel<double><<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>((const double*)d_D, (double*)d_out, plane);
-  else encode_stft_kernel<float><<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>((const float*)d_D, (float*)d_out, plane);
+  const unsigned blocks = grid_for(plane, 256, 16);
+  if (is_double) encode_stft_kernel<double><<<blocks, 256, 0, (cudaStream_t)stream>>>((const double*)d_D, (double*)d_out, plane);
+  else encode_stft_kernel<float><<<blocks, 256, 0, (cudaStream_t)stream>>>((const float*)d_D, (float*)d_out, plane);
   DS_CHECK_CUDA(cudaGetLastError());
   return DS_OK;
 }
@@ -297,10 +293,8 @@ int ds_encode_stft(const void* d_D, void* d_out, long long plane, int is_double,
 int ds_griffinlim_update(const float* d_rebuilt, float* d_tprev, float* d_spec, float momentum, int first, int B, int T, void* stream) {
   DS_REQUIRE(d_rebuilt && d_tprev && d_spec && B > 0 && T > 0 && momentum >= 0.f, "ds_griffinlim_update: bad arguments");
   const long long plane = (long long)NH * T, total = plane * B;
-  long long blocks = (total + 255) / 256;
-  const long long cap = (long long)num_sms() * 16;
-  if (blocks > cap) blocks = cap;
-  griffinlim_update_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(d_rebuilt, reinterpret_cast<float2*>(d_tprev), d_spec,
+  const unsigned blocks = grid_for(total, 256, 16);
+  griffinlim_update_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(d_rebuilt, reinterpret_cast<float2*>(d_tprev), d_spec,
                                                                                 momentum / (1.0f + momentum), first, plane, total);
   DS_CHECK_CUDA(cudaGetLastError());
   return DS_OK;

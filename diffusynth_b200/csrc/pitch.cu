@@ -22,20 +22,6 @@ constexpr int R = NC / 32;                      // points per lane
 constexpr int XS_PITCH = NC + NC / R;           // staging row (fft_warp.cuh)
 constexpr int FR = 8;                           // frames (warps) per block
 constexpr int MIX_TILE = 1024;                  // track samples per mix block
-constexpr double kPi = 3.14159265358979323846;
-// resampy's kaiser_best filter: 64 zero crossings per side, roll-off and Kaiser beta
-constexpr int RS_ZEROS = 64;
-constexpr double RS_ROLLOFF = 0.9475937167399596, RS_BETA = 14.769656459379492;
-
-// item of a global index: the k with off[k] <= g < off[k+1] (off is a prefix array of B+1 entries, off[0] = 0)
-__device__ __forceinline__ int find_item(const long long* __restrict__ off, int B, long long g) {
-  int lo = 0, hi = B - 1;
-  while (lo < hi) {
-    const int mid = (lo + hi + 1) >> 1;
-    if (__ldg(off + mid) <= g) lo = mid; else hi = mid - 1;
-  }
-  return lo;
-}
 
 __device__ __forceinline__ float hann2048(int m) { return 0.5f - 0.5f * cospif((float)m / 1024.0f); }
 
@@ -217,32 +203,13 @@ pitch_resample_kernel(const float* __restrict__ ys, float* __restrict__ out, con
   }
 }
 
-// ---- track mix: track[j] = sum over notes n covering j, in input order, of gain_n * src[src_off_n + j - onset_n] ---------------
-// a gather over track samples (one block per MIX_TILE samples) through the per-tile note lists, so the sum order is fixed.
-__global__ void __launch_bounds__(256)
-pitch_mix_kernel(const float* __restrict__ src, float* __restrict__ track, long long track_len, const int* __restrict__ tile_ptr,
-                 const int* __restrict__ tile_notes, const long long* __restrict__ src_off, const long long* __restrict__ len,
-                 const long long* __restrict__ onset, const float* __restrict__ gain) {
-  pdl_enter();
-  const int p0 = __ldg(tile_ptr + blockIdx.x), p1 = __ldg(tile_ptr + blockIdx.x + 1);
-  for (int q = threadIdx.x; q < MIX_TILE; q += blockDim.x) {
-    const long long j = (long long)blockIdx.x * MIX_TILE + q;
-    if (j >= track_len) break;
-    float acc = 0.f;
-    for (int p = p0; p < p1; ++p) {
-      const int n = __ldg(tile_notes + p);
-      const long long r = j - __ldg(onset + n);
-      if (r >= 0 && r < __ldg(len + n)) acc = fmaf(__ldg(gain + n), __ldg(src + __ldg(src_off + n) + r), acc);
-    }
-    track[j] = acc;
-  }
-}
-
-// ---- arrangement mix: pitch_mix_kernel's gather with a linear fade over the last fade_n samples of every note (fade_n =
-// min(fade_out[n], len[n]), clamped on the host) and, when `peak` is non-null, one max |track| partial per tile.  A sample before
-// the ramp takes pitch_mix_kernel's exact fmaf(gain, src, acc), so a fade-free note has no envelope multiply at all.  Every thread
-// owns ARR_SPT samples 256 apart and walks the tile's notes once for all of them (a note's metadata is loaded once per thread, not
-// once per sample); each sample still sums its notes in input order, as pitch_mix_kernel does.  256 threads per block.
+// ---- track mix (ds_mix_arrangement, and ds_mix_track without fades or peak): track[j] = sum over notes n covering j, in input
+// order, of gain_n * env_n * src[src_off_n + j - onset_n].  A gather over track samples (one block per MIX_TILE samples) through the
+// per-tile note lists, so the sum order is fixed.  env_n is a linear fade over the last fade_n = min(fade_out[n], len[n]) samples
+// (clamped on the host); a sample before the ramp takes a plain fmaf(gain, src, acc), so a fade-free note has no envelope multiply
+// at all.  When `peak` is non-null, each tile also writes its max |track| partial.  Every thread owns ARR_SPT samples 256 apart
+// and walks the tile's notes once for all of them (a note's metadata is loaded once per thread, not once per sample); each sample
+// still sums its notes in input order.  256 threads per block.
 constexpr int ARR_SPT = MIX_TILE / 256;
 __global__ void __launch_bounds__(256)
 pitch_arrange_kernel(const float* __restrict__ src, float* __restrict__ track, long long track_len, const int* __restrict__ tile_ptr,
@@ -319,33 +286,27 @@ double bessel_i0(double x) {
   return sum;
 }
 
-size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
-
-// Host-side plan of one batched pitch shift: the per-item metadata (uploaded as one block at the start of the workspace) and the
-// workspace carve-up.  Metadata: loff, fin, fout, yoff (B+1 prefix arrays each), tcap, nval (B each), as int64; rate (B) float64.
+// Host-side plan of one batched pitch shift: the per-item metadata, staged at the start of the workspace, and the stages after
+// it.  Metadata: loff, fin, fout, yoff (B+1 prefix arrays each), tcap, nval (B each) in one int64 array, then rate (B) float64.
 struct PitchPlan {
-  std::vector<long long> meta;         // int64 arrays followed by the float64 rates (bit copies)
-  int B = 0;
-  size_t off_D = 0, off_S = 0, off_frames = 0, off_ys = 0, bytes = 0;
+  std::vector<long long> idx;
+  std::vector<double> rate;
+  Workspace ws;
+  size_t off_idx = 0, off_rate = 0, off_D = 0, off_S = 0, off_frames = 0, off_ys = 0;
   long long n_in_frames = 0, n_out_frames = 0, n_ys = 0, n_samples = 0;
 };
 
-int check_pitch_args(const long long* lengths, const double* n_steps, int B, const char* who) {
+int plan_pitch(const long long* lengths, const double* n_steps, int B, const char* who, PitchPlan& p) {
   DS_REQUIRE(lengths && n_steps && B > 0, "%s: lengths and n_steps must be non-null and B > 0 (B = %d)", who, B);
   for (int k = 0; k < B; ++k) {
     DS_REQUIRE(lengths[k] > 0, "%s: item %d has length %lld (must be > 0)", who, k, lengths[k]);
     DS_REQUIRE(std::isfinite(n_steps[k]) && std::fabs(n_steps[k]) <= 24.0, "%s: item %d has n_steps %g (must be finite, |n_steps| <= 24)",
                who, k, n_steps[k]);
   }
-  return DS_OK;
-}
-
-void make_plan(const long long* lengths, const double* n_steps, int B, PitchPlan& p) {
-  p.B = B;
   const size_t n1 = (size_t)B + 1;
-  p.meta.assign(4 * n1 + 3 * (size_t)B, 0);
-  long long *loff = p.meta.data(), *fin = loff + n1, *fout = fin + n1, *yoff = fout + n1, *tcap = yoff + n1, *nval = tcap + B;
-  double* rate = reinterpret_cast<double*>(nval + B);
+  p.idx.assign(4 * n1 + 2 * (size_t)B, 0);
+  p.rate.assign(B, 0.0);
+  long long *loff = p.idx.data(), *fin = loff + n1, *fout = fin + n1, *yoff = fout + n1, *tcap = yoff + n1, *nval = tcap + B;
   for (int k = 0; k < B; ++k) {
     const long long L = lengths[k];
     const double rt = std::exp2(-n_steps[k] / 12.0);
@@ -365,32 +326,35 @@ void make_plan(const long long* lengths, const double* n_steps, int B, PitchPlan
     yoff[k + 1] = yoff[k] + len;
     tcap[k] = cap;
     nval[k] = nv;
-    rate[k] = rt;
+    p.rate[k] = rt;
   }
   p.n_samples = loff[B];
   p.n_in_frames = fin[B];
   p.n_out_frames = fout[B];
   p.n_ys = yoff[B];
-  size_t o = align256(p.meta.size() * sizeof(long long));
-  p.off_D = o;      o = align256(o + (size_t)p.n_in_frames * NBIN * sizeof(float2));
-  p.off_S = o;      o = align256(o + (size_t)p.n_out_frames * NBIN * sizeof(float2));
-  p.off_frames = o; o = align256(o + (size_t)p.n_out_frames * NFFT * sizeof(float));
-  p.off_ys = o;     o = align256(o + (size_t)p.n_ys * sizeof(float));
-  p.bytes = o;
+  p.off_idx = p.ws.stage(p.idx.data(), p.idx.size());
+  p.off_rate = p.ws.stage(p.rate.data(), p.rate.size());
+  p.off_D = p.ws.reserve((size_t)p.n_in_frames * NBIN * sizeof(float2));
+  p.off_S = p.ws.reserve((size_t)p.n_out_frames * NBIN * sizeof(float2));
+  p.off_frames = p.ws.reserve((size_t)p.n_out_frames * NFFT * sizeof(float));
+  p.off_ys = p.ws.reserve((size_t)p.n_ys * sizeof(float));
+  return DS_OK;
 }
 
-// Per-tile note lists of a mix: CSR over tiles of MIX_TILE track samples, notes in input order; followed by the per-note arrays.
+// Per-tile note lists of a mix (CSR over tiles of MIX_TILE track samples, notes in input order) and the clamped fades, staged with
+// the per-note arrays; one peak partial per tile after them when normalising.
 struct MixPlan {
   std::vector<int> tile_ptr, tile_notes;
-  size_t off_notes = 0, off_src = 0, off_len = 0, off_onset = 0, off_gain = 0, bytes = 0;
-  size_t off_fade = 0, off_peak = 0;          // arrangement mix only: the clamped fades, then the per-tile peak partials
+  std::vector<long long> fade;
+  Workspace ws;
+  size_t off_notes = 0, off_src = 0, off_len = 0, off_onset = 0, off_gain = 0, off_fade = 0, off_peak = 0;
   int n_tiles = 0;
 };
 
-// fade_out (nullable) and target_peak are the arrangement mix's: fades >= 0, a finite target_peak >= 0; src_offsets (nullable:
-// the workspace queries do not take them) >= 0.
-int check_mix_args(const long long* lengths, const long long* onsets, int K, long long track_len, const char* who,
-                   const long long* fade_out = nullptr, float target_peak = 0.f, const long long* src_offsets = nullptr) {
+// The arrangement mix's checks and plan; ds_mix_track comes here with all-zero fades and target_peak 0.  src_offsets and gains are
+// null in the workspace queries, which do not take them.
+int plan_mix(const long long* src_offsets, const long long* lengths, const long long* onsets, const float* gains,
+             const long long* fade_out, int K, float target_peak, long long track_len, const char* who, MixPlan& p) {
   DS_REQUIRE(lengths && onsets && K > 0 && track_len > 0, "%s: lengths and onsets must be non-null, K > 0 and track_len > 0", who);
   DS_REQUIRE(std::isfinite(target_peak) && target_peak >= 0.f, "%s: target_peak %g (must be finite and >= 0)", who, (double)target_peak);
   for (int n = 0; n < K; ++n) {
@@ -398,14 +362,10 @@ int check_mix_args(const long long* lengths, const long long* onsets, int K, lon
     DS_REQUIRE(onsets[n] >= 0, "%s: note %d has onset %lld (must be >= 0)", who, n, onsets[n]);
     DS_REQUIRE(onsets[n] + lengths[n] <= track_len, "%s: note %d ends at %lld, past the track length %lld", who, n,
                onsets[n] + lengths[n], track_len);
-    DS_REQUIRE(!fade_out || fade_out[n] >= 0, "%s: note %d has fade_out %lld (must be >= 0)", who, n, fade_out ? fade_out[n] : 0LL);
+    DS_REQUIRE(fade_out[n] >= 0, "%s: note %d has fade_out %lld (must be >= 0)", who, n, fade_out[n]);
     DS_REQUIRE(!src_offsets || src_offsets[n] >= 0, "%s: note %d has source offset %lld (must be >= 0)", who, n,
                src_offsets ? src_offsets[n] : 0LL);
   }
-  return DS_OK;
-}
-
-void make_mix_plan(const long long* lengths, const long long* onsets, int K, long long track_len, MixPlan& p) {
   p.n_tiles = (int)((track_len + MIX_TILE - 1) / MIX_TILE);
   std::vector<int> count(p.n_tiles + 1, 0);
   for (int n = 0; n < K; ++n)
@@ -416,29 +376,48 @@ void make_mix_plan(const long long* lengths, const long long* onsets, int K, lon
   std::vector<int> fill(p.tile_ptr.begin(), p.tile_ptr.end() - 1);
   for (int n = 0; n < K; ++n)                                 // ascending n: every tile's list is in input order
     for (long long t = onsets[n] / MIX_TILE; t <= (onsets[n] + lengths[n] - 1) / MIX_TILE; ++t) p.tile_notes[fill[t]++] = n;
-  size_t o = align256(p.tile_ptr.size() * sizeof(int));
-  p.off_notes = o; o = align256(o + p.tile_notes.size() * sizeof(int));
-  p.off_src = o;   o = align256(o + (size_t)K * sizeof(long long));
-  p.off_len = o;   o = align256(o + (size_t)K * sizeof(long long));
-  p.off_onset = o; o = align256(o + (size_t)K * sizeof(long long));
-  p.off_gain = o;  o = align256(o + (size_t)K * sizeof(float));
-  p.bytes = o;
+  p.fade.resize(K);
+  for (int n = 0; n < K; ++n) p.fade[n] = fade_out[n] < lengths[n] ? fade_out[n] : lengths[n];
+  p.ws.stage(p.tile_ptr.data(), p.tile_ptr.size());
+  p.off_notes = p.ws.stage(p.tile_notes.data(), p.tile_notes.size());
+  p.off_src = p.ws.stage(src_offsets, K);
+  p.off_len = p.ws.stage(lengths, K);
+  p.off_onset = p.ws.stage(onsets, K);
+  p.off_gain = p.ws.stage(gains, K);
+  p.off_fade = p.ws.stage(p.fade.data(), K);
+  if (target_peak > 0.f) p.off_peak = p.ws.reserve((size_t)p.n_tiles * sizeof(float));
+  return DS_OK;
 }
 
-// make_mix_plan's layout followed by the K clamped fades and, when normalising, one peak partial per tile
-void make_arrangement_plan(const long long* lengths, const long long* onsets, int K, long long track_len, bool normalise, MixPlan& p) {
-  make_mix_plan(lengths, onsets, K, track_len, p);
-  size_t o = p.bytes;
-  p.off_fade = o; o = align256(o + (size_t)K * sizeof(long long));
-  p.off_peak = o; if (normalise) o = align256(o + (size_t)p.n_tiles * sizeof(float));
-  p.bytes = o;
+int mix_workspace(const long long* lengths, const long long* onsets, const long long* fade_out, int K, float target_peak,
+                  long long track_len, long long* bytes, const char* who) {
+  MixPlan p;
+  int rc = plan_mix(nullptr, lengths, onsets, nullptr, fade_out, K, target_peak, track_len, who, p);
+  if (rc) return rc;
+  *bytes = (long long)p.ws.bytes;
+  return DS_OK;
 }
 
-unsigned grid_for(long long n, int per_block) {
-  long long b = (n + per_block - 1) / per_block;
-  const long long cap = (long long)num_sms() * 32;
-  if (b > cap) b = cap;
-  return (unsigned)(b > 0 ? b : 1);
+int mix(const float* d_src, const long long* src_offsets, const long long* lengths, const long long* onsets, const float* gains,
+        const long long* fade_out, int K, float target_peak, float* d_track, long long track_len, void* d_ws, long long ws_bytes,
+        void* stream, const char* who) {
+  MixPlan p;
+  int rc = plan_mix(src_offsets, lengths, onsets, gains, fade_out, K, target_peak, track_len, who, p);
+  if (rc) return rc;
+  DS_REQUIRE(ws_bytes >= (long long)p.ws.bytes, "%s: workspace of %lld bytes, %zu needed", who, ws_bytes, p.ws.bytes);
+  cudaStream_t st = (cudaStream_t)stream;
+  uint8_t* ws = (uint8_t*)d_ws;
+  float* peak = target_peak > 0.f ? (float*)(ws + p.off_peak) : nullptr;
+  DS_CHECK_CUDA(p.ws.upload(ws, st));
+  DS_CHECK_CUDA(launch_pdl(pitch_arrange_kernel, dim3((unsigned)p.n_tiles), dim3(256), (size_t)0, st, d_src, d_track, track_len,
+                           (const int*)ws, (const int*)(ws + p.off_notes), (const long long*)(ws + p.off_src),
+                           (const long long*)(ws + p.off_len), (const long long*)(ws + p.off_onset), (const float*)(ws + p.off_gain),
+                           (const long long*)(ws + p.off_fade), peak));
+  if (peak)
+    DS_CHECK_CUDA(launch_pdl(pitch_peak_scale_kernel, dim3(grid_for(track_len, 512, 2)), dim3(512), (size_t)0, st, d_track, track_len,
+                             (const float*)peak, p.n_tiles, target_peak));
+  DS_CHECK_CUDA(cudaGetLastError());
+  return DS_OK;
 }
 
 }  // namespace
@@ -450,11 +429,10 @@ extern "C" {
 
 int ds_pitch_shift_workspace(const long long* lengths, const double* n_steps, int B, long long* bytes, long long* stage_offsets) {
   DS_REQUIRE(bytes, "ds_pitch_shift_workspace: bytes must be non-null");
-  int rc = check_pitch_args(lengths, n_steps, B, "ds_pitch_shift_workspace");
-  if (rc) return rc;
   PitchPlan p;
-  make_plan(lengths, n_steps, B, p);
-  *bytes = (long long)p.bytes;
+  int rc = plan_pitch(lengths, n_steps, B, "ds_pitch_shift_workspace", p);
+  if (rc) return rc;
+  *bytes = (long long)p.ws.bytes;
   if (stage_offsets) {
     stage_offsets[0] = (long long)p.off_D;
     stage_offsets[1] = (long long)p.off_S;
@@ -467,26 +445,24 @@ int ds_pitch_shift_workspace(const long long* lengths, const double* n_steps, in
 int ds_pitch_shift(const float* d_in, float* d_out, const long long* lengths, const double* n_steps, int B, void* d_ws, long long ws_bytes,
                    void* stream) {
   DS_REQUIRE(d_in && d_out && d_ws, "ds_pitch_shift: d_in, d_out and d_ws must be non-null");
-  int rc = check_pitch_args(lengths, n_steps, B, "ds_pitch_shift");
-  if (rc) return rc;
   PitchPlan p;
-  make_plan(lengths, n_steps, B, p);
-  DS_REQUIRE(ws_bytes >= (long long)p.bytes, "ds_pitch_shift: workspace of %lld bytes, %zu needed", ws_bytes, p.bytes);
+  int rc = plan_pitch(lengths, n_steps, B, "ds_pitch_shift", p);
+  if (rc) return rc;
+  DS_REQUIRE(ws_bytes >= (long long)p.ws.bytes, "ds_pitch_shift: workspace of %lld bytes, %zu needed", ws_bytes, p.ws.bytes);
   float2 *tw512, *tw1024, *tw2048;
   rc = get_twiddles((cudaStream_t)stream, &tw512, &tw1024, &tw2048);
   if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   uint8_t* ws = (uint8_t*)d_ws;
   const size_t n1 = (size_t)B + 1;
-  const long long* m = (const long long*)ws;
-  const long long *loff = m, *fin = loff + n1, *fout = fin + n1, *yoff = fout + n1, *tcap = yoff + n1, *nval = tcap + B;
-  const double* rate = (const double*)(nval + B);
+  const long long *loff = (const long long*)(ws + p.off_idx), *fin = loff + n1, *fout = fin + n1, *yoff = fout + n1, *tcap = yoff + n1,
+                  *nval = tcap + B;
+  const double* rate = (const double*)(ws + p.off_rate);
   float2* D = (float2*)(ws + p.off_D);
   float2* S = (float2*)(ws + p.off_S);
   float* frames = (float*)(ws + p.off_frames);
   float* ys = (float*)(ws + p.off_ys);
-  // pageable source: the copy is staged before cudaMemcpyAsync returns, so the host plan may go out of scope
-  DS_CHECK_CUDA(cudaMemcpyAsync(ws, p.meta.data(), p.meta.size() * sizeof(long long), cudaMemcpyHostToDevice, st));
+  DS_CHECK_CUDA(p.ws.upload(ws, st));
   const size_t smem = FR * XS_PITCH * sizeof(float2);
   DS_CHECK_CUDA(cudaFuncSetAttribute(pitch_stft_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   DS_CHECK_CUDA(cudaFuncSetAttribute(pitch_istft_frames_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -496,9 +472,9 @@ int ds_pitch_shift(const float* d_in, float* d_out, const long long* lengths, co
                            (const float2*)D, S, fin, fout, rate, B));
   DS_CHECK_CUDA(launch_pdl(pitch_istft_frames_kernel, dim3((unsigned)((p.n_out_frames + FR - 1) / FR)), dim3(256), smem, st,
                            (const float2*)S, frames, p.n_out_frames, (const float2*)tw1024, (const float2*)tw2048));
-  DS_CHECK_CUDA(launch_pdl(pitch_ola_kernel, dim3(grid_for(p.n_ys, 256)), dim3(256), (size_t)0, st, (const float*)frames, ys, fout, yoff,
-                           tcap, B));
-  DS_CHECK_CUDA(launch_pdl(pitch_resample_kernel, dim3(grid_for(p.n_samples, 256)), dim3(256), (size_t)0, st, (const float*)ys, d_out,
+  DS_CHECK_CUDA(launch_pdl(pitch_ola_kernel, dim3(grid_for(p.n_ys, 256, 32)), dim3(256), (size_t)0, st, (const float*)frames, ys, fout,
+                           yoff, tcap, B));
+  DS_CHECK_CUDA(launch_pdl(pitch_resample_kernel, dim3(grid_for(p.n_samples, 256, 32)), dim3(256), (size_t)0, st, (const float*)ys, d_out,
                            loff, yoff, nval, rate, B, (float)(1.0 / bessel_i0(RS_BETA))));
   DS_CHECK_CUDA(cudaGetLastError());
   return DS_OK;
@@ -506,49 +482,21 @@ int ds_pitch_shift(const float* d_in, float* d_out, const long long* lengths, co
 
 int ds_mix_track_workspace(const long long* lengths, const long long* onsets, int K, long long track_len, long long* bytes) {
   DS_REQUIRE(bytes, "ds_mix_track_workspace: bytes must be non-null");
-  int rc = check_mix_args(lengths, onsets, K, track_len, "ds_mix_track_workspace");
-  if (rc) return rc;
-  MixPlan p;
-  make_mix_plan(lengths, onsets, K, track_len, p);
-  *bytes = (long long)p.bytes;
-  return DS_OK;
+  return mix_workspace(lengths, onsets, std::vector<long long>(K > 0 ? K : 0).data(), K, 0.f, track_len, bytes,
+                       "ds_mix_track_workspace");
 }
 
 int ds_mix_track(const float* d_src, const long long* src_off, const long long* lengths, const long long* onsets, const float* gains, int K,
                  float* d_track, long long track_len, void* d_ws, long long ws_bytes, void* stream) {
   DS_REQUIRE(d_src && d_track && d_ws && src_off && gains, "ds_mix_track: d_src, d_track, d_ws, src_off and gains must be non-null");
-  int rc = check_mix_args(lengths, onsets, K, track_len, "ds_mix_track");
-  if (rc) return rc;
-  for (int n = 0; n < K; ++n) DS_REQUIRE(src_off[n] >= 0, "ds_mix_track: note %d has source offset %lld", n, src_off[n]);
-  MixPlan p;
-  make_mix_plan(lengths, onsets, K, track_len, p);
-  DS_REQUIRE(ws_bytes >= (long long)p.bytes, "ds_mix_track: workspace of %lld bytes, %zu needed", ws_bytes, p.bytes);
-  std::vector<uint8_t> host(p.bytes, 0);
-  memcpy(host.data(), p.tile_ptr.data(), p.tile_ptr.size() * sizeof(int));
-  memcpy(host.data() + p.off_notes, p.tile_notes.data(), p.tile_notes.size() * sizeof(int));
-  memcpy(host.data() + p.off_src, src_off, (size_t)K * sizeof(long long));
-  memcpy(host.data() + p.off_len, lengths, (size_t)K * sizeof(long long));
-  memcpy(host.data() + p.off_onset, onsets, (size_t)K * sizeof(long long));
-  memcpy(host.data() + p.off_gain, gains, (size_t)K * sizeof(float));
-  cudaStream_t st = (cudaStream_t)stream;
-  uint8_t* ws = (uint8_t*)d_ws;
-  DS_CHECK_CUDA(cudaMemcpyAsync(ws, host.data(), p.bytes, cudaMemcpyHostToDevice, st));
-  DS_CHECK_CUDA(launch_pdl(pitch_mix_kernel, dim3((unsigned)p.n_tiles), dim3(256), (size_t)0, st, d_src, d_track, track_len,
-                           (const int*)ws, (const int*)(ws + p.off_notes), (const long long*)(ws + p.off_src),
-                           (const long long*)(ws + p.off_len), (const long long*)(ws + p.off_onset), (const float*)(ws + p.off_gain)));
-  DS_CHECK_CUDA(cudaGetLastError());
-  return DS_OK;
+  return mix(d_src, src_off, lengths, onsets, gains, std::vector<long long>(K > 0 ? K : 0).data(), K, 0.f, d_track, track_len, d_ws,
+             ws_bytes, stream, "ds_mix_track");
 }
 
 int ds_mix_arrangement_workspace(const long long* lengths, const long long* onsets, const long long* fade_out, int K, float target_peak,
                                  long long track_len, long long* bytes) {
   DS_REQUIRE(bytes && fade_out, "ds_mix_arrangement_workspace: bytes and fade_out must be non-null");
-  int rc = check_mix_args(lengths, onsets, K, track_len, "ds_mix_arrangement_workspace", fade_out, target_peak);
-  if (rc) return rc;
-  MixPlan p;
-  make_arrangement_plan(lengths, onsets, K, track_len, target_peak > 0.f, p);
-  *bytes = (long long)p.bytes;
-  return DS_OK;
+  return mix_workspace(lengths, onsets, fade_out, K, target_peak, track_len, bytes, "ds_mix_arrangement_workspace");
 }
 
 int ds_mix_arrangement(const float* d_src, const long long* src_offsets, const long long* lengths, const long long* onsets,
@@ -556,37 +504,8 @@ int ds_mix_arrangement(const float* d_src, const long long* src_offsets, const l
                        void* d_ws, long long ws_bytes, void* stream) {
   DS_REQUIRE(d_src && d_track && d_ws && src_offsets && gains && fade_out,
              "ds_mix_arrangement: d_src, d_track, d_ws, src_offsets, gains and fade_out must be non-null");
-  int rc = check_mix_args(lengths, onsets, K, track_len, "ds_mix_arrangement", fade_out, target_peak, src_offsets);
-  if (rc) return rc;
-  const bool normalise = target_peak > 0.f;
-  MixPlan p;
-  make_arrangement_plan(lengths, onsets, K, track_len, normalise, p);
-  DS_REQUIRE(ws_bytes >= (long long)p.bytes, "ds_mix_arrangement: workspace of %lld bytes, %zu needed", ws_bytes, p.bytes);
-  std::vector<uint8_t> host(p.off_peak, 0);                 // everything but the partials, which the mix kernel writes
-  memcpy(host.data(), p.tile_ptr.data(), p.tile_ptr.size() * sizeof(int));
-  memcpy(host.data() + p.off_notes, p.tile_notes.data(), p.tile_notes.size() * sizeof(int));
-  memcpy(host.data() + p.off_src, src_offsets, (size_t)K * sizeof(long long));
-  memcpy(host.data() + p.off_len, lengths, (size_t)K * sizeof(long long));
-  memcpy(host.data() + p.off_onset, onsets, (size_t)K * sizeof(long long));
-  memcpy(host.data() + p.off_gain, gains, (size_t)K * sizeof(float));
-  long long* fade = (long long*)(host.data() + p.off_fade);
-  for (int n = 0; n < K; ++n) fade[n] = fade_out[n] < lengths[n] ? fade_out[n] : lengths[n];
-  cudaStream_t st = (cudaStream_t)stream;
-  uint8_t* ws = (uint8_t*)d_ws;
-  float* peak = normalise ? (float*)(ws + p.off_peak) : nullptr;
-  DS_CHECK_CUDA(cudaMemcpyAsync(ws, host.data(), host.size(), cudaMemcpyHostToDevice, st));
-  DS_CHECK_CUDA(launch_pdl(pitch_arrange_kernel, dim3((unsigned)p.n_tiles), dim3(256), (size_t)0, st, d_src, d_track, track_len,
-                           (const int*)ws, (const int*)(ws + p.off_notes), (const long long*)(ws + p.off_src),
-                           (const long long*)(ws + p.off_len), (const long long*)(ws + p.off_onset), (const float*)(ws + p.off_gain),
-                           (const long long*)(ws + p.off_fade), peak));
-  if (normalise) {
-    long long blocks = (track_len + 511) / 512;
-    if (blocks > 2LL * num_sms()) blocks = 2LL * num_sms();
-    DS_CHECK_CUDA(launch_pdl(pitch_peak_scale_kernel, dim3((unsigned)blocks), dim3(512), (size_t)0, st, d_track, track_len,
-                             (const float*)peak, p.n_tiles, target_peak));
-  }
-  DS_CHECK_CUDA(cudaGetLastError());
-  return DS_OK;
+  return mix(d_src, src_offsets, lengths, onsets, gains, fade_out, K, target_peak, d_track, track_len, d_ws, ws_bytes, stream,
+             "ds_mix_arrangement");
 }
 
 }  // extern "C"

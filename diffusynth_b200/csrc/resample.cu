@@ -22,9 +22,6 @@
 namespace ds {
 namespace {
 
-constexpr int RS_ZEROS = 64;
-constexpr double RS_ROLLOFF = 0.9475937167399596, RS_BETA = 14.769656459379492;   // resampy kaiser_best (as pitch.cu)
-constexpr double kPi = 3.14159265358979323846;
 constexpr int THREADS = 256, WARPS = THREADS / 32;
 constexpr long long TABLE_CAP = 1LL << 20;     // coefficients per (o, t) pair; larger tables take the direct path
 constexpr int WIN_CAP = 24576;                 // staged input floats per CTA; a pair needing more takes the direct path
@@ -44,15 +41,6 @@ struct RsPair {
   long long up, down, F, taps4;
   double ratio;
 };
-
-__device__ __forceinline__ int find_item(const long long* __restrict__ off, int B, long long g) {
-  int lo = 0, hi = B - 1;
-  while (lo < hi) {
-    const int mid = (lo + hi + 1) >> 1;
-    if (__ldg(off + mid) <= g) lo = mid; else hi = mid - 1;
-  }
-  return lo;
-}
 
 // h(m - p/up) in float64, rounded once to fp32; zero outside the filter's support |m - p/up| <= 64/s, which is decided in integers
 // (|m*up - p| <= 64*max(up, down)) so that the taps exactly at the edge count.  Shared by the table build and the direct path, so
@@ -202,18 +190,16 @@ resample_kernel(const float* __restrict__ x, float* __restrict__ y, const RsItem
   }
 }
 
-size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
-
 struct ResamplePlan {
   std::vector<RsItem> items;
   std::vector<long long> tiles, ptiles, poff;            // prefix offsets: resample tiles, peak tiles, table coefficients
   std::vector<RsPair> pairs;
-  size_t off_items = 0, off_tiles = 0, off_ptiles = 0, off_pairs = 0, off_poff = 0, meta_bytes = 0;
-  size_t off_tab = 0, off_peak = 0, bytes = 0, smem = 0;
+  Workspace ws;
+  size_t off_items = 0, off_tiles = 0, off_ptiles = 0, off_pairs = 0, off_poff = 0, off_tab = 0, off_peak = 0, smem = 0;
 };
 
-int check_args(const long long* lengths, const long long* sr_in, const long long* sr_out, const long long* out_lengths, int B,
-               const char* who) {
+int plan_resample(const long long* lengths, const long long* sr_in, const long long* sr_out, const long long* out_lengths, int B,
+                  const char* who, ResamplePlan& p) {
   DS_REQUIRE(lengths && sr_in && sr_out && B > 0, "%s: lengths, sr_in and sr_out must be non-null and B > 0 (B = %d)", who, B);
   for (int k = 0; k < B; ++k) {
     DS_REQUIRE(lengths[k] > 0 && lengths[k] <= DS_RESAMPLE_MAX_LENGTH, "%s: item %d has length %lld (must be in 1..%lld)", who, k,
@@ -224,11 +210,6 @@ int check_args(const long long* lengths, const long long* sr_in, const long long
       DS_REQUIRE(out_lengths[k] > 0 && out_lengths[k] <= DS_RESAMPLE_MAX_LENGTH, "%s: item %d has output length %lld (must be in 1..%lld)",
                  who, k, out_lengths[k], (long long)DS_RESAMPLE_MAX_LENGTH);
   }
-  return DS_OK;
-}
-
-void make_plan(const long long* lengths, const long long* sr_in, const long long* sr_out, const long long* out_lengths, int B,
-               ResamplePlan& p) {
   const char* env = getenv("DS_RESAMPLE_DIRECT");             // A/B timing and tests: every resampled item takes the direct path
   const bool force_direct = env && atoi(env) != 0;
   p.items.assign(B, RsItem{});
@@ -286,25 +267,15 @@ void make_plan(const long long* lengths, const long long* sr_in, const long long
     p.tiles[k + 1] = p.tiles[k] + (it.out_len + it.tile_out - 1) / it.tile_out;
     p.ptiles[k + 1] = p.ptiles[k] + (L + PEAK_TILE - 1) / PEAK_TILE;
   }
-  const size_t P = p.pairs.size();
-  size_t o = 0;
-  p.off_items = o;  o = align256(o + p.items.size() * sizeof(RsItem));
-  p.off_tiles = o;  o = align256(o + p.tiles.size() * sizeof(long long));
-  p.off_ptiles = o; o = align256(o + p.ptiles.size() * sizeof(long long));
-  p.off_pairs = o;  o = align256(o + (P ? P : 1) * sizeof(RsPair));
-  p.off_poff = o;   o = align256(o + p.poff.size() * sizeof(long long));
-  p.meta_bytes = o;
-  p.off_tab = o;    o = align256(o + (size_t)p.poff.back() * sizeof(float));
-  p.off_peak = o;   o = align256(o + (size_t)B * sizeof(unsigned));
-  p.bytes = o;
+  p.off_items = p.ws.stage(p.items.data(), p.items.size());
+  p.off_tiles = p.ws.stage(p.tiles.data(), p.tiles.size());
+  p.off_ptiles = p.ws.stage(p.ptiles.data(), p.ptiles.size());
+  p.off_pairs = p.ws.stage(p.pairs.data(), p.pairs.size());
+  p.off_poff = p.ws.stage(p.poff.data(), p.poff.size());
+  p.off_tab = p.ws.reserve((size_t)p.poff.back() * sizeof(float));
+  p.off_peak = p.ws.reserve((size_t)B * sizeof(unsigned));
   p.smem = smem_floats * sizeof(float);
-}
-
-unsigned grid_for(long long n, int per_block) {
-  long long b = (n + per_block - 1) / per_block;
-  const long long cap = (long long)num_sms() * 32;
-  if (b > cap) b = cap;
-  return (unsigned)(b > 0 ? b : 1);
+  return DS_OK;
 }
 
 }  // namespace
@@ -317,28 +288,20 @@ extern "C" {
 int ds_resample_workspace(const long long* lengths, const long long* sr_in, const long long* sr_out, const long long* out_lengths, int B,
                           long long* bytes) {
   DS_REQUIRE(bytes, "ds_resample_workspace: bytes must be non-null");
-  int rc = check_args(lengths, sr_in, sr_out, out_lengths, B, "ds_resample_workspace");
-  if (rc) return rc;
   ResamplePlan p;
-  make_plan(lengths, sr_in, sr_out, out_lengths, B, p);
-  *bytes = (long long)p.bytes;
+  int rc = plan_resample(lengths, sr_in, sr_out, out_lengths, B, "ds_resample_workspace", p);
+  if (rc) return rc;
+  *bytes = (long long)p.ws.bytes;
   return DS_OK;
 }
 
 int ds_resample(const float* d_in, float* d_out, const long long* lengths, const long long* sr_in, const long long* sr_out,
                 const long long* out_lengths, int normalize_peak, int B, void* d_ws, long long ws_bytes, void* stream) {
   DS_REQUIRE(d_in && d_out && d_ws, "ds_resample: d_in, d_out and d_ws must be non-null");
-  int rc = check_args(lengths, sr_in, sr_out, out_lengths, B, "ds_resample");
-  if (rc) return rc;
   ResamplePlan p;
-  make_plan(lengths, sr_in, sr_out, out_lengths, B, p);
-  DS_REQUIRE(ws_bytes >= (long long)p.bytes, "ds_resample: workspace of %lld bytes, %zu needed", ws_bytes, p.bytes);
-  std::vector<uint8_t> host(p.meta_bytes, 0);
-  memcpy(host.data() + p.off_items, p.items.data(), p.items.size() * sizeof(RsItem));
-  memcpy(host.data() + p.off_tiles, p.tiles.data(), p.tiles.size() * sizeof(long long));
-  memcpy(host.data() + p.off_ptiles, p.ptiles.data(), p.ptiles.size() * sizeof(long long));
-  if (!p.pairs.empty()) memcpy(host.data() + p.off_pairs, p.pairs.data(), p.pairs.size() * sizeof(RsPair));
-  memcpy(host.data() + p.off_poff, p.poff.data(), p.poff.size() * sizeof(long long));
+  int rc = plan_resample(lengths, sr_in, sr_out, out_lengths, B, "ds_resample", p);
+  if (rc) return rc;
+  DS_REQUIRE(ws_bytes >= (long long)p.ws.bytes, "ds_resample: workspace of %lld bytes, %zu needed", ws_bytes, p.ws.bytes);
   cudaStream_t st = (cudaStream_t)stream;
   uint8_t* ws = (uint8_t*)d_ws;
   const RsItem* items = (const RsItem*)(ws + p.off_items);
@@ -346,10 +309,9 @@ int ds_resample(const float* d_in, float* d_out, const long long* lengths, const
   const long long* ptiles = (const long long*)(ws + p.off_ptiles);
   float* tab = (float*)(ws + p.off_tab);
   unsigned* peak = (unsigned*)(ws + p.off_peak);
-  // pageable source: the copy is staged before cudaMemcpyAsync returns, so the host plan may go out of scope
-  DS_CHECK_CUDA(cudaMemcpyAsync(ws, host.data(), p.meta_bytes, cudaMemcpyHostToDevice, st));
+  DS_CHECK_CUDA(p.ws.upload(ws, st));
   const long long n_coef = p.poff.back();
-  DS_CHECK_CUDA(launch_pdl(resample_table_kernel, dim3(grid_for(n_coef > B ? n_coef : B, THREADS)), dim3(THREADS), (size_t)0, st,
+  DS_CHECK_CUDA(launch_pdl(resample_table_kernel, dim3(grid_for(n_coef > B ? n_coef : B, THREADS, 32)), dim3(THREADS), (size_t)0, st,
                            (const RsPair*)(ws + p.off_pairs), (const long long*)(ws + p.off_poff), (int)p.pairs.size(), tab, peak, B));
   if (normalize_peak)
     DS_CHECK_CUDA(launch_pdl(resample_peak_kernel, dim3((unsigned)p.ptiles[B]), dim3(THREADS), (size_t)0, st, d_in, items, ptiles, B,

@@ -25,15 +25,6 @@ struct ZmItem {
   long long H, W, h, w;
 };
 
-__device__ __forceinline__ int find_item(const long long* __restrict__ off, int B, long long g) {
-  int lo = 0, hi = B - 1;
-  while (lo < hi) {
-    const int mid = (lo + hi + 1) >> 1;
-    if (__ldg(off + mid) <= g) lo = mid; else hi = mid - 1;
-  }
-  return lo;
-}
-
 constexpr int CH = 8;                             // values a thread loads before it uses them: the walks are serial, the loads need not be
 
 __device__ __forceinline__ double pole() { return sqrt(3.0) - 2.0; }
@@ -141,15 +132,14 @@ zoom_rows_kernel(const ZmItem* __restrict__ items, const long long* __restrict__
   }
 }
 
-size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
-
 struct ZoomPlan {
   std::vector<ZmItem> items;
   std::vector<long long> colpre, rowpre;
-  size_t off_items = 0, off_colpre = 0, off_rowpre = 0, meta_bytes = 0, off_coef = 0, off_mid = 0, bytes = 0;
+  Workspace ws;
+  size_t off_items = 0, off_colpre = 0, off_rowpre = 0, off_coef = 0, off_mid = 0;
 };
 
-int check_args(const long long* in_shapes, const long long* out_shapes, int B, const char* who) {
+int plan_zoom(const long long* in_shapes, const long long* out_shapes, int B, const char* who, ZoomPlan& p) {
   DS_REQUIRE(in_shapes && out_shapes && B > 0, "%s: in_shapes and out_shapes must be non-null and B > 0 (B = %d)", who, B);
   for (int k = 0; k < B; ++k) {
     const long long H = in_shapes[2 * k], W = in_shapes[2 * k + 1], h = out_shapes[2 * k], w = out_shapes[2 * k + 1];
@@ -158,10 +148,6 @@ int check_args(const long long* in_shapes, const long long* out_shapes, int B, c
                "%s: item %d is %lld x %lld -> %lld x %lld (every dimension must be in 1..%lld)", who, k, H, W, h, w,
                (long long)DS_MASK_ZOOM_MAX_DIM);
   }
-  return DS_OK;
-}
-
-void make_plan(const long long* in_shapes, const long long* out_shapes, int B, ZoomPlan& p) {
   p.items.assign(B, ZmItem{});
   p.colpre.assign(B + 1, 0);
   p.rowpre.assign(B + 1, 0);
@@ -181,21 +167,12 @@ void make_plan(const long long* in_shapes, const long long* out_shapes, int B, Z
     p.colpre[k + 1] = p.colpre[k] + it.W;
     p.rowpre[k + 1] = p.rowpre[k] + it.h;
   }
-  size_t o = 0;
-  p.off_items = o;  o = align256(o + p.items.size() * sizeof(ZmItem));
-  p.off_colpre = o; o = align256(o + p.colpre.size() * sizeof(long long));
-  p.off_rowpre = o; o = align256(o + p.rowpre.size() * sizeof(long long));
-  p.meta_bytes = o;
-  p.off_coef = o;   o = align256(o + (size_t)in_off * sizeof(double));
-  p.off_mid = o;    o = align256(o + (size_t)mid_off * sizeof(double));
-  p.bytes = o;
-}
-
-unsigned grid_for(long long n) {
-  long long b = (n + THREADS - 1) / THREADS;
-  const long long cap = (long long)num_sms() * 16;
-  if (b > cap) b = cap;
-  return (unsigned)(b > 0 ? b : 1);
+  p.off_items = p.ws.stage(p.items.data(), p.items.size());
+  p.off_colpre = p.ws.stage(p.colpre.data(), p.colpre.size());
+  p.off_rowpre = p.ws.stage(p.rowpre.data(), p.rowpre.size());
+  p.off_coef = p.ws.reserve((size_t)in_off * sizeof(double));
+  p.off_mid = p.ws.reserve((size_t)mid_off * sizeof(double));
+  return DS_OK;
 }
 
 }  // namespace
@@ -207,36 +184,29 @@ extern "C" {
 
 int ds_mask_zoom_workspace(const long long* in_shapes, const long long* out_shapes, int B, long long* bytes) {
   DS_REQUIRE(bytes, "ds_mask_zoom_workspace: bytes must be non-null");
-  int rc = check_args(in_shapes, out_shapes, B, "ds_mask_zoom_workspace");
-  if (rc) return rc;
   ZoomPlan p;
-  make_plan(in_shapes, out_shapes, B, p);
-  *bytes = (long long)p.bytes;
+  int rc = plan_zoom(in_shapes, out_shapes, B, "ds_mask_zoom_workspace", p);
+  if (rc) return rc;
+  *bytes = (long long)p.ws.bytes;
   return DS_OK;
 }
 
 int ds_mask_zoom(const float* d_in, float* d_out, const long long* in_shapes, const long long* out_shapes, int B, void* d_ws,
                  long long ws_bytes, void* stream) {
   DS_REQUIRE(d_in && d_out && d_ws, "ds_mask_zoom: d_in, d_out and d_ws must be non-null");
-  int rc = check_args(in_shapes, out_shapes, B, "ds_mask_zoom");
-  if (rc) return rc;
   ZoomPlan p;
-  make_plan(in_shapes, out_shapes, B, p);
-  DS_REQUIRE(ws_bytes >= (long long)p.bytes, "ds_mask_zoom: workspace of %lld bytes, %zu needed", ws_bytes, p.bytes);
-  std::vector<uint8_t> host(p.meta_bytes, 0);
-  memcpy(host.data() + p.off_items, p.items.data(), p.items.size() * sizeof(ZmItem));
-  memcpy(host.data() + p.off_colpre, p.colpre.data(), p.colpre.size() * sizeof(long long));
-  memcpy(host.data() + p.off_rowpre, p.rowpre.data(), p.rowpre.size() * sizeof(long long));
+  int rc = plan_zoom(in_shapes, out_shapes, B, "ds_mask_zoom", p);
+  if (rc) return rc;
+  DS_REQUIRE(ws_bytes >= (long long)p.ws.bytes, "ds_mask_zoom: workspace of %lld bytes, %zu needed", ws_bytes, p.ws.bytes);
   cudaStream_t st = (cudaStream_t)stream;
   uint8_t* ws = (uint8_t*)d_ws;
   const ZmItem* items = (const ZmItem*)(ws + p.off_items);
   double* coef = (double*)(ws + p.off_coef);
   double* mid = (double*)(ws + p.off_mid);
-  // pageable source: the copy is staged before cudaMemcpyAsync returns, so the host plan may go out of scope
-  DS_CHECK_CUDA(cudaMemcpyAsync(ws, host.data(), p.meta_bytes, cudaMemcpyHostToDevice, st));
-  DS_CHECK_CUDA(launch_pdl(zoom_cols_kernel, dim3(grid_for(p.colpre[B])), dim3(THREADS), (size_t)0, st, d_in, items,
+  DS_CHECK_CUDA(p.ws.upload(ws, st));
+  DS_CHECK_CUDA(launch_pdl(zoom_cols_kernel, dim3(grid_for(p.colpre[B], THREADS, 16)), dim3(THREADS), (size_t)0, st, d_in, items,
                            (const long long*)(ws + p.off_colpre), B, coef, mid));
-  DS_CHECK_CUDA(launch_pdl(zoom_rows_kernel, dim3(grid_for(p.rowpre[B])), dim3(THREADS), (size_t)0, st, items,
+  DS_CHECK_CUDA(launch_pdl(zoom_rows_kernel, dim3(grid_for(p.rowpre[B], THREADS, 16)), dim3(THREADS), (size_t)0, st, items,
                            (const long long*)(ws + p.off_rowpre), B, mid, d_out));
   DS_CHECK_CUDA(cudaGetLastError());
   return DS_OK;

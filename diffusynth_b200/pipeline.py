@@ -11,8 +11,8 @@ import torch
 
 from . import _lib, ops, weights as W
 from ._lib import check
-from .codec import MORPH_PATHS, SAMPLE_RATE, _layout, _pack, morph_rows, resample_packed, shift_and_mix, spectrogram_to_waveform, \
-    waveform_to_spectrogram, zoom_packed
+from .codec import MORPH_PATHS, SAMPLE_RATE, _check_peak, _layout, _pack, morph_rows, resample_packed, shift_and_mix, \
+    spectrogram_to_waveform, waveform_to_spectrogram, zoom_packed
 from .sampler import DiffSynthSampler
 from .unet import ConditionedUnet
 from .vqgan import VQGAN
@@ -463,10 +463,10 @@ class TextToTimbre:
         takes them.  The (track, duration) rows of ALL tracks are synthesised with one graph launch per distinct width, each row
         with its own instrument latent and condition; every distinct (row, semitones) item is pitch-shifted in one call; every note
         is placed with its gain times its track's gain, faded out linearly over the last fade_out_sec of its waveform, and summed
-        in one call (ds_mix_arrangement).  ``target_peak``: None, or max |result| after a peak normalisation on the device.
-        ``noise_feeds`` (tests): one per row (arrangement_plan), in row order.  Returns the fp32 piece [max(onset + note length)]."""
-        if target_peak is not None and not (np.isfinite(float(target_peak)) and float(target_peak) > 0.0):
-            raise ValueError(f"target_peak must be None or a finite value > 0, got {target_peak}")
+        in one call (ds_mix_arrangement).  ``target_peak``: None, or max |result| after a peak normalisation on the device, a
+        finite value > 0 (codec._check_peak, before any synthesis).  ``noise_feeds`` (tests): one per row (arrangement_plan), in row
+        order.  Returns the fp32 piece [max(onset + note length)]."""
+        _check_peak(target_peak)
         return self._render(tracks, sample_steps, noising_strength, attack, before_release, sampler, time_resolution, vae_scale,
                             noise_feeds, fades=True, target_peak=target_peak)
 

@@ -247,7 +247,9 @@ int ds_pitch_shift(const float* d_in, float* d_out, const long long* lengths, co
                    void* stream);
 /* Track mix (track_maker.py's placement loop): d_track[j] = sum over notes n in input order, fp32, of
    gains[n] * d_src[src_offsets[n] + j - onsets[n]] where 0 <= j - onsets[n] < lengths[n]; no normalisation, no envelope.  A gather
-   over track samples, bit-identical run to run.  Every onsets[n] + lengths[n] <= track_len.  d_ws: ds_mix_track_workspace bytes. */
+   over track samples, bit-identical run to run.  Every onsets[n] + lengths[n] <= track_len, src_offsets[n] >= 0.  This is
+   ds_mix_arrangement with every fade_out 0 and target_peak 0, and its workspace holds those K int64 fades too: as with every
+   call here, size d_ws from ds_mix_track_workspace, never from a formula. */
 int ds_mix_track_workspace(const long long* lengths, const long long* onsets, int K, long long track_len, long long* bytes);
 int ds_mix_track(const float* d_src, const long long* src_offsets, const long long* lengths, const long long* onsets, const float* gains,
                  int K, float* d_track, long long track_len, void* d_ws, long long ws_bytes, void* stream);

@@ -9,7 +9,7 @@ random init, 20 DDIM steps, the default tiling policy.  Prints one JSON line (an
 maximum SM clock read in the same run; the device-timed medians (CUDA events around each call, which ends in a device synchronise)
 of --repeats calls of each, alternating the two; the graph launches of each; the rel-L2 between the loop's sum and a fade-free,
 unnormalised render_arrangement; and, for the mix alone, the
-call's device-timed median, its kernels' times from torch.profiler in a separate run, and the bytes the mix needs (every note sample
+call's device-timed median (with fades, with fades and a peak, and as mix_track: the same notes without fades), its kernels' times from torch.profiler in a separate run, and the bytes the mix needs (every note sample
 read once, the track written once; the normalisation reads and writes the track again) over the kernel time, against the
 B200's 7.7 TB/s HBM3e data-sheet bandwidth.  Exits non-zero without a CUDA device.
 
@@ -125,18 +125,19 @@ def main() -> int:
         return codec.mix_arrangement(src, offs, lengths, onsets, gains, fades, target_peak=peak, track_len=track_len)
 
     mix_ms = {}
-    for peak in (None, 0.9):
-        mix(peak)
+    for name, fn in (("plain", lambda: mix(None)), ("peak", lambda: mix(0.9)),
+                     ("track", lambda: codec.mix_track(src, offs, lengths, onsets, gains, track_len=track_len))):
+        fn()
         torch.cuda.synchronize()
         t = []
         for _ in range(20):
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-            mix(peak)
+            fn()
             e1.record()
             e1.synchronize()
             t.append(e0.elapsed_time(e1))
-        mix_ms["peak" if peak else "plain"] = t
+        mix_ms[name] = t
     kern = {}
     try:                                                                        # a separate, profiled run
         from torch.profiler import ProfilerActivity, profile
@@ -156,6 +157,7 @@ def main() -> int:
     scale_bytes = 8.0 * track_len
     mix_line = dict(notes=K, note_samples=L, track_samples=track_len, source_mb=round(K * L * 4 / 1e6, 1),
                     call_ms_plain=round(float(np.median(mix_ms["plain"])), 4), call_ms_peak=round(float(np.median(mix_ms["peak"])), 4),
+                    call_ms_track=round(float(np.median(mix_ms["track"])), 4),
                     call_note="host plan + one metadata copy + kernels, CUDA events around the call",
                     kernel_ms_profiled={k: round(v, 4) for k, v in kern.items()} or "not measured")
     if "pitch_arrange_kernel" in kern:
