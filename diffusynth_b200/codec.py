@@ -241,9 +241,10 @@ def mix_track(packed: torch.Tensor, src_offsets, lengths, onsets, gains, track_l
 
 
 def _mix(packed: torch.Tensor, src_offsets, lengths, onsets, gains, track_len, fade: Optional[np.ndarray] = None,
-         peak: float = 0.0) -> torch.Tensor:
-    """mix_track (``fade`` None: ds_mix_track) or mix_arrangement (int64 ``fade``: ds_mix_arrangement, whose extra arguments are
-    the fades before the note count and the peak after it): host arrays, workspace query, allocation, launch."""
+         peak: float = 0.0, pans: Optional[np.ndarray] = None) -> torch.Tensor:
+    """mix_track (``fade`` None: ds_mix_track), mix_arrangement (int64 ``fade``: ds_mix_arrangement, whose extra arguments are
+    the fades before the note count and the peak after it) or mix_stereo (fp32 ``pans`` too: ds_mix_stereo, which takes the pans
+    before the fades, and a [2, track_len] output): host arrays, workspace query, allocation, launch."""
     lib = _lib.load()
     off = np.ascontiguousarray(src_offsets, dtype=np.int64)
     L = np.ascontiguousarray(lengths, dtype=np.int64)
@@ -252,12 +253,17 @@ def _mix(packed: torch.Tensor, src_offsets, lengths, onsets, gains, track_len, f
     K = len(L)
     if track_len is None:
         track_len = int((on + L).max())
-    name, fk = ("ds_mix_track", (K,)) if fade is None else ("ds_mix_arrangement", (fade.ctypes.data, K, peak))
+    if pans is not None:
+        name, wk, fk = "ds_mix_stereo", (fade.ctypes.data, pans.ctypes.data, K, peak), (pans.ctypes.data, fade.ctypes.data, K, peak)
+    else:
+        name, fk = ("ds_mix_track", (K,)) if fade is None else ("ds_mix_arrangement", (fade.ctypes.data, K, peak))
+        wk = fk
     nbytes = C.c_longlong(0)
-    check(getattr(lib, name + "_workspace")(L.ctypes.data, on.ctypes.data, *fk, int(track_len), C.byref(nbytes)), name + "_workspace")
+    check(getattr(lib, name + "_workspace")(L.ctypes.data, on.ctypes.data, *wk, int(track_len), C.byref(nbytes)), name + "_workspace")
     packed = packed.float().contiguous()
     ws = torch.empty((nbytes.value,), dtype=torch.uint8, device=packed.device)
-    track = torch.empty((int(track_len),), dtype=torch.float32, device=packed.device)
+    shape = (int(track_len),) if pans is None else (2, int(track_len))
+    track = torch.empty(shape, dtype=torch.float32, device=packed.device)
     check(getattr(lib, name)(packed.data_ptr(), off.ctypes.data, L.ctypes.data, on.ctypes.data, g.ctypes.data, *fk, track.data_ptr(),
                              int(track_len), ws.data_ptr(), nbytes.value, ops._stream()), name)
     return track
@@ -279,23 +285,53 @@ def mix_arrangement(packed: torch.Tensor, src_offsets, lengths, onsets, gains, f
     """mix_track with a linear fade over the last fade_out[n] samples of every note (clamped to the note; 0 = none) and, when
     ``target_peak`` is given, the track scaled on the device so that max |track| == target_peak (ds_mix_arrangement).  Notes
     without a fade are summed exactly as mix_track sums them.  Summed in note order, bit-identical run to run."""
-    fade = np.ascontiguousarray(fade_out, dtype=np.int64)
     peak = _check_peak(target_peak)
+    return _mix(packed, src_offsets, lengths, onsets, gains, track_len, _check_fades(fade_out), peak)
+
+
+def _check_fades(fade_out) -> np.ndarray:
+    """Per note: int64 samples >= 0."""
+    fade = np.ascontiguousarray(fade_out, dtype=np.int64)
     if np.any(fade < 0):
         raise ValueError(f"fade_out must be >= 0, got {fade_out}")
-    return _mix(packed, src_offsets, lengths, onsets, gains, track_len, fade, peak)
+    return fade
 
 
-def shift_and_mix(sources, semitones, note_source, onsets, gains, fades=None, target_peak: Optional[float] = None) -> torch.Tensor:
+def _check_pans(pans, count: int) -> np.ndarray:
+    """One fp32 pan per note, finite, in [-1, 1]."""
+    p = np.ascontiguousarray(pans, dtype=np.float32).reshape(-1)
+    if p.shape != (count,) or not np.all(np.isfinite(p)) or np.any(np.abs(p) > 1):
+        raise ValueError(f"pans must be {count} finite values in [-1, 1], got {pans}")
+    return p
+
+
+@torch.no_grad()
+def mix_stereo(packed: torch.Tensor, src_offsets, lengths, onsets, gains, pans, fade_out=None, target_peak: Optional[float] = None,
+               track_len: Optional[int] = None) -> torch.Tensor:
+    """mix_arrangement into two channels (ds_mix_stereo): note n is panned by pans[n] in [-1, 1] (-1 left, 0 centre, 1 right) with
+    the constant-power law g_L = g cos(pi (1 + p) / 4), g_R = g cos(pi (1 - p) / 4), evaluated in float64 and rounded once, with a
+    hard pan exactly 0 in the other channel.  ``fade_out``: None (no fades) or per note, as mix_arrangement takes it.  With
+    ``target_peak``, both channels are scaled by one factor so that max |x| over both is the target.  Returns the planar fp32
+    [2, track_len] (left, right); summed in note order, bit-identical run to run."""
+    K = len(lengths)
+    fade = np.zeros(K, dtype=np.int64) if fade_out is None else _check_fades(fade_out)
+    return _mix(packed, src_offsets, lengths, onsets, gains, track_len, fade, _check_peak(target_peak), _check_pans(pans, K))
+
+
+def shift_and_mix(sources, semitones, note_source, onsets, gains, fades=None, target_peak: Optional[float] = None,
+                  pans=None) -> torch.Tensor:
     """The arrangement stage after synthesis: every source (1-D fp32 device tensor) is pitch-shifted by its semitones in ONE batched
     call, then note n -- source note_source[n] at sample onsets[n], scaled by gains[n] -- is mixed in ONE call.  Two library
-    calls plus their workspace queries, whatever the number of notes.  ``fades`` (per note, in samples) or ``target_peak``
-    mix through mix_arrangement; without either, through mix_track."""
+    calls plus their workspace queries, whatever the number of notes.  ``pans`` (per note) mix through mix_stereo into [2, L];
+    otherwise ``fades`` (per note, in samples) or ``target_peak`` mix through mix_arrangement; without either, through
+    mix_track."""
     lengths = [int(s.numel()) for s in sources]
     shifted = pitch_shift_packed(torch.cat([s.reshape(-1) for s in sources]), lengths, semitones)
     starts = np.concatenate([[0], np.cumsum(lengths)[:-1]]).astype(np.int64)
     idx = np.asarray(note_source, dtype=np.int64)
     note_len = np.asarray(lengths, dtype=np.int64)[idx]
+    if pans is not None:
+        return mix_stereo(shifted, starts[idx], note_len, onsets, gains, pans, fades, target_peak)
     if fades is None and target_peak is None:
         return mix_track(shifted, starts[idx], note_len, onsets, gains)
     fades = np.zeros(len(idx), dtype=np.int64) if fades is None else fades

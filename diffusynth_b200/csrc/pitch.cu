@@ -11,6 +11,7 @@
 #include "common.cuh"
 #include "fft_warp.cuh"
 #include <cmath>
+#include <type_traits>
 #include <vector>
 #include "../../include/diffusynth_b200.h"
 
@@ -203,30 +204,39 @@ pitch_resample_kernel(const float* __restrict__ ys, float* __restrict__ out, con
   }
 }
 
-// ---- track mix (ds_mix_arrangement, and ds_mix_track without fades or peak): track[j] = sum over notes n covering j, in input
-// order, of gain_n * env_n * src[src_off_n + j - onset_n].  A gather over track samples (one block per MIX_TILE samples) through the
-// per-tile note lists, so the sum order is fixed.  env_n is a linear fade over the last fade_n = min(fade_out[n], len[n]) samples
-// (clamped on the host); a sample before the ramp takes a plain fmaf(gain, src, acc), so a fade-free note has no envelope multiply
-// at all.  When `peak` is non-null, each tile also writes its max |track| partial.  Every thread owns ARR_SPT samples 256 apart
-// and walks the tile's notes once for all of them (a note's metadata is loaded once per thread, not once per sample); each sample
-// still sums its notes in input order.  256 threads per block.
+// ---- track mix (ds_mix_arrangement, ds_mix_stereo, and ds_mix_track without fades or peak): channel c of the output, planar
+// [CH][track_len], is out_c[j] = sum over notes n covering j, in input order, of gain_n,c * env_n * src[src_off_n + j - onset_n].
+// A gather over track samples (one block per MIX_TILE samples) through the per-tile note lists, so the sum order is fixed.  env_n
+// is a linear fade over the last fade_n = min(fade_out[n], len[n]) samples (clamped on the host); a sample before the ramp takes a
+// plain fmaf(gain, src, acc), so a fade-free note has no envelope multiply at all.  When `peak` is non-null, each tile also writes
+// its max |out| partial over every channel.  Every thread owns ARR_SPT samples 256 apart and walks the tile's notes once for all
+// of them (a note's metadata is loaded once per thread, not once per sample); each sample still sums its notes in input order.
+// CH = 1 takes one fp32 gain per note, CH = 2 one float2 (left, right) from plan_mix's pan law.  256 threads per block.
 constexpr int ARR_SPT = MIX_TILE / 256;
+template <int CH> using MixGain = std::conditional_t<CH == 1, float, float2>;
+__device__ __forceinline__ void gain_channels(float v, float (&g)[1]) { g[0] = v; }
+__device__ __forceinline__ void gain_channels(float2 v, float (&g)[2]) { g[0] = v.x; g[1] = v.y; }
+
+template <int CH>
 __global__ void __launch_bounds__(256)
 pitch_arrange_kernel(const float* __restrict__ src, float* __restrict__ track, long long track_len, const int* __restrict__ tile_ptr,
                      const int* __restrict__ tile_notes, const long long* __restrict__ src_off, const long long* __restrict__ len,
-                     const long long* __restrict__ onset, const float* __restrict__ gain, const long long* __restrict__ fade,
+                     const long long* __restrict__ onset, const MixGain<CH>* __restrict__ gain, const long long* __restrict__ fade,
                      float* __restrict__ peak) {
   pdl_enter();
   __shared__ float red[8];
   const int p0 = __ldg(tile_ptr + blockIdx.x), p1 = __ldg(tile_ptr + blockIdx.x + 1);
   const long long j0 = (long long)blockIdx.x * MIX_TILE + threadIdx.x;
-  float acc[ARR_SPT];
+  float acc[CH][ARR_SPT];
 #pragma unroll
-  for (int k = 0; k < ARR_SPT; ++k) acc[k] = 0.f;
+  for (int c = 0; c < CH; ++c)
+#pragma unroll
+    for (int k = 0; k < ARR_SPT; ++k) acc[c][k] = 0.f;
   for (int p = p0; p < p1; ++p) {
     const int n = __ldg(tile_notes + p);
     const long long on = __ldg(onset + n), L = __ldg(len + n), F = __ldg(fade + n);   // (samples past track_len have r >= L)
-    const float g = __ldg(gain + n);
+    float g[CH];
+    gain_channels(__ldg(gain + n), g);
     const float* sn = src + __ldg(src_off + n);
 #pragma unroll
     for (int k = 0; k < ARR_SPT; ++k) {
@@ -234,8 +244,11 @@ pitch_arrange_kernel(const float* __restrict__ src, float* __restrict__ track, l
       if (r < 0 || r >= L) continue;
       const float s = __ldg(sn + r);
       const long long left = L - r;                                       // 1 on the note's last sample
-      if (left > F) acc[k] = fmaf(g, s, acc[k]);
-      else acc[k] = fmaf(g * ((float)left / (float)F), s, acc[k]);
+#pragma unroll
+      for (int c = 0; c < CH; ++c) {
+        if (left > F) acc[c][k] = fmaf(g[c], s, acc[c][k]);
+        else acc[c][k] = fmaf(g[c] * ((float)left / (float)F), s, acc[c][k]);
+      }
     }
   }
   float pk = 0.f;
@@ -243,8 +256,11 @@ pitch_arrange_kernel(const float* __restrict__ src, float* __restrict__ track, l
   for (int k = 0; k < ARR_SPT; ++k) {
     const long long j = j0 + 256 * k;
     if (j < track_len) {
-      track[j] = acc[k];
-      pk = fmaxf(pk, fabsf(acc[k]));
+#pragma unroll
+      for (int c = 0; c < CH; ++c) {
+        track[c * track_len + j] = acc[c][k];
+        pk = fmaxf(pk, fabsf(acc[c][k]));
+      }
     }
   }
   if (!peak) return;
@@ -258,7 +274,8 @@ pitch_arrange_kernel(const float* __restrict__ src, float* __restrict__ track, l
 }
 
 // ---- peak normalisation: every block reduces the n_tiles partials (a maximum: exact in any order), then scales its grid-stride
-// share of the track by target / max in place.  An all-zero track stays zero.
+// share of the track by target / max in place (both channels of a stereo mix: track_len is 2 * its length, one common scale).  An
+// all-zero track stays zero.
 __global__ void __launch_bounds__(512)
 pitch_peak_scale_kernel(float* __restrict__ track, long long track_len, const float* __restrict__ peak, int n_tiles, float target) {
   pdl_enter();
@@ -342,18 +359,24 @@ int plan_pitch(const long long* lengths, const double* n_steps, int B, const cha
 }
 
 // Per-tile note lists of a mix (CSR over tiles of MIX_TILE track samples, notes in input order) and the clamped fades, staged with
-// the per-note arrays; one peak partial per tile after them when normalising.
+// the per-note arrays; one peak partial per tile after them when normalising.  A stereo mix stages its (left, right) gains in
+// place of the fp32 gains.
 struct MixPlan {
   std::vector<int> tile_ptr, tile_notes;
   std::vector<long long> fade;
+  std::vector<float2> gain2;
   Workspace ws;
   size_t off_notes = 0, off_src = 0, off_len = 0, off_onset = 0, off_gain = 0, off_fade = 0, off_peak = 0;
   int n_tiles = 0;
 };
 
-// The arrangement mix's checks and plan; ds_mix_track comes here with all-zero fades and target_peak 0.  src_offsets and gains are
-// null in the workspace queries, which do not take them.
-int plan_mix(const long long* src_offsets, const long long* lengths, const long long* onsets, const float* gains,
+// Constant-power pan law, cos(pi u / 4) for u = 1 + p (left) or 1 - p (right), in float64; cos(pi / 2) is 6.1e-17 in float64,
+// so u == 2 (a hard pan) is exactly 0 and leaks nothing into the other channel.
+double pan_cos(double u) { return u == 2.0 ? 0.0 : std::cos(kPi * u / 4.0); }
+
+// The mix's checks and plan; ds_mix_track comes here with all-zero fades and target_peak 0, and only ds_mix_stereo(_workspace)
+// passes pans.  src_offsets and gains are null in the workspace queries, which do not take them.
+int plan_mix(const long long* src_offsets, const long long* lengths, const long long* onsets, const float* gains, const float* pans,
              const long long* fade_out, int K, float target_peak, long long track_len, const char* who, MixPlan& p) {
   DS_REQUIRE(lengths && onsets && K > 0 && track_len > 0, "%s: lengths and onsets must be non-null, K > 0 and track_len > 0", who);
   DS_REQUIRE(std::isfinite(target_peak) && target_peak >= 0.f, "%s: target_peak %g (must be finite and >= 0)", who, (double)target_peak);
@@ -365,6 +388,8 @@ int plan_mix(const long long* src_offsets, const long long* lengths, const long 
     DS_REQUIRE(fade_out[n] >= 0, "%s: note %d has fade_out %lld (must be >= 0)", who, n, fade_out[n]);
     DS_REQUIRE(!src_offsets || src_offsets[n] >= 0, "%s: note %d has source offset %lld (must be >= 0)", who, n,
                src_offsets ? src_offsets[n] : 0LL);
+    DS_REQUIRE(!pans || (std::isfinite(pans[n]) && std::fabs(pans[n]) <= 1.f), "%s: note %d has pan %g (must be finite, |pan| <= 1)",
+               who, n, pans ? (double)pans[n] : 0.0);
   }
   p.n_tiles = (int)((track_len + MIX_TILE - 1) / MIX_TILE);
   std::vector<int> count(p.n_tiles + 1, 0);
@@ -383,38 +408,54 @@ int plan_mix(const long long* src_offsets, const long long* lengths, const long 
   p.off_src = p.ws.stage(src_offsets, K);
   p.off_len = p.ws.stage(lengths, K);
   p.off_onset = p.ws.stage(onsets, K);
-  p.off_gain = p.ws.stage(gains, K);
+  if (pans) {
+    p.gain2.assign(K, make_float2(0.f, 0.f));
+    for (int n = 0; gains && n < K; ++n)        // gL = g cos(pi (1 + p) / 4), gR = g cos(pi (1 - p) / 4), rounded once
+      p.gain2[n] = make_float2((float)(gains[n] * pan_cos(1.0 + pans[n])), (float)(gains[n] * pan_cos(1.0 - pans[n])));
+    p.off_gain = p.ws.stage(p.gain2.data(), K);
+  } else {
+    p.off_gain = p.ws.stage(gains, K);
+  }
   p.off_fade = p.ws.stage(p.fade.data(), K);
   if (target_peak > 0.f) p.off_peak = p.ws.reserve((size_t)p.n_tiles * sizeof(float));
   return DS_OK;
 }
 
-int mix_workspace(const long long* lengths, const long long* onsets, const long long* fade_out, int K, float target_peak,
-                  long long track_len, long long* bytes, const char* who) {
+int mix_workspace(const long long* lengths, const long long* onsets, const long long* fade_out, const float* pans, int K,
+                  float target_peak, long long track_len, long long* bytes, const char* who) {
   MixPlan p;
-  int rc = plan_mix(nullptr, lengths, onsets, nullptr, fade_out, K, target_peak, track_len, who, p);
+  int rc = plan_mix(nullptr, lengths, onsets, nullptr, pans, fade_out, K, target_peak, track_len, who, p);
   if (rc) return rc;
   *bytes = (long long)p.ws.bytes;
   return DS_OK;
 }
 
+template <int CH>
+cudaError_t launch_arrange(const MixPlan& p, const float* d_src, float* d_out, long long track_len, const uint8_t* ws, float* peak,
+                           cudaStream_t st) {
+  return launch_pdl(pitch_arrange_kernel<CH>, dim3((unsigned)p.n_tiles), dim3(256), (size_t)0, st, d_src, d_out, track_len,
+                    (const int*)ws, (const int*)(ws + p.off_notes), (const long long*)(ws + p.off_src), (const long long*)(ws + p.off_len),
+                    (const long long*)(ws + p.off_onset), (const MixGain<CH>*)(ws + p.off_gain), (const long long*)(ws + p.off_fade),
+                    peak);
+}
+
+// d_out: [track_len] mono, or planar [2][track_len] when pans is non-null
 int mix(const float* d_src, const long long* src_offsets, const long long* lengths, const long long* onsets, const float* gains,
-        const long long* fade_out, int K, float target_peak, float* d_track, long long track_len, void* d_ws, long long ws_bytes,
-        void* stream, const char* who) {
+        const float* pans, const long long* fade_out, int K, float target_peak, float* d_out, long long track_len, void* d_ws,
+        long long ws_bytes, void* stream, const char* who) {
   MixPlan p;
-  int rc = plan_mix(src_offsets, lengths, onsets, gains, fade_out, K, target_peak, track_len, who, p);
+  int rc = plan_mix(src_offsets, lengths, onsets, gains, pans, fade_out, K, target_peak, track_len, who, p);
   if (rc) return rc;
   DS_REQUIRE(ws_bytes >= (long long)p.ws.bytes, "%s: workspace of %lld bytes, %zu needed", who, ws_bytes, p.ws.bytes);
   cudaStream_t st = (cudaStream_t)stream;
   uint8_t* ws = (uint8_t*)d_ws;
   float* peak = target_peak > 0.f ? (float*)(ws + p.off_peak) : nullptr;
   DS_CHECK_CUDA(p.ws.upload(ws, st));
-  DS_CHECK_CUDA(launch_pdl(pitch_arrange_kernel, dim3((unsigned)p.n_tiles), dim3(256), (size_t)0, st, d_src, d_track, track_len,
-                           (const int*)ws, (const int*)(ws + p.off_notes), (const long long*)(ws + p.off_src),
-                           (const long long*)(ws + p.off_len), (const long long*)(ws + p.off_onset), (const float*)(ws + p.off_gain),
-                           (const long long*)(ws + p.off_fade), peak));
+  DS_CHECK_CUDA(pans ? launch_arrange<2>(p, d_src, d_out, track_len, ws, peak, st)
+                     : launch_arrange<1>(p, d_src, d_out, track_len, ws, peak, st));
+  const long long n_out = (pans ? 2 : 1) * track_len;
   if (peak)
-    DS_CHECK_CUDA(launch_pdl(pitch_peak_scale_kernel, dim3(grid_for(track_len, 512, 2)), dim3(512), (size_t)0, st, d_track, track_len,
+    DS_CHECK_CUDA(launch_pdl(pitch_peak_scale_kernel, dim3(grid_for(n_out, 512, 2)), dim3(512), (size_t)0, st, d_out, n_out,
                              (const float*)peak, p.n_tiles, target_peak));
   DS_CHECK_CUDA(cudaGetLastError());
   return DS_OK;
@@ -482,21 +523,21 @@ int ds_pitch_shift(const float* d_in, float* d_out, const long long* lengths, co
 
 int ds_mix_track_workspace(const long long* lengths, const long long* onsets, int K, long long track_len, long long* bytes) {
   DS_REQUIRE(bytes, "ds_mix_track_workspace: bytes must be non-null");
-  return mix_workspace(lengths, onsets, std::vector<long long>(K > 0 ? K : 0).data(), K, 0.f, track_len, bytes,
+  return mix_workspace(lengths, onsets, std::vector<long long>(K > 0 ? K : 0).data(), nullptr, K, 0.f, track_len, bytes,
                        "ds_mix_track_workspace");
 }
 
 int ds_mix_track(const float* d_src, const long long* src_off, const long long* lengths, const long long* onsets, const float* gains, int K,
                  float* d_track, long long track_len, void* d_ws, long long ws_bytes, void* stream) {
   DS_REQUIRE(d_src && d_track && d_ws && src_off && gains, "ds_mix_track: d_src, d_track, d_ws, src_off and gains must be non-null");
-  return mix(d_src, src_off, lengths, onsets, gains, std::vector<long long>(K > 0 ? K : 0).data(), K, 0.f, d_track, track_len, d_ws,
-             ws_bytes, stream, "ds_mix_track");
+  return mix(d_src, src_off, lengths, onsets, gains, nullptr, std::vector<long long>(K > 0 ? K : 0).data(), K, 0.f, d_track, track_len,
+             d_ws, ws_bytes, stream, "ds_mix_track");
 }
 
 int ds_mix_arrangement_workspace(const long long* lengths, const long long* onsets, const long long* fade_out, int K, float target_peak,
                                  long long track_len, long long* bytes) {
   DS_REQUIRE(bytes && fade_out, "ds_mix_arrangement_workspace: bytes and fade_out must be non-null");
-  return mix_workspace(lengths, onsets, fade_out, K, target_peak, track_len, bytes, "ds_mix_arrangement_workspace");
+  return mix_workspace(lengths, onsets, fade_out, nullptr, K, target_peak, track_len, bytes, "ds_mix_arrangement_workspace");
 }
 
 int ds_mix_arrangement(const float* d_src, const long long* src_offsets, const long long* lengths, const long long* onsets,
@@ -504,8 +545,23 @@ int ds_mix_arrangement(const float* d_src, const long long* src_offsets, const l
                        void* d_ws, long long ws_bytes, void* stream) {
   DS_REQUIRE(d_src && d_track && d_ws && src_offsets && gains && fade_out,
              "ds_mix_arrangement: d_src, d_track, d_ws, src_offsets, gains and fade_out must be non-null");
-  return mix(d_src, src_offsets, lengths, onsets, gains, fade_out, K, target_peak, d_track, track_len, d_ws, ws_bytes, stream,
+  return mix(d_src, src_offsets, lengths, onsets, gains, nullptr, fade_out, K, target_peak, d_track, track_len, d_ws, ws_bytes, stream,
              "ds_mix_arrangement");
+}
+
+int ds_mix_stereo_workspace(const long long* lengths, const long long* onsets, const long long* fade_out, const float* pans, int K,
+                            float target_peak, long long track_len, long long* bytes) {
+  DS_REQUIRE(bytes && fade_out && pans, "ds_mix_stereo_workspace: bytes, fade_out and pans must be non-null");
+  return mix_workspace(lengths, onsets, fade_out, pans, K, target_peak, track_len, bytes, "ds_mix_stereo_workspace");
+}
+
+int ds_mix_stereo(const float* d_src, const long long* src_offsets, const long long* lengths, const long long* onsets, const float* gains,
+                  const float* pans, const long long* fade_out, int K, float target_peak, float* d_out, long long track_len, void* d_ws,
+                  long long ws_bytes, void* stream) {
+  DS_REQUIRE(d_src && d_out && d_ws && src_offsets && gains && pans && fade_out,
+             "ds_mix_stereo: d_src, d_out, d_ws, src_offsets, gains, pans and fade_out must be non-null");
+  return mix(d_src, src_offsets, lengths, onsets, gains, pans, fade_out, K, target_peak, d_out, track_len, d_ws, ws_bytes, stream,
+             "ds_mix_stereo");
 }
 
 }  // extern "C"

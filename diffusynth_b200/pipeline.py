@@ -3,7 +3,7 @@ condition vectors -> DiffSynthSampler.sample (CFG, respaced DDIM/DDPM) -> Vector
 STFT+ decode + iSTFT -> waveforms, and its data-parallel form (prompts sharded over ranks, one all-gather)."""
 from __future__ import annotations
 
-from dataclasses import dataclass
+from dataclasses import dataclass, field
 from typing import Optional, Tuple
 
 import numpy as np
@@ -49,6 +49,7 @@ class ArrangementPlan:
     fades: list                  # per note: fade-out of its track in samples
     lengths: list                # per note: samples of its waveform, 256 * (4 * width - 1)
     track_len: int               # max(onset + length) over every track
+    pans: list = field(default_factory=list)   # per note: pan of its track, in [-1, 1] (0 for a 5-tuple track)
 
 
 class _Tail:
@@ -428,18 +429,26 @@ class TextToTimbre:
 
     @staticmethod
     def arrangement_plan(tracks, time_resolution: int = 256, vae_scale: int = 4, sample_rate: int = 16000) -> ArrangementPlan:
-        """Host side of render_arrangement: ``tracks`` of ``(instrument_latent, condition, notes, gain, fade_out_sec)`` -> track_plan
-        per track, joined: the synthesis rows (one per distinct (track, duration)) and their widths, the pitch items (one per
-        distinct (row, semitones)), and per note in mix order (tracks in order, notes in order) its item, onset, gain (note gain *
-        track gain), fade (round(fade_out_sec * 16000) samples) and length; the track length is the end of the last note."""
+        """Host side of render_arrangement: ``tracks`` of ``(instrument_latent, condition, notes, gain, fade_out_sec[, pan])`` ->
+        track_plan per track, joined: the synthesis rows (one per distinct (track, duration)) and their widths, the pitch items (one
+        per distinct (row, semitones)), and per note in mix order (tracks in order, notes in order) its item, onset, gain (note gain *
+        track gain), fade (round(fade_out_sec * 16000) samples), pan (the track's, 0 without one) and length; the track length is
+        the end of the last note."""
         if len(tracks) == 0:
             raise ValueError("an arrangement needs at least one track")
-        rows, widths, items, note_item, onsets, gains, fades, lengths = [], [], [], [], [], [], [], []
-        for k, (_, _, notes, gain, fade_sec) in enumerate(tracks):
+        rows, widths, items, note_item, onsets, gains, fades, pans, lengths = [], [], [], [], [], [], [], [], []
+        for k, track in enumerate(tracks):
+            if len(track) not in (5, 6):
+                raise ValueError(f"track {k}: expected (instrument_latent, condition, notes, gain, fade_out_sec[, pan]), got "
+                                 f"{len(track)} fields")
+            _, _, notes, gain, fade_sec = track[:5]
+            pan = float(track[5]) if len(track) == 6 else 0.0
             if len(notes) == 0:
                 raise ValueError(f"track {k} has no notes")
             if not np.isfinite(float(fade_sec)) or float(fade_sec) < 0:
                 raise ValueError(f"track {k}: fade_out_sec must be finite and >= 0, got {fade_sec}")
+            if not np.isfinite(pan) or abs(pan) > 1:
+                raise ValueError(f"track {k}: pan must be finite and in [-1, 1], got {track[5]}")
             fade = int(round(float(fade_sec) * sample_rate))
             p = TextToTimbre.track_plan(notes, time_resolution, vae_scale, sample_rate)
             r0, i0 = len(rows), len(items)
@@ -450,14 +459,15 @@ class TextToTimbre:
             onsets += p.onsets
             gains += [g * float(gain) for g in p.gains]
             fades += [fade] * len(p.onsets)
+            pans += [pan] * len(p.onsets)
             lengths += p.lengths
         track_len = max(o + n for o, n in zip(onsets, lengths))
-        return ArrangementPlan(rows, widths, items, note_item, onsets, gains, fades, lengths, track_len)
+        return ArrangementPlan(rows, widths, items, note_item, onsets, gains, fades, lengths, track_len, pans)
 
     @torch.no_grad()
     def render_arrangement(self, tracks, sample_steps: int = 20, noising_strength: float = 1.0, attack: float = 0.5,
                            before_release: float = 0.5, sampler: str = "ddim", target_peak: Optional[float] = None,
-                           time_resolution: int = 256, vae_scale: int = 4, noise_feeds=None) -> torch.Tensor:
+                           time_resolution: int = 256, vae_scale: int = 4, noise_feeds=None, stereo: bool = False) -> torch.Tensor:
         """Several instruments rendered into one piece on the device: track_maker.DiffSynth over several Tracks, summed.  ``tracks``
         is a list of ``(instrument_latent [1,4,128,64], condition [1,512], notes, gain, fade_out_sec)``, ``notes`` as render_track
         takes them.  The (track, duration) rows of ALL tracks are synthesised with one graph launch per distinct width, each row
@@ -465,18 +475,25 @@ class TextToTimbre:
         is placed with its gain times its track's gain, faded out linearly over the last fade_out_sec of its waveform, and summed
         in one call (ds_mix_arrangement).  ``target_peak``: None, or max |result| after a peak normalisation on the device, a
         finite value > 0 (codec._check_peak, before any synthesis).  ``noise_feeds`` (tests): one per row (arrangement_plan), in row
-        order.  Returns the fp32 piece [max(onset + note length)]."""
+        order.  Returns the fp32 piece [max(onset + note length)].
+
+        ``stereo=True`` mixes into two channels instead (ds_mix_stereo) and returns the planar [2, max(onset + note length)], left
+        then right.  A track may then carry a sixth field, its pan in [-1, 1] (-1 left, 0 centre, 1 right; a 5-tuple track is
+        centred), applied to each of its notes with a constant-power law (codec.mix_stereo); ``target_peak`` scales both channels
+        by one factor.  With ``stereo=False`` a 6-tuple track is an error."""
         _check_peak(target_peak)
+        if not stereo and any(len(t) == 6 for t in tracks):
+            raise ValueError("a track with a pan (6 fields) needs stereo=True")
         return self._render(tracks, sample_steps, noising_strength, attack, before_release, sampler, time_resolution, vae_scale,
-                            noise_feeds, fades=True, target_peak=target_peak)
+                            noise_feeds, fades=True, target_peak=target_peak, stereo=stereo)
 
     def _render(self, tracks, sample_steps, noising_strength, attack, before_release, sampler, time_resolution, vae_scale, noise_feeds,
-                fades: bool, target_peak: Optional[float]) -> torch.Tensor:
+                fades: bool, target_peak: Optional[float], stereo: bool = False) -> torch.Tensor:
         """render_arrangement's body: the plan, one synthesis launch per distinct width, one pitch shift and one mix.  ``fades``
-        False (render_track) mixes through ds_mix_track, without the tracks' fades."""
+        False (render_track) mixes through ds_mix_track, without the tracks' fades; ``stereo`` through ds_mix_stereo."""
         plan = self.arrangement_plan(tracks, time_resolution, vae_scale)
         latents, conditions = [], []
-        for k, (lat, cond, _, _, _) in enumerate(tracks):
+        for k, (lat, cond) in enumerate(t[:2] for t in tracks):
             if tuple(lat.shape) != (1, self.channels, self.height, 64):
                 raise ValueError(f"track {k}: instrument_latent must be [1, {self.channels}, {self.height}, 64], got {tuple(lat.shape)}")
             if cond.dim() != 2 or cond.shape[0] != 1:
@@ -490,8 +507,8 @@ class TextToTimbre:
                                         noise_feeds)
         sources = [timbres[r].waveforms[0] for r, _ in plan.items]
         track = shift_and_mix(sources, [s for _, s in plan.items], plan.note_item, plan.onsets, plan.gains,
-                              fades=plan.fades if fades else None, target_peak=target_peak)
-        assert track.numel() == plan.track_len
+                              fades=plan.fades if fades else None, target_peak=target_peak, pans=plan.pans if stereo else None)
+        assert track.shape[-1] == plan.track_len
         return track
 
 

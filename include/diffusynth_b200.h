@@ -266,6 +266,20 @@ int ds_mix_arrangement_workspace(const long long* lengths, const long long* onse
 int ds_mix_arrangement(const float* d_src, const long long* src_offsets, const long long* lengths, const long long* onsets,
                        const float* gains, const long long* fade_out, int K, float target_peak, float* d_track, long long track_len,
                        void* d_ws, long long ws_bytes, void* stream);
+/* Stereo arrangement mix: ds_mix_arrangement into two channels, with a constant-power pan per note.  d_out is planar fp32
+   [2][track_len], left then right: d_out[c * track_len + j] = sum over notes n in input order, fp32, of
+   g_c[n] * env_n(i) * d_src[src_offsets[n] + i], with i and env_n as in ds_mix_arrangement (one envelope for both channels).  The
+   pan law is host arithmetic in float64, rounded once to fp32 per note and channel: g_L = fl32(gains[n] * c(1 + pans[n])),
+   g_R = fl32(gains[n] * c(1 - pans[n])), c(u) = cos(pi u / 4) with c(2) = 0 exactly.  So pan -1 is hard left (g_L = gains[n]
+   exactly, g_R = 0), pan 0 gives g_L == g_R (-3 dB each) and pans p and -p swap the two gains exactly.  target_peak > 0 then
+   scales both channels in place by ONE factor, target_peak / max over both channels of |d_out| (the balance between channels is
+   kept; no host synchronisation; an all-zero piece stays zero).  Every check of ds_mix_arrangement applies; pans is non-null and
+   every pans[n] is finite with |pans[n]| <= 1.  d_ws: ds_mix_stereo_workspace bytes.  Bit-identical run to run. */
+int ds_mix_stereo_workspace(const long long* lengths, const long long* onsets, const long long* fade_out, const float* pans, int K,
+                            float target_peak, long long track_len, long long* bytes);
+int ds_mix_stereo(const float* d_src, const long long* src_offsets, const long long* lengths, const long long* onsets, const float* gains,
+                  const float* pans, const long long* fade_out, int K, float target_peak, float* d_out, long long track_len, void* d_ws,
+                  long long ws_bytes, void* stream);
 
 /* ----------------------------------------------------------------------------------------
  * Sample-rate conversion of uploaded audio (tools.adjust_audio_length, tools.py:126-151, as sound2sound_with_text.py:75-82 calls
