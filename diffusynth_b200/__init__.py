@@ -8,7 +8,7 @@ from . import weights  # noqa: F401  (pure-python parameter inventory; safe ever
 
 __all__ = ["weights", "DiffSynthSampler", "ConditionedUnet", "VQGAN", "VectorQuantizerEMA", "Decoder", "Encoder",
            "TextToTimbre", "TextEncoder", "spectrogram_to_waveform", "waveform_to_spectrogram", "pitch_shift", "mix_track", "mix_arrangement",
-           "mix_stereo", "morph_rows"]
+           "mix_stereo", "fftconvolve", "morph_rows"]
 
 
 def __getattr__(name):
@@ -29,7 +29,7 @@ def __getattr__(name):
         return TextToTimbre
     if name in ("spectrogram_to_waveform", "waveform_to_spectrogram", "encodeBatch2GradioOutput_STFT", "InputBatch2Encode_STFT",
                 "spectrogram_images", "latent_images", "latent_representation_to_Gradio_image", "griffinlim",
-                "pitch_shift", "mix_track", "mix_arrangement", "mix_stereo", "shift_and_mix", "morph_rows"):
+                "pitch_shift", "mix_track", "mix_arrangement", "mix_stereo", "shift_and_mix", "fftconvolve", "morph_rows"):
         from . import codec
         return getattr(codec, name)
     raise AttributeError(name)

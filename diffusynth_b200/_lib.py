@@ -97,6 +97,8 @@ _SIGNATURES = {
     "ds_mix_arrangement": (_I, [_P, _P, _P, _P, _P, _P, _I, _F, _P, _L, _P, _L, _P]),
     "ds_mix_stereo_workspace": (_I, [_P, _P, _P, _P, _I, _F, _L, _P]),
     "ds_mix_stereo": (_I, [_P, _P, _P, _P, _P, _P, _P, _I, _F, _P, _L, _P, _L, _P]),
+    "ds_fftconvolve_workspace": (_I, [_P, _I, _P, _I, _P, _P, _P, _F, _P]),
+    "ds_fftconvolve": (_I, [_P, _P, _P, _P, _I, _P, _I, _P, _P, _P, _I, _F, _P, _L, _P]),
     "ds_resample_workspace": (_I, [_P, _P, _P, _P, _I, _P]),
     "ds_resample": (_I, [_P, _P, _P, _P, _P, _P, _I, _I, _P, _L, _P]),
     "ds_mask_zoom_workspace": (_I, [_P, _P, _I, _P]),

@@ -319,23 +319,178 @@ def mix_stereo(packed: torch.Tensor, src_offsets, lengths, onsets, gains, pans, 
 
 
 def shift_and_mix(sources, semitones, note_source, onsets, gains, fades=None, target_peak: Optional[float] = None,
-                  pans=None) -> torch.Tensor:
+                  pans=None, impulse_response: Optional[torch.Tensor] = None, sends=None) -> torch.Tensor:
     """The arrangement stage after synthesis: every source (1-D fp32 device tensor) is pitch-shifted by its semitones in ONE batched
     call, then note n -- source note_source[n] at sample onsets[n], scaled by gains[n] -- is mixed in ONE call.  Two library
     calls plus their workspace queries, whatever the number of notes.  ``pans`` (per note) mix through mix_stereo into [2, L];
     otherwise ``fades`` (per note, in samples) or ``target_peak`` mix through mix_arrangement; without either, through
-    mix_track."""
+    mix_track.
+
+    ``impulse_response`` (an fp32 device tensor [H, M], H = 1, or 2 with ``pans``: left and right) adds convolution reverb: the
+    result is dry + IR * bus, [L + M - 1] or [2, L + M - 1], where the dry mix is the mix above without its peak, zero past L, and
+    the send bus is the same mix with gains[n] * sends[n] (post-fader, post-pan; ``sends`` per note, None = all 1).  One IR
+    convolves every channel; two convolve left with left and right with right.  ``target_peak`` scales the sum, both channels by
+    one factor.  Four library calls plus their workspace queries: the pitch shift, two mixes and one fftconvolve_packed."""
     lengths = [int(s.numel()) for s in sources]
     shifted = pitch_shift_packed(torch.cat([s.reshape(-1) for s in sources]), lengths, semitones)
     starts = np.concatenate([[0], np.cumsum(lengths)[:-1]]).astype(np.int64)
     idx = np.asarray(note_source, dtype=np.int64)
     note_len = np.asarray(lengths, dtype=np.int64)[idx]
-    if pans is not None:
-        return mix_stereo(shifted, starts[idx], note_len, onsets, gains, pans, fades, target_peak)
-    if fades is None and target_peak is None:
-        return mix_track(shifted, starts[idx], note_len, onsets, gains)
+    if impulse_response is None:
+        if pans is not None:
+            return mix_stereo(shifted, starts[idx], note_len, onsets, gains, pans, fades, target_peak)
+        if fades is None and target_peak is None:
+            return mix_track(shifted, starts[idx], note_len, onsets, gains)
+        fades = np.zeros(len(idx), dtype=np.int64) if fades is None else fades
+        return mix_arrangement(shifted, starts[idx], note_len, onsets, gains, fades, target_peak)
     fades = np.zeros(len(idx), dtype=np.int64) if fades is None else fades
-    return mix_arrangement(shifted, starts[idx], note_len, onsets, gains, fades, target_peak)
+    L, (H, M) = int((np.asarray(onsets, dtype=np.int64) + note_len).max()), impulse_response.shape
+    bus_gains = np.asarray(gains, dtype=np.float64) * (1.0 if sends is None else np.asarray(sends, dtype=np.float64))
+    if pans is not None:
+        dry = mix_stereo(shifted, starts[idx], note_len, onsets, gains, pans, fades, track_len=L + M - 1)
+        bus = mix_stereo(shifted, starts[idx], note_len, onsets, bus_gains, pans, fades, track_len=L)
+    else:
+        dry = mix_arrangement(shifted, starts[idx], note_len, onsets, gains, fades, track_len=L + M - 1)
+        bus = mix_arrangement(shifted, starts[idx], note_len, onsets, bus_gains, fades, track_len=L)
+    ch = bus.numel() // L
+    fftconvolve_packed(bus.reshape(-1), [L] * ch, impulse_response.reshape(-1), [M] * H, h_index=[0] * ch if H == 1 else [0, 1],
+                       out=dry.reshape(-1), accumulate=True, target_peak=target_peak)
+    return dry
+
+
+# ---- convolution (scipy.signal.fftconvolve; reverb of arrangements) ------------------------------------------------------------
+CONV_MODES = ("full", "same", "valid")
+
+
+def fftconvolve_range(n: int, m: int, mode: str = "full"):
+    """(start, length) of ``scipy.signal.fftconvolve(in1, in2, mode)`` for a 1-D in1 of n samples and in2 of m samples, within the
+    full convolution of n + m - 1 samples: "full" (0, n + m - 1); "same", centred on in1, ((m - 1) // 2, n); "valid"
+    (min(n, m) - 1, max(n, m) - min(n, m) + 1), which covers scipy's swap of the inputs when in2 is the longer."""
+    if mode not in CONV_MODES:
+        raise ValueError(f"mode must be one of {CONV_MODES}, got {mode!r}")
+    n, m = int(n), int(m)
+    if mode == "full":
+        return 0, n + m - 1
+    if mode == "same":
+        return (m - 1) // 2, n
+    return min(n, m) - 1, abs(n - m) + 1
+
+
+@torch.no_grad()
+def fftconvolve_packed(x: torch.Tensor, x_lengths, h: torch.Tensor, h_lengths, h_index=None, out_start=None, out_lengths=None,
+                       out: Optional[torch.Tensor] = None, accumulate: bool = False, target_peak: Optional[float] = None) -> torch.Tensor:
+    """Batched linear convolution by ds_fftconvolve: items packed back to back in the fp32 device tensor ``x`` (item k: x_lengths[k]
+    samples), IRs packed in ``h`` (IR i: h_lengths[i] samples); item k is convolved with IR h_index[k] (default k) and writes
+    out_lengths[k] samples of its full convolution starting at out_start[k] (default: the whole convolution), packed in item order.
+    ``out``: an fp32 device tensor of that size to write into; ``accumulate`` adds the convolution to what ``out`` holds.
+    ``target_peak`` scales every output of the call by one factor so that max |out| is the target."""
+    lib = _lib.load()
+    xl = np.ascontiguousarray(x_lengths, dtype=np.int64).reshape(-1)
+    hl = np.ascontiguousarray(h_lengths, dtype=np.int64).reshape(-1)
+    B, H = len(xl), len(hl)
+    hi = np.arange(B, dtype=np.int64) if h_index is None else np.ascontiguousarray(np.broadcast_to(np.asarray(h_index, dtype=np.int64), (B,)))
+    if ((hi < 0) | (hi >= H)).any():
+        raise ValueError(f"h_index must be in [0, {H}), got {hi.tolist()}")
+    st = np.zeros(B, dtype=np.int64) if out_start is None else np.ascontiguousarray(np.broadcast_to(np.asarray(out_start, dtype=np.int64), (B,)))
+    ol = xl + hl[hi] - 1 - st if out_lengths is None else np.ascontiguousarray(np.broadcast_to(np.asarray(out_lengths, dtype=np.int64), (B,)))
+    ol = np.ascontiguousarray(ol, dtype=np.int64)
+    peak = _check_peak(target_peak)
+    if accumulate and out is None:
+        raise ValueError("accumulate=True needs an output tensor to add to")
+    x = x.float().contiguous()
+    h = h.to(x.device, torch.float32).contiguous()
+    assert x.dim() == 1 and x.numel() == int(xl.sum()), "packed length of x must equal the sum of x_lengths"
+    assert h.dim() == 1 and h.numel() == int(hl.sum()), "packed length of h must equal the sum of h_lengths"
+    nbytes = C.c_longlong(0)
+    check(lib.ds_fftconvolve_workspace(xl.ctypes.data, B, hl.ctypes.data, H, hi.ctypes.data, st.ctypes.data, ol.ctypes.data, peak,
+                                       C.byref(nbytes)), "ds_fftconvolve_workspace")
+    total = int(ol.sum())
+    if out is None:
+        out = torch.empty((total,), dtype=torch.float32, device=x.device)
+    assert out.dtype == torch.float32 and out.is_contiguous() and out.numel() == total and out.device == x.device
+    ws = torch.empty((nbytes.value,), dtype=torch.uint8, device=x.device)
+    check(lib.ds_fftconvolve(x.data_ptr(), h.data_ptr(), out.data_ptr(), xl.ctypes.data, B, hl.ctypes.data, H, hi.ctypes.data,
+                             st.ctypes.data, ol.ctypes.data, 1 if accumulate else 0, peak, ws.data_ptr(), nbytes.value, ops._stream()),
+          "ds_fftconvolve")
+    return out
+
+
+def _check_impulse_response(ir, stereo: bool) -> torch.Tensor:
+    """An impulse response as render_arrangement takes it -- [M], or with ``stereo`` [2, M] (left, right); a host or device tensor
+    or a numpy array, finite and non-empty -> an fp32 CUDA tensor [H, M] (H = 1 or 2)."""
+    t = torch.from_numpy(np.asarray(ir)) if isinstance(ir, np.ndarray) else torch.as_tensor(ir)
+    if t.dim() == 2 and t.shape[0] == 2 and not stereo:
+        raise ValueError("a [2, M] impulse response (left, right) needs stereo=True")
+    if not (t.dim() == 1 or (t.dim() == 2 and t.shape[0] == 2)) or t.is_complex():
+        raise ValueError(f"impulse_response must be a real [M] or, in stereo, [2, M] array, got shape {tuple(t.shape)}")
+    if t.shape[-1] == 0:
+        raise ValueError("impulse_response is empty")
+    t = t.float().reshape(-1, t.shape[-1])
+    if not bool(torch.isfinite(t).all()):
+        raise ValueError("impulse_response must be finite in fp32")
+    return t.to(t.device if t.is_cuda else _device()).contiguous()
+
+
+def _check_sends(sends, count: int) -> np.ndarray:
+    """One float64 reverb send level per track, finite and >= 0."""
+    s = np.asarray(sends, dtype=np.float64).reshape(-1)
+    if s.shape != (count,) or not np.all(np.isfinite(s)) or np.any(s < 0):
+        raise ValueError(f"reverb_sends must be {count} finite values >= 0, got {sends}")
+    return s
+
+
+def _is_complex(a) -> bool:
+    return a.is_complex() if torch.is_tensor(a) else np.iscomplexobj(a)
+
+
+def _conv_operand(a, what: str):
+    """The 1-D signals of one fftconvolve operand: a list of them, or an array / tensor of 1 or 2 axes (NotImplementedError for
+    more batch axes and complex data, ValueError for an empty signal)."""
+    is_list = isinstance(a, (list, tuple))
+    items, max_nd = (list(a), 1) if is_list else ([a], 2)
+    if any(np.ndim(t) > max_nd for t in items):
+        raise NotImplementedError(f"{what}: only 1-D signals, or one batch axis before them, are implemented")
+    if not items or any(np.ndim(t) < 1 for t in items):
+        raise ValueError(f"{what}: expected 1-D signals, a [B, N] batch or a list of 1-D signals")
+    if any(_is_complex(t) for t in items):
+        raise NotImplementedError(f"{what}: complex inputs are not implemented")
+    if any(0 in tuple(np.shape(t)) for t in items):
+        raise ValueError(f"{what} is empty (scipy.signal.fftconvolve returns an empty array; this drop-in does not)")
+
+
+def fftconvolve(in1, in2, mode: str = "full", axes=-1):
+    """On-device, batched ``scipy.signal.fftconvolve(in1, in2, mode)`` along the last axis (ds_fftconvolve: partitioned FFTs in
+    fp32).  ``in1``: [N], [B, N] or a list of 1-D signals; ``in2``: [M] or [1, M] (one IR for every item, transformed once),
+    [B, M], or a list with one IR per item.  Modes are scipy's: "same" is centred on in1, "valid" has max(N, M) - min(N, M) + 1
+    samples (fftconvolve_range).  The result has in1's layout (numpy in, numpy out; fp32).  Deviations: ``axes`` other than -1,
+    complex data and more than one batch axis raise NotImplementedError, and an empty input raises ValueError where scipy returns
+    an empty array."""
+    if not (axes == -1 or (isinstance(axes, (list, tuple)) and list(axes) == [-1])):
+        raise NotImplementedError(f"only axes=-1 is implemented, got {axes!r}")
+    if mode not in CONV_MODES:
+        raise ValueError(f"mode must be one of {CONV_MODES}, got {mode!r}")
+    _conv_operand(in1, "in1")
+    _conv_operand(in2, "in2")
+    parts, shapes, layout = _layout(in1, 1, "expected [N], [B, N] or a list of 1-D signals")
+    xl = [n for n, in shapes]
+    B = len(xl)
+    if isinstance(in2, (list, tuple)):
+        hparts = list(in2)
+    elif np.ndim(in2) == 1 or np.shape(in2)[0] == 1:
+        hparts = [in2]
+    else:
+        hparts = [in2[i] for i in range(np.shape(in2)[0])]
+    if len(hparts) not in (1, B):
+        raise ValueError(f"in2 must hold one IR or one per item ({B}), got {len(hparts)}")
+    hl = [int(np.shape(t)[-1]) for t in hparts]
+    hi = [0] * B if len(hparts) == 1 else list(range(B))
+    rng = [fftconvolve_range(n, hl[i], mode) for n, i in zip(xl, hi)]
+    if layout[0] == "batch" and len({n for _, n in rng}) > 1:
+        raise ValueError("a [B, N] input needs IRs that give every row the same output length; pass lists instead")
+    x = _pack(parts)
+    h = _pack([t.reshape(-1) if torch.is_tensor(t) else np.reshape(t, -1) for t in hparts], device=x.device)
+    out = fftconvolve_packed(x, xl, h, hl, hi, [s for s, _ in rng], [n for _, n in rng])
+    return _unpack(out, [(n,) for _, n in rng], layout)
 
 
 # ---- sample-rate conversion (tools.adjust_audio_length's librosa.resample, tools.py:126-151) ----------------------------------

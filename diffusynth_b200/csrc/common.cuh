@@ -92,6 +92,10 @@ struct Workspace {
   }
 };
 
+// Peak normalisation (pitch.cu; the arrangement mixes and convolve.cu): reduces n_tiles max |x| partials on the device and scales
+// d_out[0, n) in place by target / max, leaving an all-zero output zero.  One PDL launch, no host synchronisation.
+cudaError_t launch_peak_scale(float* d_out, long long n, const float* peak, int n_tiles, float target, cudaStream_t st);
+
 // resampy's kaiser_best filter (pitch.cu, resample.cu): 64 zero crossings per side, roll-off and Kaiser beta
 constexpr double kPi = 3.14159265358979323846;
 constexpr int RS_ZEROS = 64;

@@ -60,6 +60,33 @@ __device__ __forceinline__ void store_bitrev(float2* __restrict__ xs, const floa
   for (int r = 0; r < R; ++r) xs[pidx<R>(hi | (int)(__brev((unsigned)r) >> (32 - LR)))] = x[r];
 }
 
+// ---- 2048-point real transforms from the 1024-point complex one (pitch.cu, convolve.cu) ------------------------------------
+// Forward: z[n] = x[2n] + i x[2n+1] went through fft_warp<-1, R> and store_bitrev into xs; the 1025 bins of the real spectrum are
+//   X[k] = (Z[k] + conj Z[1024-k])/2 - i/2 e^{-2 pi i k/2048} (Z[k] - conj Z[1024-k]),  k = 0..1024, written to out[k].
+template <int R>
+__device__ __forceinline__ void rfft2048_unpack(const float2* __restrict__ xs, float2* __restrict__ out, const float2* __restrict__ tw2048,
+                                                int lane) {
+  constexpr int NC = 32 * R;
+  for (int b = lane; b < NC + 1; b += 32) {
+    const float2 zk = xs[pidx<R>(b & (NC - 1))], zc = xs[pidx<R>((NC - b) & (NC - 1))];
+    const float2 e = make_float2(0.5f * (zk.x + zc.x), 0.5f * (zk.y - zc.y));
+    const float2 d = make_float2(0.5f * (zk.x - zc.x), 0.5f * (zk.y + zc.y));
+    float2 w = b < NC ? __ldg(tw2048 + b) : make_float2(-1.f, 0.f);
+    w.y = -w.y;
+    const float2 o = cmul(d, w);                          // then multiply by -i: (x, y) -> (y, -x)
+    out[b] = make_float2(e.x + o.y, e.y - o.x);
+  }
+}
+// Inverse: the input of fft_warp<+1, R> at point k from the bins a = X[k] and c = X[1024-k],
+//   Z[k] = (X[k] + conj X[1024-k]) + i e^{2 pi i k/2048} (X[k] - conj X[1024-k]); irfft ignores Im of DC and Nyquist (k == 0).
+//   The caller scales the transform's result by 1/2048, as numpy's irfft does.
+__device__ __forceinline__ float2 irfft2048_pack(float2 a, float2 c, const float2* __restrict__ tw2048, int k) {
+  if (k == 0) { a.y = 0.f; c.y = 0.f; }
+  const float2 e = make_float2(a.x + c.x, a.y - c.y);
+  const float2 o = cmul(make_float2(a.x - c.x, a.y + c.y), __ldg(tw2048 + k));
+  return make_float2(e.x - o.y, e.y + o.x);
+}
+
 // Per-device twiddle tables e^{+2 pi i j/N}, j < N/2, for N = 512, 1024 and 2048 (istft.cu).  Built on first use; that first
 // call must not be under stream capture.
 int get_twiddles(cudaStream_t stream, float2** tw512, float2** tw1024, float2** tw2048);

@@ -53,17 +53,7 @@ pitch_stft_kernel(const float* __restrict__ y, const long long* __restrict__ lof
   fft_warp<-1, R>(x, tw1024, lane);
   store_bitrev<R>(xs[fr], x, lane);
   __syncwarp();
-  // X[k] = (Z[k] + conj Z[1024-k])/2 - i/2 e^{-2 pi i k/2048} (Z[k] - conj Z[1024-k]),  k = 0..1024
-  float2* out = D + g * NBIN;
-  for (int b = lane; b < NBIN; b += 32) {
-    const float2 zk = xs[fr][pidx<R>(b & (NC - 1))], zc = xs[fr][pidx<R>((NC - b) & (NC - 1))];
-    const float2 e = make_float2(0.5f * (zk.x + zc.x), 0.5f * (zk.y - zc.y));
-    const float2 d = make_float2(0.5f * (zk.x - zc.x), 0.5f * (zk.y + zc.y));
-    float2 w = b < NC ? __ldg(tw2048 + b) : make_float2(-1.f, 0.f);
-    w.y = -w.y;
-    const float2 o = cmul(d, w);                          // then multiply by -i: (x, y) -> (y, -x)
-    out[b] = make_float2(e.x + o.y, e.y - o.x);
-  }
+  rfft2048_unpack<R>(xs[fr], D + g * NBIN, tw2048, lane);
 }
 
 // ---- phase vocoder (librosa.phase_vocoder, hop 512): one thread per (item, bin), output frames walked in order ----------------
@@ -107,7 +97,6 @@ pitch_vocoder_kernel(const float2* __restrict__ D, float2* __restrict__ S, const
 }
 
 // ---- inverse STFT frames: S [frames][1025] -> windowed frames [frames][2048]; one frame per warp -------------------------------
-// Z[k] = (X[k] + conj X[1024-k]) + i e^{2 pi i k/2048} (X[k] - conj X[1024-k]); irfft ignores Im of DC and Nyquist.
 __global__ void __launch_bounds__(256)
 pitch_istft_frames_kernel(const float2* __restrict__ S, float* __restrict__ frames, long long n_frames,
                           const float2* __restrict__ tw1024, const float2* __restrict__ tw2048) {
@@ -122,11 +111,7 @@ pitch_istft_frames_kernel(const float2* __restrict__ S, float* __restrict__ fram
 #pragma unroll
   for (int r = 0; r < R; ++r) {
     const int k = lane + 32 * r;
-    float2 a = __ldg(X + k), c = __ldg(X + NC - k);
-    if (k == 0) { a.y = 0.f; c.y = 0.f; }
-    const float2 e = make_float2(a.x + c.x, a.y - c.y);
-    const float2 o = cmul(make_float2(a.x - c.x, a.y + c.y), __ldg(tw2048 + k));
-    x[r] = make_float2(e.x - o.y, e.y + o.x);
+    x[r] = irfft2048_pack(__ldg(X + k), __ldg(X + NC - k), tw2048, k);
   }
   fft_warp<+1, R>(x, tw1024, lane);
   store_bitrev<R>(xs[fr], x, lane);
@@ -453,15 +438,17 @@ int mix(const float* d_src, const long long* src_offsets, const long long* lengt
   DS_CHECK_CUDA(p.ws.upload(ws, st));
   DS_CHECK_CUDA(pans ? launch_arrange<2>(p, d_src, d_out, track_len, ws, peak, st)
                      : launch_arrange<1>(p, d_src, d_out, track_len, ws, peak, st));
-  const long long n_out = (pans ? 2 : 1) * track_len;
-  if (peak)
-    DS_CHECK_CUDA(launch_pdl(pitch_peak_scale_kernel, dim3(grid_for(n_out, 512, 2)), dim3(512), (size_t)0, st, d_out, n_out,
-                             (const float*)peak, p.n_tiles, target_peak));
+  if (peak) DS_CHECK_CUDA(launch_peak_scale(d_out, (pans ? 2 : 1) * track_len, peak, p.n_tiles, target_peak, st));
   DS_CHECK_CUDA(cudaGetLastError());
   return DS_OK;
 }
 
 }  // namespace
+
+cudaError_t launch_peak_scale(float* d_out, long long n, const float* peak, int n_tiles, float target, cudaStream_t st) {
+  return launch_pdl(pitch_peak_scale_kernel, dim3(grid_for(n, 512, 2)), dim3(512), (size_t)0, st, d_out, n, peak, n_tiles, target);
+}
+
 }  // namespace ds
 
 using namespace ds;

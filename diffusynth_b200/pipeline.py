@@ -11,7 +11,7 @@ import torch
 
 from . import _lib, ops, weights as W
 from ._lib import check
-from .codec import MORPH_PATHS, SAMPLE_RATE, _check_peak, _layout, _pack, morph_rows, resample_packed, shift_and_mix, \
+from .codec import MORPH_PATHS, SAMPLE_RATE, _check_impulse_response, _check_peak, _check_sends, _layout, _pack, morph_rows, resample_packed, shift_and_mix, \
     spectrogram_to_waveform, waveform_to_spectrogram, zoom_packed
 from .sampler import DiffSynthSampler
 from .unet import ConditionedUnet
@@ -50,6 +50,7 @@ class ArrangementPlan:
     lengths: list                # per note: samples of its waveform, 256 * (4 * width - 1)
     track_len: int               # max(onset + length) over every track
     pans: list = field(default_factory=list)   # per note: pan of its track, in [-1, 1] (0 for a 5-tuple track)
+    sends: list = field(default_factory=list)  # per note: reverb send level of its track (1.0 without reverb_sends)
 
 
 class _Tail:
@@ -428,15 +429,17 @@ class TextToTimbre:
                             sampler, time_resolution, vae_scale, noise_feeds, fades=False, target_peak=None)
 
     @staticmethod
-    def arrangement_plan(tracks, time_resolution: int = 256, vae_scale: int = 4, sample_rate: int = 16000) -> ArrangementPlan:
+    def arrangement_plan(tracks, time_resolution: int = 256, vae_scale: int = 4, sample_rate: int = 16000,
+                         reverb_sends=None) -> ArrangementPlan:
         """Host side of render_arrangement: ``tracks`` of ``(instrument_latent, condition, notes, gain, fade_out_sec[, pan])`` ->
         track_plan per track, joined: the synthesis rows (one per distinct (track, duration)) and their widths, the pitch items (one
         per distinct (row, semitones)), and per note in mix order (tracks in order, notes in order) its item, onset, gain (note gain *
-        track gain), fade (round(fade_out_sec * 16000) samples), pan (the track's, 0 without one) and length; the track length is
-        the end of the last note."""
+        track gain), fade (round(fade_out_sec * 16000) samples), pan (the track's, 0 without one), reverb send (reverb_sends[track],
+        one finite value >= 0 per track; 1.0 when None) and length; the track length is the end of the last note."""
         if len(tracks) == 0:
             raise ValueError("an arrangement needs at least one track")
-        rows, widths, items, note_item, onsets, gains, fades, pans, lengths = [], [], [], [], [], [], [], [], []
+        track_sends = [1.0] * len(tracks) if reverb_sends is None else [float(v) for v in _check_sends(reverb_sends, len(tracks))]
+        rows, widths, items, note_item, onsets, gains, fades, pans, sends, lengths = [], [], [], [], [], [], [], [], [], []
         for k, track in enumerate(tracks):
             if len(track) not in (5, 6):
                 raise ValueError(f"track {k}: expected (instrument_latent, condition, notes, gain, fade_out_sec[, pan]), got "
@@ -460,14 +463,16 @@ class TextToTimbre:
             gains += [g * float(gain) for g in p.gains]
             fades += [fade] * len(p.onsets)
             pans += [pan] * len(p.onsets)
+            sends += [track_sends[k]] * len(p.onsets)
             lengths += p.lengths
         track_len = max(o + n for o, n in zip(onsets, lengths))
-        return ArrangementPlan(rows, widths, items, note_item, onsets, gains, fades, lengths, track_len, pans)
+        return ArrangementPlan(rows, widths, items, note_item, onsets, gains, fades, lengths, track_len, pans, sends)
 
     @torch.no_grad()
     def render_arrangement(self, tracks, sample_steps: int = 20, noising_strength: float = 1.0, attack: float = 0.5,
                            before_release: float = 0.5, sampler: str = "ddim", target_peak: Optional[float] = None,
-                           time_resolution: int = 256, vae_scale: int = 4, noise_feeds=None, stereo: bool = False) -> torch.Tensor:
+                           time_resolution: int = 256, vae_scale: int = 4, noise_feeds=None, stereo: bool = False,
+                           impulse_response=None, reverb_sends=None) -> torch.Tensor:
         """Several instruments rendered into one piece on the device: track_maker.DiffSynth over several Tracks, summed.  ``tracks``
         is a list of ``(instrument_latent [1,4,128,64], condition [1,512], notes, gain, fade_out_sec)``, ``notes`` as render_track
         takes them.  The (track, duration) rows of ALL tracks are synthesised with one graph launch per distinct width, each row
@@ -480,18 +485,35 @@ class TextToTimbre:
         ``stereo=True`` mixes into two channels instead (ds_mix_stereo) and returns the planar [2, max(onset + note length)], left
         then right.  A track may then carry a sixth field, its pan in [-1, 1] (-1 left, 0 centre, 1 right; a 5-tuple track is
         centred), applied to each of its notes with a constant-power law (codec.mix_stereo); ``target_peak`` scales both channels
-        by one factor.  With ``stereo=False`` a 6-tuple track is an error."""
+        by one factor.  With ``stereo=False`` a 6-tuple track is an error.
+
+        ``impulse_response`` adds convolution reverb (codec.shift_and_mix): a 16 kHz impulse response [M], or with ``stereo=True``
+        [2, M] (left, right), as a host or device tensor or a numpy array, used as given, so its level is the wet level.  An IR
+        recorded at another rate is converted first with codec.resample(ir, sr, 16000).  ``reverb_sends``: one finite send level
+        >= 0 per track (None: 1.0 for every track; an error without an IR).  The send is post-fader and post-pan: the send bus is
+        every note with its gain times its track's send, with the same fades and pans.  The result is dry + IR * bus, the piece
+        followed by the reverb tail: [L + M - 1], or planar [2, L + M - 1] in stereo, L = max(onset + note length).  A mono IR
+        convolves both channels of a stereo piece; a [2, M] IR convolves left with left and right with right.  ``target_peak``
+        applies after the reverb is added, with one factor over both channels.  Every argument is checked before synthesis."""
         _check_peak(target_peak)
         if not stereo and any(len(t) == 6 for t in tracks):
             raise ValueError("a track with a pan (6 fields) needs stereo=True")
+        if impulse_response is None and reverb_sends is not None:
+            raise ValueError("reverb_sends needs an impulse_response")
+        if reverb_sends is not None:
+            _check_sends(reverb_sends, len(tracks))
+        ir = None if impulse_response is None else _check_impulse_response(impulse_response, stereo)
         return self._render(tracks, sample_steps, noising_strength, attack, before_release, sampler, time_resolution, vae_scale,
-                            noise_feeds, fades=True, target_peak=target_peak, stereo=stereo)
+                            noise_feeds, fades=True, target_peak=target_peak, stereo=stereo, impulse_response=ir,
+                            reverb_sends=reverb_sends)
 
     def _render(self, tracks, sample_steps, noising_strength, attack, before_release, sampler, time_resolution, vae_scale, noise_feeds,
-                fades: bool, target_peak: Optional[float], stereo: bool = False) -> torch.Tensor:
+                fades: bool, target_peak: Optional[float], stereo: bool = False, impulse_response: Optional[torch.Tensor] = None,
+                reverb_sends=None) -> torch.Tensor:
         """render_arrangement's body: the plan, one synthesis launch per distinct width, one pitch shift and one mix.  ``fades``
-        False (render_track) mixes through ds_mix_track, without the tracks' fades; ``stereo`` through ds_mix_stereo."""
-        plan = self.arrangement_plan(tracks, time_resolution, vae_scale)
+        False (render_track) mixes through ds_mix_track, without the tracks' fades; ``stereo`` through ds_mix_stereo; a checked
+        ``impulse_response`` [H, M] adds a second mix (the send bus) and one convolution."""
+        plan = self.arrangement_plan(tracks, time_resolution, vae_scale, reverb_sends=reverb_sends)
         latents, conditions = [], []
         for k, (lat, cond) in enumerate(t[:2] for t in tracks):
             if tuple(lat.shape) != (1, self.channels, self.height, 64):
@@ -507,8 +529,9 @@ class TextToTimbre:
                                         noise_feeds)
         sources = [timbres[r].waveforms[0] for r, _ in plan.items]
         track = shift_and_mix(sources, [s for _, s in plan.items], plan.note_item, plan.onsets, plan.gains,
-                              fades=plan.fades if fades else None, target_peak=target_peak, pans=plan.pans if stereo else None)
-        assert track.shape[-1] == plan.track_len
+                              fades=plan.fades if fades else None, target_peak=target_peak, pans=plan.pans if stereo else None,
+                              impulse_response=impulse_response, sends=plan.sends)
+        assert track.shape[-1] == plan.track_len + (0 if impulse_response is None else impulse_response.shape[1] - 1)
         return track
 
 

@@ -280,6 +280,27 @@ int ds_mix_stereo_workspace(const long long* lengths, const long long* onsets, c
 int ds_mix_stereo(const float* d_src, const long long* src_offsets, const long long* lengths, const long long* onsets, const float* gains,
                   const float* pans, const long long* fade_out, int K, float target_peak, float* d_out, long long track_len, void* d_ws,
                   long long ws_bytes, void* stream);
+/* Batched linear convolution (scipy.signal.fftconvolve along the last axis; a project extension, used for convolution reverb):
+   B signals packed back to back in d_x (item k: x_lengths[k] = N_k samples, fp32) and H impulse responses packed in d_h (IR i:
+   h_lengths[i] samples).  Item k is convolved with IR h_index[k] (items may share an IR, whose spectra are computed once), and
+   writes out_lengths[k] samples of its full convolution (N_k + M - 1 samples, M = h_lengths[h_index[k]]) starting at full index
+   out_start[k], packed back to back in item order in d_out: mode "full" is out_start 0, out_lengths N + M - 1; "same" and
+   "valid" are crops of it.  Arithmetic: uniformly partitioned FFTs, P = 1024, 2048-point real transforms in fp32.  Output
+   segment s is Y_s = sum over q in ASCENDING order of X_{s-q} * H_q (1025 complex bins each), inverse-transformed to the 2047
+   samples at s * 1024; output j = seg_s[j - 1024 s] + seg_{s-1}[j - 1024 (s-1)], added in that order.  No atomics: item k's
+   result does not depend on the rest of the batch (a batch equals each item run alone, bit for bit) and repeats bit for bit.
+   accumulate 0 overwrites d_out; 1 writes fl(d_out[j] + conv[j]).  target_peak > 0 then scales ALL outputs of the call in place
+   by ONE factor, target_peak / max |d_out| over every item (both channels of a stereo piece are items of one call; an all-zero
+   output stays zero; no host synchronisation); 0 leaves them unscaled.  Checks, before any device work: non-null pointers;
+   B, H >= 1; every length >= 1; 0 <= h_index[k] < H; out_start[k] >= 0 and out_start[k] + out_lengths[k] <= N_k + M - 1;
+   finite target_peak >= 0; accumulate 0 or 1; ws_bytes large enough.  d_ws: ds_fftconvolve_workspace bytes (the metadata, the
+   spectra of every block and partition, 8200 bytes per 1024 samples, and the segments, 8192 bytes per 1024 output samples
+   computed).  4 launches, 3 without a peak, and one host-to-device copy, whatever B, N and M. */
+int ds_fftconvolve_workspace(const long long* x_lengths, int B, const long long* h_lengths, int H, const long long* h_index,
+                             const long long* out_start, const long long* out_lengths, float target_peak, long long* bytes);
+int ds_fftconvolve(const float* d_x, const float* d_h, float* d_out, const long long* x_lengths, int B, const long long* h_lengths, int H,
+                   const long long* h_index, const long long* out_start, const long long* out_lengths, int accumulate, float target_peak,
+                   void* d_ws, long long ws_bytes, void* stream);
 
 /* ----------------------------------------------------------------------------------------
  * Sample-rate conversion of uploaded audio (tools.adjust_audio_length, tools.py:126-151, as sound2sound_with_text.py:75-82 calls
